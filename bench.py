@@ -26,6 +26,10 @@ Each sub-result has its own `value`, `roofline`, `e2e`, `clocks`, `cpu_baseline`
   cpu_baseline / --impl reference : the CPU oracle (C restatement of the reference's algorithm: a full Float64 row
               dot per update; Julia is not installed here), on all host cores and on 1 thread (the reference itself
               is single-threaded: src/SamplingHelper.jl:42-50).
+
+  --dump-outputs DIR : after the timed steps, what the last timed step of the printed workload computed, as
+              DIR/<name>.npy (spins in float32, flip counts in float64), so that two builds can be compared output for
+              output: the inputs depend only on the arguments.
 """
 import argparse
 import json
@@ -33,11 +37,13 @@ import math
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from, which may be read-only
 
 import numpy as np  # noqa: E402
 
@@ -157,7 +163,7 @@ class Runtime:
         self.nccl_log = None
         if self.world > 1:
             # NCCL's own communicator lines (ranks, transport, NVLS) go to a file and are quoted in the c5 sub-result
-            self.nccl_log = f"/tmp/isb_nccl_{os.getpid()}.log"
+            self.nccl_log = os.path.join(tempfile.gettempdir(), f"isb_nccl_{os.getpid()}.log")
             os.environ.setdefault("NCCL_DEBUG", "INFO")
             os.environ.setdefault("NCCL_DEBUG_SUBSYS", "INIT")
             os.environ.setdefault("NCCL_DEBUG_FILE", self.nccl_log)
@@ -252,6 +258,23 @@ def base_line(value, world, steps, warmup, ms_per_step, dtype, cfg):
     return {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": steps, "warmup": warmup,
             "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": dtype, "data": "synthetic", "config": cfg}
+
+
+DUMP_BYTES = 60 << 20          # below 64 MB (decimal) with the .npy headers
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: `arrays` (name -> one row per replica) as path/<name>.npy, int8 spins as float32 and everything
+    else as float64.  Above DUMP_BYTES in all, every array keeps the same fixed, seeded sample of replicas (sorted)."""
+    os.makedirs(path, exist_ok=True)
+    out = {k: np.asarray(a, dtype=np.float32 if np.asarray(a).dtype == np.int8 else np.float64) for k, a in arrays.items()}
+    R = len(next(iter(out.values())))
+    row_bytes = sum(a[0].nbytes for a in out.values())
+    keep = slice(None)
+    if R * row_bytes > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(R, DUMP_BYTES // row_bytes, replace=False))
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a[keep])
 
 
 # ---------------------------------------------------------------------------------------------- CPU arm (oracle)
@@ -380,7 +403,7 @@ def reference_arm(args, out):
 
 
 # ---------------------------------------------------------------------------------------------- C2: dense sweeps
-def run_c2(rt, args, steps, warmup, cpu=True):
+def run_c2(rt, args, steps, warmup, cpu=True, dump=None):
     from isingmodel_jl_b200 import synth, SpinSystems, SingleSpinFlip, SamplingHelper
     L = rt.L
     sweeps = args.sweeps
@@ -396,12 +419,15 @@ def run_c2(rt, args, steps, warmup, cpu=True):
     ua = SingleSpinFlip.GlauberDynamics(ss, T0)
     ens = ss._ensemble()
     rt.last_stats = ens.last_stats
+    last = {}
 
     def step(k):
-        ens.ssf_run(L.RULE_GLAUBER, nsteps, order=L.ORDER_SEQUENTIAL, seed=12345 + rt.rank, step_offset=k * nsteps,
-                    T=T, steps_per_T=N_SITES)
+        last["out"] = ens.ssf_run(L.RULE_GLAUBER, nsteps, order=L.ORDER_SEQUENTIAL, seed=12345 + rt.rank,
+                                  step_offset=k * nsteps, T=T, steps_per_T=N_SITES)
 
     steps, t_dev, stats, clocks = rt.run_steps(lambda: ens.set_spins(S0p), step, warmup, steps)
+    if dump and rt.rank == 0:
+        dump_outputs(dump, {"spins": ens.get_spins(), "flips": last["out"]["flips"]})
 
     def e2e_step(k):
         rt.flush.zero_()
@@ -474,7 +500,7 @@ def c1_config(args):
             "updates_per_step_per_gpu": 1024 * 4096 * sweeps, "sharding": "replicas (no collective)", "l2": "flushed between timed steps"}
 
 
-def run_c1(rt, args, steps, warmup, cpu=True):
+def run_c1(rt, args, steps, warmup, cpu=True, dump=None):
     """BASELINE config 1: built from a sparse J exactly as the reference's tests / demo build theirs."""
     import scipy.sparse as sp
     from isingmodel_jl_b200 import synth, SpinSystems, SingleSpinFlip, SamplingHelper
@@ -491,11 +517,15 @@ def run_c1(rt, args, steps, warmup, cpu=True):
     ens = ss._ensemble()
     rt.last_stats = ens.last_stats
     Tarr = np.array([T1])
+    last = {}
 
     def step(k):
-        ens.ssf_run(L.RULE_METROPOLIS, nsteps, seed=99 + rt.rank, step_offset=k * nsteps, T=Tarr, steps_per_T=nsteps)
+        last["out"] = ens.ssf_run(L.RULE_METROPOLIS, nsteps, seed=99 + rt.rank, step_offset=k * nsteps, T=Tarr,
+                                  steps_per_T=nsteps)
 
     steps, t_dev, stats, clocks = rt.run_steps(lambda: ens.set_spins(pin), step, warmup, steps)
+    if dump and rt.rank == 0:
+        dump_outputs(dump, {"spins": ens.get_spins(), "flips": last["out"]["flips"]})
     rt.barrier()
     n_e2e = min(steps, 5)
     t0 = time.perf_counter()
@@ -604,7 +634,7 @@ def sca_config(which, desc, W, R, nst, prec_name=None):
     return c
 
 
-def run_sca(rt, args, which, precs, steps, warmup, cpu=True):
+def run_sca(rt, args, which, precs, steps, warmup, cpu=True, dump=None):
     """precs[0] is the primary precision (top level of the result, with e2e); the others are timed the same way and
     reported under `precisions`."""
     from isingmodel_jl_b200 import synth, SpinSystems, OnBipartiteGraph, SamplingHelper
@@ -639,6 +669,8 @@ def run_sca(rt, args, which, precs, steps, warmup, cpu=True):
         nsteps_i, t_dev, stats, clocks = rt.run_steps(reset, step, warmup, steps if i == 0 else None)
         e2e = None
         if i == 0:
+            if dump and rt.rank == 0:
+                dump_outputs(dump, {"spins": ens.get_spins(), "hidden": ens.get_hidden()})
             def e2e_step(k):
                 rt.flush.zero_()
                 rt.torch.cuda.synchronize()
@@ -712,7 +744,7 @@ def run_sca(rt, args, which, precs, steps, warmup, cpu=True):
 
 
 # ---------------------------------------------------------------------------------------------- C5: row-sharded SCA
-def run_c5(rt, args, prec_name, steps, warmup):
+def run_c5(rt, args, prec_name, steps, warmup, dump=None):
     """BASELINE config 5: dense J with N = 8192 x GPUs (65536 on 8), rows of W = (J + qI)/2 sharded across the GPUs,
     R replicas, SCA annealing, the freshly sampled spin blocks exchanged after every half-step (NVLink)."""
     from isingmodel_jl_b200 import synth, rowshard
@@ -741,6 +773,8 @@ def run_c5(rt, args, prec_name, steps, warmup):
         sca.run(nst, T, seed=31, step_offset=k * nst)
 
     steps, t_dev, _, clocks = rt.run_steps(lambda: sca.set_spins(S0), step, warmup, steps)
+    if dump and rt.rank == 0:
+        dump_outputs(dump, {"spins": sca.get_spins()})
     launches = (sca.launches - l0) * steps // (steps + warmup)
     pin = rt.pinned((R, n))
     pin[:] = S0
@@ -827,7 +861,11 @@ def main():
                     help="all (default): the C2 headline + every other BASELINE config as `workloads` sub-results")
     ap.add_argument("--sca-steps", type=int, default=None, help="SCA steps per bench step (c3: 200, c4: 1000, c5: 10)")
     ap.add_argument("--sub-warmup", type=int, default=3, help="warm-up steps of the sub-workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the printed workload computed as DIR/<name>.npy (rank 0's replicas)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times bounded samples and has no outputs to compare")
     # ONE JSON line on stdout: whatever a library prints there (NCCL's version banner under NCCL_DEBUG, compiler chatter)
     # is sent to stderr at the file-descriptor level; the line itself goes to the saved descriptor at the end
     out = os.fdopen(os.dup(1), "w")
@@ -839,16 +877,17 @@ def main():
     rt = Runtime(args)
     tensor_precs = args.prec.split(",") if args.prec and args.workload != "c2" else ["i8x3", "fp16x2", "bf16x3", "bf16x1"]
     c5_prec = tensor_precs[0] if tensor_precs[0] in ("bf16x3", "bf16x2", "bf16x1", "i8x3", "i8x2", "i8x4") else "i8x3"
+    dump = args.dump_outputs
     if args.workload == "c2":
-        line = run_c2(rt, args, args.steps, args.warmup)
+        line = run_c2(rt, args, args.steps, args.warmup, dump=dump)
     elif args.workload == "c1":
-        line = run_c1(rt, args, args.steps, args.warmup)
+        line = run_c1(rt, args, args.steps, args.warmup, dump=dump)
     elif args.workload in ("c3", "c4"):
-        line = run_sca(rt, args, args.workload, tensor_precs, args.steps, args.warmup)
+        line = run_sca(rt, args, args.workload, tensor_precs, args.steps, args.warmup, dump=dump)
     elif args.workload == "c5":
-        line = run_c5(rt, args, c5_prec, args.steps, args.warmup)
+        line = run_c5(rt, args, c5_prec, args.steps, args.warmup, dump=dump)
     else:
-        line = run_c2(rt, args, args.steps, args.warmup)
+        line = run_c2(rt, args, args.steps, args.warmup, dump=dump)
         subs = {}
         if rt.world == 1:
             subs["c1"] = run_c1(rt, args, None, args.sub_warmup)
