@@ -194,6 +194,32 @@ int isb_ssf_run_hist(isb_ens *e, int rule, int64_t nsteps, int order, const int3
                      const double *Tsched, int64_t nT, int64_t steps_per_T, int64_t trace_every,
                      int64_t *hist);
 
+/* Parallel tempering (replica exchange) with the round loop on the device: R = ladders * n_levels replicas, replica
+ * r = ladder * n_levels + slot; level_of[r] (in/out, a permutation of 0..n_levels-1 within each ladder) is the index into
+ * levels[] that replica r holds.  Round k (absolute round K = round_offset + k) is exactly
+ *   isb_ssf_run(rule, steps_per_round, order, (start + k*steps_per_round) mod N, ISB_FLUCT_PHILOX, seed,
+ *               step_offset + k*steps_per_round, Tsched = {1.0}, steps_per_T = trace_every = steps_per_round)
+ * with per-replica factors levels[level_of[r]], followed by one exchange in every ladder g: for
+ * lo = K&1, K&1 + 2, ... <= n_levels-2, with a, b the replicas holding lo and lo+1,
+ *   d = (1/levels[lo] - 1/levels[lo+1]) * (E_a - E_b)      (IEEE round-to-nearest, no contraction)
+ *   u = (w + 1/2) 2^-32, w = word .x of Philox4x32-10(counter (lo32(K), hi32(K), g, 5 << 28 | lo), key seed)
+ * and levels lo, lo+1 (and their temperature factors) swap between a and b when d >= 0 or u < exp(d); the spins stay.
+ * E is the energy the sweep kernel traced at the last step of the round (isb_ssf_run's out_E).
+ *   rule              : ISB_RULE_GLAUBER or ISB_RULE_METROPOLIS; order: sequential, random or checkerboard.
+ *   out_E, out_M      : [rounds][n_levels][ladders]: energy / magnetisation traced in round k by the replica that held
+ *                       level l during that round (before the swaps).
+ *   out_Q             : [rounds][n_levels][ladders/2]: overlap (sum_i s_i^a s_i^b) / N of the replicas of ladders 2p and
+ *                       2p+1 that held level l during round k, at its end (an even number of ladders is required).
+ *   out_accepted      : [n_levels-1] accepted swaps per level pair in this call (proposed: ladders x rounds of the
+ *                       pair's parity).  out_flips: [R] flips per replica summed over the rounds.
+ * Every output may be NULL.  On return level_of holds the final assignment and the ensemble's temperature factors are
+ * levels[level_of], so a later isb_ssf_run continues the ladders; two calls of K rounds (start, step_offset and
+ * round_offset continued) equal one call of 2K rounds bit for bit.  rounds = 0 is a no-op. */
+int isb_ssf_run_pt(isb_ens *e, int rule, int n_levels, const double *levels, int64_t rounds, int64_t steps_per_round,
+                   int order, int start, uint64_t seed, uint64_t step_offset, uint64_t round_offset,
+                   int32_t *level_of, double *out_E, double *out_M, double *out_Q,
+                   int64_t *out_accepted, int64_t *out_flips);
+
 /* Fluctuations exactly as ISB_FLUCT_PHILOX generates them inside isb_ssf_run, for parity tests:
  * out[r*nsteps + k], r in [r0, r0+nr). rule selects the transform. prec as the model's. */
 int isb_philox_fluct(isb_ctx *ctx, int rule, int prec, uint64_t seed, uint64_t step_offset,

@@ -84,6 +84,7 @@ SIGNATURES = {
     "isb_ssf_run_snap": (_i, [_vp, _i, _i64, _i, _vp, _i, _i, _vp, _u64, _u64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp,
                               _i64]),
     "isb_ssf_run_hist": (_i, [_vp, _i, _i64, _i, _vp, _i, _i, _vp, _u64, _u64, _vp, _i64, _i64, _i64, _vp]),
+    "isb_ssf_run_pt": (_i, [_vp, _i, _i, _vp, _i64, _i64, _i, _i, _u64, _u64, _u64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "isb_philox_fluct": (_i, [_vp, _i, _i, _u64, _u64, _i, _i, _i64, _vp]),
     "isb_philox_nodes": (_i, [_vp, _i, _u64, _u64, _i64, _vp]),
     "isb_philox_raw": (_i, [_vp, _vp, _vp, _i, _vp]),
@@ -527,6 +528,30 @@ class Ensemble:
                                           int(steps_per_T), int(trace_every), ptr(E), ptr(M), ptr(flips), ptr(S),
                                           self.nv))
         return {"flips": flips, "E": E, "M": M, "S": S}
+
+    def ssf_run_pt(self, rule, levels, rounds, steps_per_round, *, order=ORDER_SEQUENTIAL, start=0, seed=0, step_offset=0,
+                   round_offset=0, level_of=None, want_E=True, want_M=False, want_Q=False):
+        """isb_ssf_run_pt: ``rounds`` rounds of ``steps_per_round`` steps, each followed by one replica exchange, all on the
+        device.  ``level_of`` (R entries, default: slot s of every ladder holds level s) is the level each replica holds.
+        Returns dict(level_of[R] (final), E / M [rounds][levels][ladders] | None, Q [rounds][levels][ladders/2] | None,
+        accepted[levels-1], flips[R])."""
+        lv = np.ascontiguousarray(levels, dtype=np.float64).reshape(-1)
+        L, rounds = lv.size, int(rounds)
+        G = self.R // L if L else 0
+        if level_of is None:       # slot s of every ladder holds level s (a mismatch of R and L is the library's error)
+            level_of = np.arange(self.R) % L if L else np.zeros(self.R)
+        lo = np.array(level_of, dtype=np.int32).reshape(-1)
+        if lo.size != self.R:
+            raise IsbError(ERR_SIZE, f"level_of has {lo.size} entries for {self.R} replicas")
+        E = np.zeros((rounds, L, G)) if want_E else None
+        M = np.zeros((rounds, L, G)) if want_M else None
+        Q = np.zeros((rounds, L, G // 2)) if want_Q else None
+        acc = np.zeros(max(L - 1, 0), dtype=np.int64)
+        flips = np.zeros(self.R, dtype=np.int64)
+        self._chk(load().isb_ssf_run_pt(self.handle, int(rule), L, ptr(lv), rounds, int(steps_per_round), int(order),
+                                        int(start), int(seed), int(step_offset), int(round_offset), ptr(lo), ptr(E),
+                                        ptr(M), ptr(Q), ptr(acc), ptr(flips)))
+        return {"level_of": lo, "E": E, "M": M, "Q": Q, "accepted": acc, "flips": flips}
 
     def bip_run(self, rule, nsteps, *, Fv=None, Fh=None, fluct_per_replica=False, seed=0, step_offset=0, T=None,
                 steps_per_T=1, trace_every=0, want_S=False):

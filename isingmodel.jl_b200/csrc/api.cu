@@ -883,6 +883,114 @@ static int ssf_run_impl(isb_ens *e, int rule, int64_t nsteps, int order, const i
     return ISB_OK;
 }
 
+int isb_ssf_run_pt(isb_ens *e, int rule, int n_levels, const double *levels, int64_t rounds, int64_t steps_per_round,
+                   int order, int start, uint64_t seed, uint64_t step_offset, uint64_t round_offset, int32_t *level_of,
+                   double *out_E, double *out_M, double *out_Q, int64_t *out_accepted, int64_t *out_flips) {
+    if (!e) return ISB_ERR_ARG;
+    isb_model *m = e->model;
+    isb_ctx *ctx = m->ctx;
+    ISB_LOCK(ctx);
+    const char *who = "isb_ssf_run_pt";
+    if (!general_graph(m)) return fail(ctx, ISB_ERR_STATE, "%s: not a general-graph ensemble", who);
+    if (rule != ISB_RULE_GLAUBER && rule != ISB_RULE_METROPOLIS)
+        return fail(ctx, ISB_ERR_ARG, "%s: rule %d has no temperature to exchange (Glauber or Metropolis only)", who, rule);
+    if (order < ISB_ORDER_SEQUENTIAL || order > ISB_ORDER_CHECKERBOARD || order == ISB_ORDER_LIST)
+        return fail(ctx, ISB_ERR_ARG, "%s: order %d is not sequential, random or checkerboard", who, order);
+    if (order == ISB_ORDER_CHECKERBOARD && !(m->kind == ISB_KIND_SPARSE || !m->fast_ok))
+        return fail(ctx, ISB_ERR_UNSUPPORTED, "%s: ISB_ORDER_CHECKERBOARD needs a periodic L x L lattice given as a sparse model", who);
+    if (n_levels < 1) return fail(ctx, ISB_ERR_ARG, "%s: n_levels = %d must be positive", who, n_levels);
+    if (n_levels > 1024) return fail(ctx, ISB_ERR_UNSUPPORTED, "%s: n_levels = %d > 1024", who, n_levels);
+    if (e->R % n_levels != 0)
+        return fail(ctx, ISB_ERR_SIZE, "%s: R = %d replicas is not a multiple of n_levels = %d", who, e->R, n_levels);
+    const int L = n_levels, G = e->R / n_levels;
+    if (!levels || !level_of) return fail(ctx, ISB_ERR_ARG, "%s: levels and level_of are required", who);
+    if (!all_finite(levels, (size_t)L)) return fail(ctx, ISB_ERR_NONFINITE, "%s: non-finite temperature level", who);
+    for (int l = 0; l < L; ++l)
+        if (!(levels[l] > 0.0)) return fail(ctx, ISB_ERR_ARG, "%s: levels[%d] = %g must be positive", who, l, levels[l]);
+    {
+        std::vector<char> seen((size_t)L);
+        for (int g = 0; g < G; ++g) {
+            std::fill(seen.begin(), seen.end(), 0);
+            for (int s = 0; s < L; ++s) {
+                const int32_t v = level_of[(size_t)g * L + s];
+                if (v < 0 || v >= L || seen[v])
+                    return fail(ctx, ISB_ERR_ARG, "%s: level_of of ladder %d is not a permutation of 0..%d", who, g, L - 1);
+                seen[v] = 1;
+            }
+        }
+    }
+    if (out_Q && G % 2 != 0) return fail(ctx, ISB_ERR_SIZE, "%s: overlaps pair ladders 2p, 2p+1; %d ladders is odd", who, G);
+    if (steps_per_round <= 0)
+        return fail(ctx, ISB_ERR_ARG, "%s: steps_per_round = %lld must be positive", who, (long long)steps_per_round);
+    if (rounds < 0) return fail(ctx, ISB_ERR_ARG, "%s: rounds = %lld is negative", who, (long long)rounds);
+    if (order != ISB_ORDER_RANDOM && (start < 0 || start >= m->n))
+        return fail(ctx, ISB_ERR_ARG, "%s: start = %d outside [0, %d)", who, start, m->n);
+    ISB_CUDA(ctx, cudaSetDevice(ctx->device));
+    begin_stats(e);
+    if (out_accepted) std::fill(out_accepted, out_accepted + (L - 1), (int64_t)0);
+    if (rounds == 0) {
+        if (out_flips) std::fill(out_flips, out_flips + e->R, (int64_t)0);
+        return ISB_OK;
+    }
+
+    // device state of the call: levels [L] | accepted [L] | flip totals [R] (8-byte words) | level_of [R] (int32)
+    const size_t R = (size_t)e->R;
+    char *st = nullptr;
+    ISB_TRY(isb::dev_reserve(ctx, isb::SCR_PT_STATE, 8 * (2 * (size_t)L + R) + 4 * R, (void **)&st));
+    double *d_levels = (double *)st;
+    unsigned long long *d_acc = (unsigned long long *)(st + 8 * (size_t)L);
+    unsigned long long *d_ftot = (unsigned long long *)(st + 16 * (size_t)L);
+    int32_t *d_level_of = (int32_t *)(st + 8 * (2 * (size_t)L + R));
+    int32_t *d_nodes = nullptr;
+    double *d_T = nullptr, *d_Er = nullptr, *d_Mr = nullptr, *d_recE = nullptr, *d_recM = nullptr, *d_recQ = nullptr;
+    if (order == ISB_ORDER_RANDOM)
+        ISB_TRY(isb::dev_reserve(ctx, isb::SCR_NODES, (size_t)steps_per_round * sizeof(int32_t), (void **)&d_nodes));
+    ISB_TRY(isb::dev_reserve(ctx, isb::SCR_T, sizeof(double), (void **)&d_T));
+    ISB_TRY(isb::dev_reserve(ctx, isb::SCR_E, R * sizeof(double), (void **)&d_Er));
+    if (out_M) ISB_TRY(isb::dev_reserve(ctx, isb::SCR_M, R * sizeof(double), (void **)&d_Mr));
+    if (out_E) ISB_TRY(isb::dev_reserve(ctx, isb::SCR_PT_E, (size_t)rounds * R * sizeof(double), (void **)&d_recE));
+    if (out_M) ISB_TRY(isb::dev_reserve(ctx, isb::SCR_PT_M, (size_t)rounds * R * sizeof(double), (void **)&d_recM));
+    if (out_Q) ISB_TRY(isb::dev_reserve(ctx, isb::SCR_PT_Q, (size_t)rounds * L * (G / 2) * sizeof(double), (void **)&d_recQ));
+    if (!e->d_tscale) ISB_CUDA(ctx, cudaMalloc(&e->d_tscale, R * sizeof(double)));
+    std::vector<double> tsc(R);
+    for (size_t r = 0; r < R; ++r) tsc[r] = levels[level_of[r]];
+    const double one = 1.0;
+    ISB_TRY(h2d(ctx, d_levels, levels, (size_t)L * sizeof(double), &e->last_h2d));
+    ISB_TRY(h2d(ctx, d_level_of, level_of, R * sizeof(int32_t), &e->last_h2d));
+    ISB_TRY(h2d(ctx, e->d_tscale, tsc.data(), R * sizeof(double), &e->last_h2d));
+    ISB_TRY(h2d(ctx, d_T, &one, sizeof(double), &e->last_h2d));
+    ISB_CUDA(ctx, cudaMemsetAsync(d_acc, 0, 8 * ((size_t)L + R), ctx->stream));
+    ISB_CUDA(ctx, cudaMemsetAsync(e->d_counters, 0, 4 * sizeof(unsigned long long), ctx->stream));
+
+    ISB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    ISB_TRY(isb::ssf_pt_run_device(e, rule, L, d_levels, rounds, steps_per_round, order, start, seed, step_offset,
+                                   round_offset, d_nodes, d_T, d_level_of, d_Er, d_Mr, d_recE, d_recM, d_recQ, d_acc, d_ftot));
+    ISB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+
+    std::vector<unsigned long long> acc((size_t)L), ftot(R);
+    unsigned long long counters[4] = {0, 0, 0, 0};
+    ISB_TRY(d2h(ctx, level_of, d_level_of, R * sizeof(int32_t), &e->last_d2h));
+    ISB_TRY(d2h(ctx, acc.data(), d_acc, (size_t)L * sizeof(unsigned long long), &e->last_d2h));
+    ISB_TRY(d2h(ctx, ftot.data(), d_ftot, R * sizeof(unsigned long long), &e->last_d2h));
+    ISB_TRY(d2h(ctx, counters, e->d_counters, sizeof counters, &e->last_d2h));
+    if (d_recE) ISB_TRY(d2h(ctx, out_E, d_recE, (size_t)rounds * R * sizeof(double), &e->last_d2h));
+    if (d_recM) ISB_TRY(d2h(ctx, out_M, d_recM, (size_t)rounds * R * sizeof(double), &e->last_d2h));
+    if (d_recQ) ISB_TRY(d2h(ctx, out_Q, d_recQ, (size_t)rounds * L * (G / 2) * sizeof(double), &e->last_d2h));
+    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
+    if (ce != cudaSuccess) return fail(ctx, ISB_ERR_CUDA, "%s: kernel failed: %s", who, cudaGetErrorString(ce));
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
+    e->last_ms = ms;
+    for (size_t r = 0; r < R; ++r) {
+        e->last_flips += (int64_t)ftot[r];
+        if (out_flips) out_flips[r] = (int64_t)ftot[r];
+    }
+    if (out_accepted)
+        for (int l = 0; l + 1 < L; ++l) out_accepted[l] = (int64_t)acc[l];
+    e->last_near_ties = (int64_t)counters[0];
+    return ISB_OK;
+}
+
 int isb_philox_fluct(isb_ctx *ctx, int rule, int prec, uint64_t seed, uint64_t step_offset, int r0, int nr,
                      int64_t nsteps, double *out) {
     (void)prec;

@@ -177,7 +177,9 @@ __host__ __device__ __forceinline__ uint32_t philox_pick(const Philox4 &p, uint3
 }
 
 // Stream domains (top 4 bits of counter word 3).
-enum : uint32_t { DOM_SSF_FLUCT = 1, DOM_SSF_NODES = 2, DOM_BIP_VISIBLE = 3, DOM_BIP_HIDDEN = 4 };
+enum : uint32_t { DOM_SSF_FLUCT = 1, DOM_SSF_NODES = 2, DOM_BIP_VISIBLE = 3, DOM_BIP_HIDDEN = 4, DOM_PT_SWAP = 5 };
+// Replica-exchange decisions (isb_ssf_run_pt): word .x of counter (lo(K), hi(K), ladder, DOM_PT_SWAP<<28 | lo) decides the
+// swap of levels (lo, lo+1) in that ladder after absolute round K.
 
 // Word assigned to step `step` of replica `replica` in a single-spin run:
 // counter = (lo(step>>2), hi(step>>2), replica, domain<<28), key = seed, word = step & 3.

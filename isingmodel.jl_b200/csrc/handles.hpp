@@ -22,7 +22,7 @@ struct isb_ctx {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    isb_devbuf scratch[13];      // grow-only device staging buffers (see isb::dev_reserve)
+    isb_devbuf scratch[17];      // grow-only device staging buffers (see isb::dev_reserve)
     // Every entry point that uses the stream, the events or the scratch buffers holds this lock for its whole
     // (synchronous) duration: calls on one context are serialised, different contexts run concurrently.
     std::recursive_mutex mtx;
@@ -93,7 +93,8 @@ double ssf_guard_from(const double *absrowsum, const double *vals, size_t nvals,
 // Grow-only device scratch buffer `slot` of the context, at least `bytes` long.
 int dev_reserve(isb_ctx *ctx, int slot, size_t bytes, void **out);
 enum { SCR_NODES = 0, SCR_FLUCT = 1, SCR_T = 2, SCR_E = 3, SCR_M = 4, SCR_FLUCT2 = 5, SCR_OUT = 6, SCR_TMP = 7,
-       SCR_TC0 = 8, SCR_TC1 = 9, SCR_S = 10, SCR_S2 = 11, SCR_HIST = 12 };
+       SCR_TC0 = 8, SCR_TC1 = 9, SCR_S = 10, SCR_S2 = 11, SCR_HIST = 12, SCR_PT_STATE = 13, SCR_PT_E = 14, SCR_PT_M = 15,
+       SCR_PT_Q = 16 };
 
 #define ISB_LOCK(ctx) std::lock_guard<std::recursive_mutex> isb_lock_guard_((ctx)->mtx)
 
@@ -144,6 +145,14 @@ int lattice_side(const void *lat);
 int ssf_lattice_run_device(isb_ens *e, void *lat, int rule, int64_t nsteps, int order, int start, int fluct_mode, const double *d_fluct,
                            uint64_t seed, uint64_t step_offset, const double *d_T, int64_t steps_per_T, int64_t trace_every,
                            double *d_E, double *d_M, int8_t *d_S);
+
+// tempering.cu: `rounds` rounds of isb_ssf_run_pt on the context stream, no host synchronisation between rounds.  Round k
+// is one sweep launch of steps_per_round steps (traced E / M of its last step into d_Eround / d_Mround [R]), the overlap
+// kernel when d_recQ is given, then the exchange kernel (level_of, e->d_tscale, acceptance counts, flip totals, records).
+int ssf_pt_run_device(isb_ens *e, int rule, int n_levels, const double *d_levels, int64_t rounds, int64_t steps_per_round,
+                      int order, int start, uint64_t seed, uint64_t step_offset, uint64_t round_offset, int32_t *d_nodes,
+                      const double *d_T, int32_t *d_level_of, double *d_Eround, double *d_Mround, double *d_recE,
+                      double *d_recM, double *d_recQ, unsigned long long *d_accepted, unsigned long long *d_flips_total);
 
 // bip_exact.cu
 int bip_run_exact_device(isb_ens *e, int rule, int64_t nsteps, int fluct_mode, const double *d_Fv,

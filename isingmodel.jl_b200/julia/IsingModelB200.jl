@@ -132,6 +132,21 @@ function ssf_run!(e, rule, nsteps; nodes = nothing, start = 1, fluct = nothing, 
                     length(Tv), steps_per_T, trace_every, _optr(E, Float64), C_NULL, C_NULL, snap, size(snap, 1)), context())
     end
 end
+# Parallel tempering with the round loop inside the library (isb_ssf_run_pt).  `level_of` (Vector{Int32}, one 0-based
+# level per replica, replica = ladder * length(levels) + slot) is updated in place.  E / M: levels x ladders x rounds
+# (column-major == the ABI's [rounds][levels][ladders]), Q: levels x ladders/2 x rounds, accepted: levels - 1, flips: R.
+function ssf_run_pt!(e, rule, levels, rounds, steps_per_round, level_of::Vector{Int32}; order = ORDER_SEQUENTIAL,
+                     start = 1, seed = 0, step_offset = 0, round_offset = 0, E = nothing, M = nothing, Q = nothing,
+                     accepted = nothing, flips = nothing)
+    lv = Vector{Float64}(levels)
+    check(ccall((:isb_ssf_run_pt, libisb), Cint,
+                (Ens, Cint, Cint, Ptr{Float64}, Int64, Int64, Cint, Cint, UInt64, UInt64, UInt64, Ptr{Int32},
+                 Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Int64}),
+                e, rule, length(lv), lv, rounds, steps_per_round, order, start - 1, seed, step_offset, round_offset,
+                level_of, _optr(E, Float64), _optr(M, Float64), _optr(Q, Float64), _optr(accepted, Int64),
+                _optr(flips, Int64)), context())
+    level_of
+end
 # Fv / Fh: (units, steps) column-major == [steps][units].  With snapV / snapH (units x R x ntr Int8) the call is
 # isb_bip_run_snap.
 function bip_run!(e, rule, nsteps; Fv = nothing, Fh = nothing, per_replica = false, seed = 0, step_offset = 0,

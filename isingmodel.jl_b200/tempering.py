@@ -104,3 +104,52 @@ class ParallelTempering:
                 self.level[la, a[acc]], self.level[la, b[acc]] = lo + 1, lo
             self._push()
         return out
+
+
+class DeviceParallelTempering:
+    """``ParallelTempering`` with the whole round loop on the device (isb_ssf_run_pt): the same ladder layout (replica =
+    ladder * len(levels) + slot), the same ``level[ladder, slot]``, ``accepted`` and ``proposed`` attributes and the same
+    ``run`` result, without a host round trip per round.  The swaps draw from the library's counter RNG (``seed``), so
+    the trajectory is a pure function of the seed and the absolute round; consecutive ``run`` calls continue it.
+    ``order``: "sequential", "random" or "checkerboard" (periodic lattices)."""
+
+    _ORDERS = {"sequential": _lib.ORDER_SEQUENTIAL, "random": _lib.ORDER_RANDOM, "checkerboard": _lib.ORDER_CHECKERBOARD}
+
+    def __init__(self, ua, levels, *, seed=0, order="sequential"):
+        self.ua, self.ss = ua, ua.spinSystem
+        self.levels = np.asarray(levels, dtype=np.float64)
+        L = len(self.levels)
+        if L < 1 or self.ss.replicas % L:
+            raise ValueError("the number of replicas must be a multiple of the number of temperature levels")
+        if order not in self._ORDERS:
+            raise ValueError(f"order must be one of {sorted(self._ORDERS)}")
+        self.nlad = self.ss.replicas // L
+        self.level = np.tile(np.arange(L), (self.nlad, 1))
+        self.seed, self.order = int(seed), order
+        self.offset = 0          # steps run so far (the Philox step offset of the next round)
+        self.round = 0           # rounds run so far (the absolute round index of the next exchange)
+        self.accepted = np.zeros(L - 1, dtype=np.int64)
+        self.proposed = np.zeros(L - 1, dtype=np.int64)
+        ua.temperature = 1.0
+        ua.temperatureScale = self.levels[self.level].reshape(-1)
+
+    def run(self, rounds, sweeps=1, *, overlaps=False):
+        """Returns E[rounds][levels][ladders]: the energy traced at each temperature level at the end of each round; with
+        ``overlaps`` also Q[rounds][levels][ladders/2], the overlap of ladders 2p and 2p+1 at each level."""
+        n = self.ss._host_spins.shape[1]
+        L = len(self.levels)
+        ens = self.ss._ensemble()
+        out = ens.ssf_run_pt(self.ua._rule, self.levels, rounds, sweeps * n, order=self._ORDERS[self.order],
+                             start=self.offset % n if self.order != "random" else 0, seed=self.seed,
+                             step_offset=self.offset, round_offset=self.round, level_of=self.level.reshape(-1),
+                             want_Q=overlaps)
+        self.ss._dev_newer = True
+        K = self.round + np.arange(rounds)
+        for lo in range(L - 1):
+            self.proposed[lo] += self.nlad * int(np.count_nonzero((K & 1) == (lo & 1)))
+        self.accepted += out["accepted"]
+        self.level = out["level_of"].reshape(self.nlad, L).astype(np.int64)
+        self.offset += rounds * sweeps * n
+        self.round += rounds
+        self.ua.temperatureScale = self.levels[self.level].reshape(-1)
+        return (out["E"], out["Q"]) if overlaps else out["E"]
