@@ -352,6 +352,9 @@ int isb_ens_last_stats(const isb_ens *e, double *kernel_ms, int64_t *launches, i
 int64_t isb_ens_last_flips(const isb_ens *e);
 /* Decisions of the last run whose |2h - fT| was below tie_eps (near-tie audit, SURVEY 7.2). */
 int64_t isb_ens_last_near_ties(const isb_ens *e);
+/* Decisions of the last run that the fixed-point sweep kernels could not settle from their integer fields and took on
+ * the reference's fresh Float64 row dot instead (DESIGN §3; 0 for runs on the Float64 kernels). */
+int64_t isb_ens_last_exact_fallbacks(const isb_ens *e);
 int isb_ens_set_tie_eps(isb_ens *e, double eps);
 /* Per-replica temperature factors (scale: R entries, NULL clears them): replica r runs every later *_run call at
  * T_r(k) = Tsched[k] * scale[r].  R reference objects that differ only in their `temperature` field

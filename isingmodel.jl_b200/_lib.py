@@ -113,6 +113,7 @@ SIGNATURES = {
     "isb_ens_last_stats": (_i, [_vp, C.POINTER(_d), C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_i64)]),
     "isb_ens_last_flips": (_i64, [_vp]),
     "isb_ens_last_near_ties": (_i64, [_vp]),
+    "isb_ens_last_exact_fallbacks": (_i64, [_vp]),
     "isb_ens_set_tie_eps": (_i, [_vp, _d]),
     "isb_ens_set_temperature_scale": (_i, [_vp, _vp]),
 }
@@ -582,4 +583,5 @@ class Ensemble:
         load().isb_ens_last_stats(self.handle, C.byref(ms), C.byref(nl), C.byref(hi), C.byref(do))
         return {"kernel_ms": ms.value, "launches": nl.value, "h2d_bytes": hi.value, "d2h_bytes": do.value,
                 "flips": load().isb_ens_last_flips(self.handle),
-                "near_ties": load().isb_ens_last_near_ties(self.handle)}
+                "near_ties": load().isb_ens_last_near_ties(self.handle),
+                "exact_fallbacks": load().isb_ens_last_exact_fallbacks(self.handle)}

@@ -206,6 +206,75 @@ static int next_pow2(int v) {
     return p;
 }
 
+// Fixed-point couplings for the sweep kernels (DESIGN §3).  q = 2^-k with the largest k (|k| <= 1000) such that every row
+// sum of |Jint| = |round(J / q)| stays below 2^30, so that the cached integer fields F = Jint s and every threshold of the
+// kernels fit an int32.  M bounds, in units of q, how far the reference's own Float64 row dot can lie from F q:
+//   |J s - q Jint s| <= e_i = sum_j |J_ij - q Jint_ij|   (each term exact, the sum rounded up by a factor 1 + 2^-40),
+//   |dot_ref - J s|  <= (n - 1) 2^-53 sum_j |J_ij| < 2^-40 sum_j |J_ij|   (sequential sum of n <= 1024 exact products),
+// M = ceil(max_i (e_i + 2^-40 sum_j |J_ij|) / q) + 1, and M = 0 when every coupling is a multiple of q (then every partial
+// sum of the reference is an exact multiple of q below 2^30 q: its dot IS F q).  The model keeps the Float64 kernels when
+// M > 2^-20 sum_j |Jint_ij| for some row with couplings (a fallback band wider than 2^-20 of that row's field scale:
+// rows far weaker than the strongest one would fall back often) or when some |h_i| / q >= 2^50 (the reference's
+// h_i + dot rounds at a step above q).  Jq: the permuted int32 rows (VEC = 4), like Jperm.
+static bool fixed_point_couplings(const std::vector<double> &Jn, const std::vector<double> &hn, int n, int npad,
+                                  std::vector<int32_t> *Jq, double *q_out, int *M_out) {
+    double smax = 0.0, hmax = 0.0;
+    for (int i = 0; i < n; ++i) {
+        double s = 0.0;
+        for (int j = 0; j < n; ++j) s += std::fabs(Jn[(size_t)i * npad + j]);
+        smax = std::max(smax, s);
+        hmax = std::max(hmax, std::fabs(hn[i]));
+    }
+    int k = smax > 0.0 ? (int)std::floor(std::log2(1073741824.0 / smax)) : 0;
+    k = std::max(-1000, std::min(1000, k));
+    std::vector<int64_t> Ji((size_t)n * n);
+    for (;; --k) {
+        if (k < -1000) return false;
+        int64_t worst = 0;
+        for (int i = 0; i < n; ++i) {
+            int64_t s = 0;
+            for (int j = 0; j < n; ++j) {
+                const double v = std::nearbyint(std::ldexp(Jn[(size_t)i * npad + j], k));
+                Ji[(size_t)i * n + j] = std::fabs(v) < 4e18 ? (int64_t)v : (int64_t)1 << 62;
+                s += std::llabs(Ji[(size_t)i * n + j]);
+                if (s >= ((int64_t)1 << 30)) break;
+            }
+            worst = std::max(worst, s);
+        }
+        if (worst < ((int64_t)1 << 30)) break;
+    }
+    const double q = std::ldexp(1.0, -k);
+    double emax = 0.0;
+    int64_t smin = (int64_t)1 << 30;   // smallest nonzero row sum of |Jint|
+    bool exact = true;
+    for (int i = 0; i < n; ++i) {
+        double e = 0.0, s = 0.0;
+        int64_t si = 0;
+        for (int j = 0; j < n; ++j) {
+            si += std::llabs(Ji[(size_t)i * n + j]);
+            const double v = Jn[(size_t)i * npad + j];
+            const double d = std::fabs(v - std::ldexp((double)Ji[(size_t)i * n + j], -k));  // exact (Sterbenz, or Jint = 0)
+            exact = exact && d == 0.0;
+            e += d;
+            s += std::fabs(v);
+        }
+        emax = std::max(emax, e * (1.0 + 0x1p-40) + s * 0x1p-40);
+        if (si > 0) smin = std::min(smin, si);
+    }
+    const double Md = exact ? 0.0 : std::ceil(emax / q) + 1.0;
+    if (Md * 0x1p20 > (double)smin || hmax / q >= 0x1p50) return false;
+    const int vec = std::min(4, npad / 32);
+    Jq->assign((size_t)npad * npad, 0);
+    for (int i = 0; i < n; ++i)
+        for (int s = 0; s < n; ++s) {
+            const int kk = s >> 5, lane = s & 31;
+            (*Jq)[(size_t)i * npad + (size_t)(kk / vec) * (32 * vec) + lane * vec + (kk % vec)] = (int32_t)Ji[(size_t)i * n + s];
+        }
+    *q_out = q;
+    *M_out = (int)Md;
+    return true;
+}
+
 int isb_model_dense(isb_ctx *ctx, int n, const double *J, int64_t ld, const double *h, int prec, int *warn,
                     isb_model **out) {
     if (!ctx) return ISB_ERR_ARG;
@@ -304,6 +373,15 @@ int isb_model_dense(isb_ctx *ctx, int n, const double *J, int64_t ld, const doub
             }
             cudaMemcpyAsync(m->Jperm, Jp.data(), nn * jsz, cudaMemcpyHostToDevice, ctx->stream);
             cudaStreamSynchronize(ctx->stream);
+            std::vector<int32_t> Jq;
+            if (m->prec == ISB_PREC_F64 && fixed_point_couplings(Jn, hn, n, npad, &Jq, &m->fix_q, &m->fix_margin)) {
+                if (cudaMalloc(&m->Jfix, nn * sizeof(int32_t)) != cudaSuccess) {
+                    rc = fail(ctx, ISB_ERR_CUDA, "isb_model_dense: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
+                    break;
+                }
+                cudaMemcpyAsync(m->Jfix, Jq.data(), nn * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream);
+                m->fixed_ok = true;
+            }
         }
         cudaError_t ce = cudaStreamSynchronize(ctx->stream);
         if (ce != cudaSuccess) rc = fail(ctx, ISB_ERR_CUDA, "isb_model_dense: upload failed: %s", cudaGetErrorString(ce));
@@ -449,6 +527,7 @@ static void model_release(isb_model *m) {
         if (m->sp) isb::sparse_model_free(m);
         cudaFree(m->J64);
         cudaFree(m->Jperm);
+        cudaFree(m->Jfix);
         cudaFree(m->h64);
         cudaFree(m->W64);
         cudaFree(m->Wt64);
@@ -545,6 +624,7 @@ void isb_ens_destroy(isb_ens *e) {
         cudaFree(e->spins);
         cudaFree(e->hidden);
         cudaFree(e->fields);
+        cudaFree(e->ifields);
         cudaFree(e->d_flips);
         cudaFree(e->d_counters);
         cudaFree(e->d_tscale);
@@ -612,6 +692,7 @@ static int copy_spins_in(isb_ens *e, int8_t *dst, int64_t ldd, int n, const int8
                                     ctx->stream));
     ISB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     e->fields_rule_sign = 0;
+    e->ifields_ok = false;
     return ISB_OK;
 }
 static int copy_spins_out(isb_ens *e, const int8_t *src, int64_t lds, int n, int8_t *s, int64_t ld, const char *who) {
@@ -724,7 +805,7 @@ static int check_schedule(isb_ctx *ctx, const char *who, const double *Tsched, i
 static void begin_stats(isb_ens *e) {
     e->last_ms = 0.0;
     e->last_launches = e->last_h2d = e->last_d2h = 0;
-    e->last_flips = e->last_near_ties = 0;
+    e->last_flips = e->last_near_ties = e->last_exact_fallbacks = 0;
 }
 
 static int ssf_run_impl(isb_ens *e, int rule, int64_t nsteps, int order, const int32_t *nodes, int start, int fluct_mode,
@@ -879,6 +960,7 @@ static int ssf_run_impl(isb_ens *e, int rule, int64_t nsteps, int order, const i
         if (out_flips) out_flips[r] = (int64_t)fl[r];
     }
     e->last_near_ties = (int64_t)counters[0];
+    e->last_exact_fallbacks = (int64_t)counters[1];
     for (size_t b = 0; b < hh.size(); ++b) hist[b] += (int64_t)hh[b];
     return ISB_OK;
 }
@@ -988,6 +1070,7 @@ int isb_ssf_run_pt(isb_ens *e, int rule, int n_levels, const double *levels, int
     if (out_accepted)
         for (int l = 0; l + 1 < L; ++l) out_accepted[l] = (int64_t)acc[l];
     e->last_near_ties = (int64_t)counters[0];
+    e->last_exact_fallbacks = (int64_t)counters[1];
     return ISB_OK;
 }
 
@@ -1239,6 +1322,7 @@ int isb_ens_last_stats(const isb_ens *e, double *kernel_ms, int64_t *launches, i
 }
 int64_t isb_ens_last_flips(const isb_ens *e) { return e ? e->last_flips : 0; }
 int64_t isb_ens_last_near_ties(const isb_ens *e) { return e ? e->last_near_ties : 0; }
+int64_t isb_ens_last_exact_fallbacks(const isb_ens *e) { return e ? e->last_exact_fallbacks : 0; }
 int isb_ens_set_temperature_scale(isb_ens *e, const double *scale) {
     if (!e) return ISB_ERR_ARG;
     isb_ctx *ctx = e->model->ctx;

@@ -48,6 +48,13 @@ struct isb_model {
     // near-tie guard of the single-spin kernels: 0 when every coupling and field is a small dyadic number (all sums are
     // exact), else 2^-30 of the largest row sum of |J| + |h| (see SsfParams::guard)
     double guard = 0.0;
+    // fixed-point copy for the sweep kernels (N <= 1024, Float64 models; DESIGN §3): Jint = round(J / fix_q), permuted like
+    // Jperm with VEC = 4, fix_q = 2^-k with every row sum of |Jint| below 2^30; fix_margin = M >= max_i (e_i + dot
+    // rounding) / fix_q, e_i = sum_j |J_ij - fix_q Jint_ij| (0 when every coupling is a multiple of fix_q)
+    bool fixed_ok = false;
+    int32_t *Jfix = nullptr;
+    double fix_q = 1.0;
+    int fix_margin = 0;
     // ---- bipartite: nv visible, nh hidden
     int nv = 0, nh = 0;
     double *W64 = nullptr;       // [nv][nh]  (row i = visible unit i; contiguous over hidden)
@@ -74,13 +81,15 @@ struct isb_ens {
     // incremental value drifts from a fresh row dot by a few ulp per flip.  A run that starts after this many steps
     // since the last fresh computation recomputes them first (sequential row dots, the reference's order).
     int64_t steps_since_refresh = 0;
+    int32_t *ifields = nullptr;  // fixed-point fields [R][npad] (exact integers Jint s; allocated by the first fixed-point run)
+    bool ifields_ok = false;     // false: rebuilt from the spins by the next fixed-point run
     unsigned long long *d_flips = nullptr;   // [R]
-    unsigned long long *d_counters = nullptr; // [0] near ties
+    unsigned long long *d_counters = nullptr; // [0] near ties, [1] exact fallbacks of the fixed-point kernels
     double tie_eps = 0.0;
     double *d_tscale = nullptr;  // optional per-replica temperature factors [R]: T_r(k) = Tsched[k] * tscale[r]
     // last-run statistics
     double last_ms = 0.0;
-    int64_t last_launches = 0, last_h2d = 0, last_d2h = 0, last_flips = 0, last_near_ties = 0;
+    int64_t last_launches = 0, last_h2d = 0, last_d2h = 0, last_flips = 0, last_near_ties = 0, last_exact_fallbacks = 0;
     void *tc = nullptr;          // tensor-core path state (bf16 spin matrices), owned by bip_tc.cu
 };
 

@@ -12,12 +12,13 @@
 
 namespace isb {
 
-int ssf_cold_chains(const isb_ctx *ctx, int npad);                            // ssf_cold.cu
-cudaError_t launch_ssf_cold(const SsfParams &p, int chains, cudaStream_t st);
+int ssf_cold_chains(const isb_ctx *ctx, int npad, bool fixed);                // ssf_cold.cu
+cudaError_t launch_ssf_cold(const SsfParams &p, int chains, bool fixed, cudaStream_t st);
 cudaError_t launch_ssf_dd(const SsfParams &p, int npl, bool list, bool tma, int cl, int grid, int threads,
                           size_t smem, cudaStream_t st);
 cudaError_t launch_ssf_ff(const SsfParams &p, int npl, bool list, bool tma, int cl, int grid, int threads,
                           size_t smem, cudaStream_t st);
+cudaError_t launch_ssf_ii(const SsfParams &p, int npl, int grid, int threads, cudaStream_t st);
 
 size_t ssf_field_elem_size(const isb_model *m) { return m->prec == ISB_PREC_F32 ? sizeof(float) : sizeof(double); }
 
@@ -51,6 +52,46 @@ __global__ void field_init_kernel(const double *__restrict__ J, const double *__
         v = hsign > 0 ? g + h[i] : g - h[i];
     }
     fields[(int64_t)r * npad + i] = (HT)v;
+}
+
+// Fixed-point fields F_i = sum_j Jint[i][j] s_j (no h: the decision adds it, csrc/ssf_kernel.cuh fixed_thresholds).
+// Integer sums do not depend on the order, so a CTA reads its columns of J once for FI_RB replicas: thread p owns position
+// p of the permuted rows (coalesced) and, J being symmetric, sums column p of Jint = row site(p).  sum over the spins
+// that are up, doubled, minus the plain sum: one predicated add per coupling and replica.
+constexpr int FI_RB = 16;
+__global__ void __launch_bounds__(256) fixed_field_init_kernel(const int32_t *__restrict__ Jfix, const int8_t *spins,
+                                                               int64_t lds, int32_t *fields, int npad, int R, int vec) {
+    extern __shared__ uint32_t up_bits[];   // [FI_RB][npad / 32]: bit j % 32 of word j / 32 = spin j of the replica is up
+    const int nw32 = npad >> 5, r0 = blockIdx.y * FI_RB;
+    for (int idx = threadIdx.x; idx < FI_RB * nw32; idx += blockDim.x) {
+        const int rr = r0 + idx / nw32, w = idx % nw32;
+        uint32_t b = 0;
+        if (rr < R)
+            for (int l = 0; l < 32; ++l) b |= (spins[(int64_t)rr * lds + w * 32 + l] > 0 ? 1u : 0u) << l;
+        up_bits[idx] = b;
+    }
+    __syncthreads();
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    int32_t up[FI_RB], all = 0;
+#pragma unroll
+    for (int r = 0; r < FI_RB; ++r) up[r] = 0;
+    for (int w = 0; w < nw32; ++w) {
+        uint32_t bw[FI_RB];
+#pragma unroll
+        for (int r = 0; r < FI_RB; ++r) bw[r] = up_bits[r * nw32 + w];
+#pragma unroll 4
+        for (int l = 0; l < 32; ++l) {
+            const int32_t v = __ldg(&Jfix[(int64_t)(w * 32 + l) * npad + p]);
+            all += v;
+#pragma unroll
+            for (int r = 0; r < FI_RB; ++r) up[r] += ((bw[r] >> l) & 1u) ? v : 0;
+        }
+    }
+    const int kv = p / (32 * vec), rm = p % (32 * vec);
+    const int site = (kv * vec + rm % vec) * 32 + rm / vec;   // inverse of the permutation of api.cu (isb_model_dense)
+#pragma unroll
+    for (int r = 0; r < FI_RB; ++r)
+        if (r0 + r < R) fields[(int64_t)(r0 + r) * npad + site] = 2 * up[r] - all;   // (wrap-around: exact in range)
 }
 
 __global__ void dense_field_kernel(const double *__restrict__ J, const double *__restrict__ h, const int8_t *spins,
@@ -237,6 +278,22 @@ int ssf_ensure_fields(isb_ens *e, int sign) {
     return ISB_OK;
 }
 
+// (Re)compute the cached fixed-point fields (they do not depend on h or the rule, and never drift).
+static int ssf_ensure_fixed_fields(isb_ens *e) {
+    isb_model *m = e->model;
+    isb_ctx *ctx = m->ctx;
+    if (!e->ifields) ISB_CUDA(ctx, cudaMalloc(&e->ifields, (size_t)e->R * m->npad * sizeof(int32_t)));
+    if (e->ifields_ok) return ISB_OK;
+    const int threads = std::min(m->npad, 256);
+    dim3 grid(m->npad / threads, (e->R + FI_RB - 1) / FI_RB);
+    fixed_field_init_kernel<<<grid, threads, FI_RB * (m->npad / 32) * sizeof(uint32_t), ctx->stream>>>(
+        m->Jfix, e->spins, e->lds, e->ifields, m->npad, e->R, std::min(4, m->npl));
+    ISB_CUDA(ctx, cudaGetLastError());
+    e->ifields_ok = true;
+    e->last_launches += 1;
+    return ISB_OK;
+}
+
 // ------------------------------------------------------------------ K1 launch
 int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_t *d_nodes, int start,
                    int fluct_mode, const double *d_fluct, uint64_t seed, uint64_t step_offset,
@@ -246,15 +303,26 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
     if (!m->fast_ok)
         return fail(ctx, ISB_ERR_UNSUPPORTED, "single-spin sweeps support N <= 1024 sites (N = %d)", m->n);
     if (nsteps <= 0) return ISB_OK;
-    int rc = ssf_ensure_fields(e, rule == ISB_RULE_HOPFIELD ? -1 : +1);
+    const bool list = order != ISB_ORDER_SEQUENTIAL;
+    // The fixed-point kernels (int32 couplings and fields, exact fallback at the decision boundary: DESIGN §3) take every
+    // untraced sequential run of a model that allows them; traces (energies compared at 1e-9) and the tie audit keep the
+    // Float64 kernels.  ISB_SSF_FIXED=0 forces the Float64 path (A/B runs).
+    bool fixed = m->fixed_ok && !list && trace_every == 0 && e->tie_eps == 0.0;
+    if (const char *env_fx = getenv("ISB_SSF_FIXED")) fixed = fixed && atoi(env_fx) != 0;
+    // a run on one path leaves the other path's cache stale
+    int rc = fixed ? ssf_ensure_fixed_fields(e) : ssf_ensure_fields(e, rule == ISB_RULE_HOPFIELD ? -1 : +1);
     if (rc) return rc;
+    if (fixed)
+        e->fields_rule_sign = 0;
+    else
+        e->ifields_ok = false;
 
     const bool hd = m->prec != ISB_PREC_F32;
     const bool jf = m->j_is_f32;
     const int npl = m->npl;
     const int jsize = jf ? 4 : 8;
     const int rowb = m->npad * jsize;
-    const int field_regs = npl * (hd ? 2 : 1);
+    const int field_regs = npl * (hd ? 2 : 1);   // (int32 fields are budgeted like Float64 ones: SsfCfg)
     const int max_chains = ssf_max_chains(field_regs);
 
     int ctas, nw;
@@ -277,6 +345,9 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
     NG = std::min(NG, 8);
     if (const char *env_ng = getenv("ISB_SSF_NG")) NG = std::max(1, std::min(NG, atoi(env_ng)));   // fewer ring slots = more L1 (A/B runs)
     if (NG < 2) tma = false;
+    // the fixed-point path has no streaming kernel: with 4 KiB rows the plain kernel (rows from L1 / L2) was faster than a
+    // TMA ring at every acceptance of the C2 anneal (38 % down to 0.1 %; profiles/ssf_fixed_ab_b200.json)
+    if (fixed) tma = false;
     const size_t smem = tma ? (size_t)NG * SSF_G * rowb + (size_t)(3 * NG + 2) * sizeof(uint64_t) + 16 : 0;
     // thread-block clusters: one multicast J-row stream per cluster of `cl` CTAs (L2 -> SM traffic / cl)
     int cl = 1;  // measured on B200: the per-SM ingest of the row stream is the limit, multicast does not lift it
@@ -288,12 +359,12 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
     if (cl > 1) ctas = (ctas + cl - 1) / cl * cl;  // padding CTAs own no chains but take part in the protocol
 
     SsfParams p{};
-    p.J = m->Jperm;
+    p.J = fixed ? (const void *)m->Jfix : m->Jperm;
     p.ldj = m->npad;
     p.hext = m->h64;
     p.spins = e->spins;
     p.lds = e->lds;
-    p.fields = e->fields;
+    p.fields = fixed ? (void *)e->ifields : e->fields;
     p.n = m->n;
     p.npad = m->npad;
     p.R = e->R;
@@ -316,6 +387,10 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
     p.ldS = m->n;
     p.flips = e->d_flips;
     p.near_ties = e->d_counters;
+    p.fallbacks = e->d_counters + 1;
+    p.fix_q = m->fix_q;
+    p.fix_invq = 1.0 / m->fix_q;   // (a power of two: exact)
+    p.fix_margin = m->fix_margin;
     p.tie_eps = e->tie_eps;
     p.nw = nw;
     p.NG = NG;
@@ -329,14 +404,14 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
     if (const char *env_od = getenv("ISB_SSF_OD_RATIO")) p.od_ratio = (float)atof(env_od);
 
     p.fluct_pitch = nsteps;
-    const bool list = order != ISB_ORDER_SEQUENTIAL;
     const int threads = 32 * (nw + 1);
     // one launch over the steps [t0, t0 + len) of the run: every per-step input is offset on the host, the kernel sees a
     // run of `len` steps (t0 is a multiple of steps_per_T and of trace_every, see below)
     // mode 2: streaming kernel (TMA ring); 1: plain kernel (rows on demand, fields in registers); 0: cold kernel (fields in
     // shared memory, 28 chains per SM: ssf_cold.cu)
-    const int cold_chains = (hd && !jf && !list && trace_every == 0 && p.guard == 0.0 && p.tie_eps == 0.0)
-                                ? ssf_cold_chains(ctx, m->npad) : 0;
+    const int cold_chains = fixed ? ssf_cold_chains(ctx, m->npad, true)
+                            : (hd && !jf && !list && trace_every == 0 && p.guard == 0.0 && p.tie_eps == 0.0)
+                                ? ssf_cold_chains(ctx, m->npad, false) : 0;
     auto launch = [&](int64_t t0, int64_t len, int mode) -> cudaError_t {
         const bool use_tma = mode == 2;
         SsfParams q = p;
@@ -355,8 +430,9 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
             if (d_M) q.out_M = d_M + i0 * e->R;
             if (d_S) q.out_S = d_S + i0 * e->R * (int64_t)m->n;
         }
-        if (mode == 0) return launch_ssf_cold(q, cold_chains, ctx->stream);
+        if (mode == 0) return launch_ssf_cold(q, cold_chains, fixed, ctx->stream);
         const size_t sm = use_tma ? smem : 0;
+        if (fixed) return launch_ssf_ii(q, npl, ctas, threads, ctx->stream);
         return hd ? launch_ssf_dd(q, npl, list, use_tma, use_tma ? cl : 1, ctas, threads, sm, ctx->stream)
                   : launch_ssf_ff(q, npl, list, use_tma, use_tma ? cl : 1, ctas, threads, sm, ctx->stream);
     };
@@ -384,12 +460,14 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
         min_work = 0.0;
     }
     seg = (seg + unit - 1) / unit * unit;
-    bool segment = tma && !list && cl == 1 && unit > 0 && nsteps > 2 * seg && (double)e->R * m->n >= min_work;
+    bool segment = (tma || fixed) && !list && cl == 1 && unit > 0 && nsteps > 2 * seg && (double)e->R * m->n >= min_work;
     if (const char *env_sg = getenv("ISB_SSF_SEGMENT")) segment = segment && atoi(env_sg) != 0;
-    double thr = 0.2;      // accepted flips per attempt above which the streaming kernel is the faster one
+    double thr = fixed ? 2.0 : 0.2;   // accepted flips per attempt above which the streaming kernel is the faster one
     if (const char *env_th = getenv("ISB_SSF_SEG_THR")) thr = atof(env_th);
     cudaError_t ce = cudaSuccess;
-    double thr_cold = 0.03;   // ... below which the shared-memory-field kernel is the fastest (one wave of 28 chains per SM)
+    // ... below which the shared-memory-field kernel is the fastest (one wave of 28 chains per SM).  Fixed point: the cold
+    // kernel overtakes the plain one between 7.7 % and 5.5 % acceptance (C2 profile, profiles/ssf_fixed_ab_b200.json)
+    double thr_cold = fixed ? 0.06 : 0.03;
     if (const char *env_tc = getenv("ISB_SSF_COLD_THR")) thr_cold = atof(env_tc);
     if (cold_chains < 16) thr_cold = -1.0;
     int forced = -1;          // ISB_SSF_MODE = 0 | 1 | 2: one launch of that kernel (A/B runs and tests)
@@ -405,7 +483,7 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
         e->last_launches += 1;
     } else {
         std::vector<unsigned long long> fl((size_t)e->R), tot((size_t)e->R, 0ull);
-        int mode = 2;
+        int mode = tma ? 2 : 1;
         int stable = 0;
         for (int64_t t0 = 0; t0 < nsteps && ce == cudaSuccess;) {
             const int64_t len = std::min(seg, nsteps - t0);

@@ -12,7 +12,8 @@
 //     fields stay bit-identical to ssf_kernel's and the launches of a segmented run can alternate freely;
 //   * one Philox4x32-10 block per lane serves 128 consecutive steps (the same words as philox_step_word_k).
 // ssf_run_device selects this kernel per segment (csrc/ssf.cu) when the previous segment's acceptance is low and the run
-// needs nothing the kernel leaves out: sequential order, Float64 fields and couplings, no traces, no near-tie guard or audit.
+// needs nothing the kernel leaves out: sequential order, no traces, no near-tie guard or audit; Float64 fields and
+// couplings, or (FIXED) the int32 fixed-point ones of the same run.
 #include <stdint.h>
 
 #include "common.cuh"
@@ -23,28 +24,35 @@ namespace isb {
 
 constexpr int SSF_COLD_CHAINS = 28;
 
+// FIXED: the fixed-point variant (int32 fields and couplings, decisions as in ssf_kernel's int32 instantiation: integer
+// thresholds, ssf_exact_field in between); the fields are packed by four, 4 KiB per chain at N = 1024.
+template <bool FIXED>
 __global__ void __launch_bounds__(32 * SSF_COLD_CHAINS, 1) ssf_cold_kernel(const SsfParams p) {
-    extern __shared__ double cold_smem[];
+    using FT = typename std::conditional<FIXED, int32_t, double>::type;
+    using FV = typename std::conditional<FIXED, int4, double2>::type;   // one 128-bit pack of fields / couplings
+    constexpr int PK = FIXED ? 4 : 2;
+    extern __shared__ __align__(16) unsigned char cold_smem[];
     constexpr uint32_t FULL = 0xffffffffu;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int r = blockIdx.x * p.nw + warp;
     if (warp >= p.nw || r >= p.R) return;
-    const int npad = p.npad, npl = npad >> 5;       // npl is even (the host checks it): field pairs (2c, 2c + 1)
-    double *F = cold_smem + (size_t)warp * npad;     // F[(k / 2) * 64 + lane * 2 + (k % 2)] = field of site k * 32 + lane
-    const double *Jg = reinterpret_cast<const double *>(p.J);
+    const int npad = p.npad, npl = npad >> 5;       // npl is a multiple of PK (the host checks it)
+    // F[(k / PK) * 32 PK + lane * PK + (k % PK)] = field of site k * 32 + lane (the permuted order of a J row)
+    FT *F = reinterpret_cast<FT *>(cold_smem) + (size_t)warp * npad;
+    const FT *Jg = reinterpret_cast<const FT *>(p.J);
     uint32_t sw = 0;
     {
-        const double *fr = reinterpret_cast<const double *>(p.fields) + (int64_t)r * npad;
+        const FT *fr = reinterpret_cast<const FT *>(p.fields) + (int64_t)r * npad;
         const int8_t *sr = p.spins + (int64_t)r * p.lds;
         for (int k = 0; k < npl; ++k) {
-            F[(k >> 1) * 64 + lane * 2 + (k & 1)] = fr[k * 32 + lane];
+            F[(k / PK) * (32 * PK) + lane * PK + (k % PK)] = fr[k * 32 + lane];
             sw |= (sr[k * 32 + lane] > 0 ? 1u : 0u) << k;
         }
     }
     const int rule = p.rule;
     const bool metro = rule == 2;
     const double tsc = p.tscale ? __ldg(&p.tscale[r]) : 1.0;
-    unsigned long long nflips = 0;
+    unsigned long long nflips = 0, nfall = 0;
     const uint64_t spT = (uint64_t)p.steps_per_T;
     uint64_t ti = 0, tr = 0;                         // t = ti * spT + tr
     int64_t cached_ti = -1;
@@ -101,44 +109,67 @@ __global__ void __launch_bounds__(32 * SSF_COLD_CHAINS, 1) ssf_cold_kernel(const
         }
         const double ftl = __dmul_rn(f, Tl);
         bool mybit = (sw >> k) & 1u;
-        const int kpos = (k >> 1) * 64 + lane * 2 + (k & 1);
-        double hk = F[kpos];                         // my own site's field; mirrors F[kpos] through the window
+        const int kpos = (k / PK) * (32 * PK) + lane * PK + (k % PK);
+        FT hk = F[kpos];                             // my own site's field; mirrors F[kpos] through the window
         uint32_t rem = __ballot_sync(FULL, mine);
+        auto fts = [&]() { return metro ? (mybit ? ftl : -ftl) : ftl; };
+        [[maybe_unused]] int flo = 0, fhi = 0;
+        if constexpr (FIXED)   // (my spin changes only when my turn in the window is over: fixed through the window)
+            fixed_thresholds(fts(), p.hsign * __ldg(&p.hext[k * 32 + lane]), p.fix_q, p.fix_invq, p.fix_margin, flo, fhi);
         while (true) {
-            const double fts = metro ? (mybit ? ftl : -ftl) : ftl;
-            const double x = __dsub_rn(2.0 * hk, fts);
-            const bool nb = !(x < 0.0);              // heaviside(0) = 1, src/SpinSystems.jl:163-171
+            bool nb;
+            if constexpr (FIXED) {
+                nb = hk >= fhi;
+                const bool near = !nb && hk >= flo && ((rem >> lane) & 1u);
+                const uint32_t nm = __ballot_sync(FULL, near);
+                if (nm) {   // rare: decide on the reference's fresh sequential row dot
+                    const double ex = ssf_exact_field(p.J64, p.ld64, p.hext, p.hsign, p.n, sw, k * 32 + lane, near);
+                    if (near) nb = !(__dsub_rn(2.0 * ex, fts()) < 0.0);
+                    nfall += __popc(nm);
+                }
+            } else {
+                nb = !(__dsub_rn(2.0 * hk, fts()) < 0.0);   // heaviside(0) = 1, src/SpinSystems.jl:163-171
+            }
             const uint32_t fm = __ballot_sync(FULL, nb != mybit) & rem;
             if (fm == 0) break;
             const int l0 = __ffs(fm) - 1;
             const uint32_t upto = (2u << l0) - 1u;   // lanes <= l0 (l0 == 31 -> all ones)
             const bool up = (__ballot_sync(FULL, nb) >> l0) & 1u;
-            const double d = up ? 2.0 : -2.0;
-            const double *row = Jg + (int64_t)(k * 32 + l0) * p.ldj;
+            const FT d = up ? (FT)2 : (FT)-2;
+            const FT *row = Jg + (int64_t)(k * 32 + l0) * p.ldj;
             hk += d * row[kpos];
-            // fields += d * J[row]: every lane owns the positions c * 64 + lane * 2 + {0, 1} of its chain's fields
-            // (four 128-bit row loads in flight per batch: the loop is a chain of L2 / L1 latencies otherwise)
-            const int nc = npl >> 1;
+            // fields += d * J[row]: every lane owns the positions c * 32 PK + lane * PK + {0 .. PK - 1} of its chain's
+            // fields (four 128-bit row loads in flight per batch: the loop is a chain of L2 / L1 latencies otherwise)
+            auto axpy = [&](FV &f, const FV &j) {
+                if constexpr (FIXED) {
+                    f.x += d * j.x;
+                    f.y += d * j.y;
+                    f.z += d * j.z;
+                    f.w += d * j.w;
+                } else {
+                    f.x += d * j.x;
+                    f.y += d * j.y;
+                }
+            };
+            const int nc = npl / PK;
             int c = 0;
             for (; c + 4 <= nc; c += 4) {
-                double2 jv[4], fv[4];
+                FV jv[4], fv[4];
 #pragma unroll
-                for (int u = 0; u < 4; ++u) jv[u] = __ldg(reinterpret_cast<const double2 *>(row + (c + u) * 64) + lane);
+                for (int u = 0; u < 4; ++u) jv[u] = __ldg(reinterpret_cast<const FV *>(row + (c + u) * (32 * PK)) + lane);
 #pragma unroll
-                for (int u = 0; u < 4; ++u) fv[u] = *(reinterpret_cast<double2 *>(F + (c + u) * 64) + lane);
+                for (int u = 0; u < 4; ++u) fv[u] = *(reinterpret_cast<FV *>(F + (c + u) * (32 * PK)) + lane);
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
-                    fv[u].x += d * jv[u].x;
-                    fv[u].y += d * jv[u].y;
-                    *(reinterpret_cast<double2 *>(F + (c + u) * 64) + lane) = fv[u];
+                    axpy(fv[u], jv[u]);
+                    *(reinterpret_cast<FV *>(F + (c + u) * (32 * PK)) + lane) = fv[u];
                 }
             }
             for (; c < nc; ++c) {
-                const double2 jv = __ldg(reinterpret_cast<const double2 *>(row + c * 64) + lane);
-                double2 *fp = reinterpret_cast<double2 *>(F + c * 64) + lane;
-                double2 fv = *fp;
-                fv.x += d * jv.x;
-                fv.y += d * jv.y;
+                const FV jv = __ldg(reinterpret_cast<const FV *>(row + c * (32 * PK)) + lane);
+                FV *fp = reinterpret_cast<FV *>(F + c * (32 * PK)) + lane;
+                FV fv = *fp;
+                axpy(fv, jv);
                 *fp = fv;
             }
             if (lane == l0) {
@@ -159,30 +190,34 @@ __global__ void __launch_bounds__(32 * SSF_COLD_CHAINS, 1) ssf_cold_kernel(const
         }
     }
     {
-        double *fr = reinterpret_cast<double *>(p.fields) + (int64_t)r * npad;
+        FT *fr = reinterpret_cast<FT *>(p.fields) + (int64_t)r * npad;
         int8_t *sr = p.spins + (int64_t)r * p.lds;
         for (int k = 0; k < npl; ++k) {
-            fr[k * 32 + lane] = F[(k >> 1) * 64 + lane * 2 + (k & 1)];
+            fr[k * 32 + lane] = F[(k / PK) * (32 * PK) + lane * PK + (k % PK)];
             if (k * 32 + lane < p.n) sr[k * 32 + lane] = ((sw >> k) & 1u) ? (int8_t)1 : (int8_t)-1;
         }
-        if (lane == 0) p.flips[r] = nflips;
+        if (lane == 0) {
+            p.flips[r] = nflips;
+            if (nfall) atomicAdd(p.fallbacks, nfall);
+        }
     }
 }
 
-// chains per CTA the shared memory holds for this model (0: the kernel does not apply)
-int ssf_cold_chains(const isb_ctx *ctx, int npad) {
-    if (npad % 64 != 0) return 0;
-    const size_t per_chain = (size_t)npad * sizeof(double);
+// chains per CTA the shared memory holds for this model (0: the kernel does not apply); fixed: the int32 variant
+int ssf_cold_chains(const isb_ctx *ctx, int npad, bool fixed) {
+    if (npad % (fixed ? 128 : 64) != 0) return 0;
+    const size_t per_chain = (size_t)npad * (fixed ? sizeof(int32_t) : sizeof(double));
     return (int)std::min<size_t>(SSF_COLD_CHAINS, (ctx->smem_optin - 1024) / per_chain);
 }
 
-cudaError_t launch_ssf_cold(const SsfParams &p, int chains, cudaStream_t st) {
+cudaError_t launch_ssf_cold(const SsfParams &p, int chains, bool fixed, cudaStream_t st) {
     SsfParams q = p;
     q.nw = chains;
-    const size_t smem = (size_t)chains * p.npad * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(ssf_cold_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = (size_t)chains * p.npad * (fixed ? sizeof(int32_t) : sizeof(double));
+    auto kern = fixed ? ssf_cold_kernel<true> : ssf_cold_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    ssf_cold_kernel<<<(p.R + chains - 1) / chains, 32 * chains, smem, st>>>(q);
+    kern<<<(p.R + chains - 1) / chains, 32 * chains, smem, st>>>(q);
     return cudaGetLastError();
 }
 

@@ -1,34 +1,38 @@
 // ssf_inst.cuh — instantiates ssf_kernel for one (field type, coupling type) pair; included by
-// ssf_inst_dd.cu (Float64 fields and couplings) / ssf_inst_ff.cu (float fields and couplings), compiled in parallel.
+// ssf_inst_dd.cu (Float64 fields and couplings) / ssf_inst_ff.cu (float fields and couplings) / ssf_inst_ii.cu (int32
+// fixed-point fields and couplings), compiled in parallel.
 #pragma once
 #include "ssf_kernel.cuh"
 
 namespace isb {
 
+template <typename K>
+static cudaError_t launch_kernel(K kern, int cluster, const SsfParams &p, int grid, int threads, size_t smem, cudaStream_t st) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    if (cluster > 1) {
+        cudaLaunchConfig_t cfg{};
+        cfg.gridDim = dim3((unsigned)grid);
+        cfg.blockDim = dim3((unsigned)threads);
+        cfg.dynamicSmemBytes = smem;
+        cfg.stream = st;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeClusterDimension;
+        attr[0].val.clusterDim.x = (unsigned)cluster;
+        attr[0].val.clusterDim.y = 1;
+        attr[0].val.clusterDim.z = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
+        return cudaLaunchKernelEx(&cfg, kern, p);
+    }
+    kern<<<grid, threads, smem, st>>>(p);
+    return cudaGetLastError();
+}
+
 template <typename HT, typename JT, int NPL>
 static cudaError_t launch_one(const SsfParams &p, bool list, bool tma, int cl, int grid, int threads, size_t smem,
                               cudaStream_t st) {
-    auto go = [&](auto kern, int cluster) -> cudaError_t {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        if (cluster > 1) {
-            cudaLaunchConfig_t cfg{};
-            cfg.gridDim = dim3((unsigned)grid);
-            cfg.blockDim = dim3((unsigned)threads);
-            cfg.dynamicSmemBytes = smem;
-            cfg.stream = st;
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeClusterDimension;
-            attr[0].val.clusterDim.x = (unsigned)cluster;
-            attr[0].val.clusterDim.y = 1;
-            attr[0].val.clusterDim.z = 1;
-            cfg.attrs = attr;
-            cfg.numAttrs = 1;
-            return cudaLaunchKernelEx(&cfg, kern, p);
-        }
-        kern<<<grid, threads, smem, st>>>(p);
-        return cudaGetLastError();
-    };
+    auto go = [&](auto kern, int cluster) { return launch_kernel(kern, cluster, p, grid, threads, smem, st); };
     if (tma && cl == 2)
         return list ? go(ssf_kernel<HT, JT, NPL, true, true, 2>, 2) : go(ssf_kernel<HT, JT, NPL, false, true, 2>, 2);
     if (tma && cl == 4)

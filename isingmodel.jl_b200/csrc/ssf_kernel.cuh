@@ -79,6 +79,12 @@ struct SsfParams {
     const double *J64;  // natural layout [npad][ld64]
     int64_t ld64;
     double hsign;       // +1: J s + h, -1: J s - h (Hopfield)
+    // Fixed-point instantiation (HT = JT = int32_t): p.J holds Jint = round(J / q), the cached fields are the exact
+    // integers F = Jint s (no h), and every decision the thresholds of fixed_thresholds cannot settle is taken on
+    // ssf_exact_field, the reference's own row dot.  fix_margin = M >= (e_max + dot rounding) / q, DESIGN §3.
+    double fix_q, fix_invq;
+    int fix_margin;
+    unsigned long long *fallbacks;  // decisions taken on ssf_exact_field (fixed-point kernels)
 };
 constexpr int SSF_EPOCH = 1024;        // steps per streamed epoch
 constexpr int SSF_EPOCH_OD = 8 * 1024;  // steps per on-demand epoch: chains re-synchronise 8x less often
@@ -91,7 +97,8 @@ __host__ __device__ constexpr int ssf_max_chains(int field_regs) {
 
 template <typename HT, int NPL>
 struct SsfCfg {
-    static constexpr int kFieldRegs = NPL * (int)sizeof(HT) / 4;
+    // (int32 fixed-point fields are budgeted like Float64 ones: their decision step and fallback need the registers)
+    static constexpr int kFieldRegs = NPL * (std::is_same<HT, int32_t>::value ? 2 : (int)sizeof(HT) / 4);
     static constexpr int kMaxChains = ssf_max_chains(kFieldRegs);
     static constexpr int kMaxThreads = 32 * (kMaxChains + 1);
 };
@@ -154,6 +161,31 @@ static __device__ __noinline__ double ssf_exact_field(const double *J64, int64_t
     return want ? __dadd_rn(acc, hsign * __ldg(hext + i)) : 0.0;
 }
 
+// Decision thresholds of the fixed-point kernels for one site and one window (fts = the site's f*T or (f*T)*s_i, hh =
+// hsign * h_i; both fixed through the window).  pred(F) is the reference's decision with the dot replaced by F * q
+// (exact: F is an integer below 2^30, q a power of two); it is monotone in F, so a = min{F in [-B, B] : pred(F)} splits
+// the integers.  The reference's own dot lies within M * q of F * q (DESIGN §3), hence
+//   F >= a + M  ->  the reference flips up,   F < a - M  ->  it flips down,   otherwise: ask ssf_exact_field.
+// With M = 0 (couplings that are exact multiples of q) lo == hi and nothing falls back.  a starts at ceil(t), t the
+// real-valued boundary, and is settled by evaluating pred itself; a boundary that does not settle in 8 steps (huge |h|
+// against q) sends every value to the exact path.
+__device__ __forceinline__ void fixed_thresholds(double fts, double hh, double q, double invq, int M, int &lo, int &hi) {
+    constexpr int B = (1 << 30) + 1;
+    auto pred = [&](int F) { return !(__dsub_rn(2.0 * __dadd_rn(__dmul_rn((double)F, q), hh), fts) < 0.0); };
+    const double t = ceil(__dmul_rn(__dsub_rn(0.5 * fts, hh), invq));
+    int a = !(t > (double)-B) ? -B : (t > (double)B ? B : (int)t);
+    int it = 0;
+    while (it < 8 && a > -B && pred(a - 1)) --a, ++it;
+    while (it < 8 && a < B && !pred(a)) ++a, ++it;
+    if (it >= 8) {
+        lo = -0x7fffffff - 1;
+        hi = 0x7fffffff;
+        return;
+    }
+    lo = a - M;   // |a| <= 2^30 + 1 and M <= 2^10 (model creation): no overflow
+    hi = a + M;
+}
+
 // CL > 1: the CTAs of a thread-block cluster (same GPC) walk the same row sequence, so the leader CTA's
 // producer issues each J row ONCE as a multicast bulk copy that lands in every CTA's ring (one L2 read for CL
 // SMs).  Followers arm their own full barriers and tell the leader (remote mbarrier arrive) when their slot is free.
@@ -162,6 +194,9 @@ static __device__ __noinline__ double ssf_exact_field(const double *J64, int64_t
 template <typename HT, typename JT, int NPL, bool LIST, bool TMA, int CL = 1, bool GUARD = false>
 __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(const SsfParams p) {
     static_assert(CL == 1 || TMA, "clusters only make sense with the TMA ring");
+    // int32 fields and couplings: the fixed-point path (sequential order, plain kernel, no traces, no tie audit; see SsfParams)
+    constexpr bool FIXED = std::is_same<HT, int32_t>::value;
+    static_assert(!FIXED || (std::is_same<JT, int32_t>::value && !LIST && !TMA && !GUARD), "fixed-point: plain sequential sweeps only");
     constexpr int G = SSF_G;
     constexpr int NPAD = NPL * 32;
     constexpr int ROWB = NPAD * (int)sizeof(JT);
@@ -305,7 +340,7 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
     // T_r = Tsched * tscale[r] (x 1.0 is exact); the factor is re-read whenever a schedule entry is fetched rather than
     // kept live: two more registers in the sweep loop cost 3 % on C2
 #define ISB_TSC() (p.tscale ? __ldg(&p.tscale[r]) : 1.0)
-    unsigned long long nflips = 0, nties = 0;
+    unsigned long long nflips = 0, nties = 0, nfall = 0;
     // Ring position of this chain within the current (streamed) epoch: qcur = group of the epoch being read
     // (-1: none yet), held = it has not been released; cslot / cph walk the ring across epochs (only streamed
     // groups are ever pushed, so producer and chains stay in step).  te = steps done in the current epoch.
@@ -468,7 +503,26 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
             HT hk = field_sel<HT, NPL>(hf, k);
             const int kpos = (k / VEC) * (32 * VEC) + lane * VEC + (k % VEC);
             uint32_t rem = __ballot_sync(FULL, mine);
+            [[maybe_unused]] int flo = 0, fhi = 0;
+            if constexpr (FIXED) {
+                const double fts = metro ? (mybit ? ftl : -ftl) : ftl;
+                fixed_thresholds(fts, p.hsign * __ldg(&p.hext[k * 32 + lane]), p.fix_q, p.fix_invq, p.fix_margin, flo, fhi);
+            }
             while (true) {
+                bool nb;
+                uint32_t fm;   // lanes still to decide whose decision flips their spin
+                if constexpr (FIXED) {
+                    nb = hk >= fhi;
+                    const bool near = !nb && hk >= flo && ((rem >> lane) & 1u);
+                    const uint32_t nm = __ballot_sync(FULL, near);
+                    if (nm) {   // rare: decide on the reference's fresh sequential row dot
+                        const double ex = ssf_exact_field(p.J64, p.ld64, p.hext, p.hsign, p.n, sw, k * 32 + lane, near);
+                        const double fts = metro ? (mybit ? ftl : -ftl) : ftl;
+                        if (near) nb = !(__dsub_rn(2.0 * ex, fts) < 0.0);
+                        nfall += __popc(nm);
+                    }
+                    fm = __ballot_sync(FULL, nb != mybit) & rem;
+                } else {
                 double h2 = 2.0 * (double)hk;
                 const double fts = metro ? (mybit ? ftl : -ftl) : ftl;
                 double x = __dsub_rn(h2, fts);
@@ -484,11 +538,12 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
                         field_set<HT, NPL>(hf, k, hk);
                     }
                 }
-                const bool nb = !(x < 0.0);  // heaviside(0) = 1, src/SpinSystems.jl:163-171
-                const uint32_t fm = __ballot_sync(FULL, nb != mybit) & rem;
+                nb = !(x < 0.0);  // heaviside(0) = 1, src/SpinSystems.jl:163-171
+                fm = __ballot_sync(FULL, nb != mybit) & rem;
                 if (audit) {
                     const uint32_t tm = __ballot_sync(FULL, fabs(x) < p.tie_eps) & rem;
                     nties += __popc(fm ? (tm & ((2u << (__ffs(fm) - 1)) - 1u)) : tm);
+                }
                 }
                 if (fm == 0) break;
                 const int l0 = __ffs(fm) - 1;
@@ -618,6 +673,7 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
         if (lane == 0) {
             p.flips[r] = nflips + ep_nflips;
             if (nties) atomicAdd(p.near_ties, nties);
+            if (nfall) atomicAdd(p.fallbacks, nfall);
         }
     }
     }  // consumer warp
