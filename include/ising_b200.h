@@ -141,6 +141,12 @@ int isb_ens_replicas(const isb_ens *e);
 /* An independent copy of the ensemble on the same model (spins, hidden layer, per-replica temperature factors; all
  * copied device to device): what `deepcopy(ss)` of the host object maps to (test/runtests.jl:22-24,30-31). */
 int isb_ens_clone(isb_ens *src, isb_ens **out);
+/* Replica r takes the state of replica src[r] (src: R entries in [0, R), repeats allowed).  The spins, the cached Float64 /
+ * float local fields and the fixed-point fields (whichever are valid) move with it, bit for bit.  A chain copied into slot
+ * r therefore continues from exactly the state it had.  Per-replica temperature factors and flip counters belong to the
+ * slot and do not move.  General-graph ensembles only (ISB_ERR_STATE for bipartite ones).  A src entry outside [0, R) is
+ * ISB_ERR_ARG and leaves the ensemble unchanged. */
+int isb_ens_select_replicas(isb_ens *e, const int32_t *src);
 /* spinConfiguration get/set: src/SpinSystems.jl:61-62,128-129 */
 int isb_ens_set_spins(isb_ens *e, const int8_t *s, int64_t ld);
 int isb_ens_get_spins(isb_ens *e, int8_t *s, int64_t ld);
@@ -219,6 +225,28 @@ int isb_ssf_run_pt(isb_ens *e, int rule, int n_levels, const double *levels, int
                    int order, int start, uint64_t seed, uint64_t step_offset, uint64_t round_offset,
                    int32_t *level_of, double *out_E, double *out_M, double *out_Q,
                    int64_t *out_accepted, int64_t *out_flips);
+
+/* Population annealing: R = n_pop * P replicas, population p = slots p*P .. p*P + P - 1 (P <= 2^20).  Temperature step k
+ * (absolute index K = T_offset + k) is exactly
+ *   isb_ssf_run(rule, steps_per_T, order, (start + k*steps_per_T) mod N, ISB_FLUCT_PHILOX, seed,
+ *               step_offset + k*steps_per_T, Tsched = {T[k]}, steps_per_T = trace_every = steps_per_T)
+ * followed, when k < nT - 1 or T_next > 0, by one resampling of every population towards T' = T[k+1] (or T_next):
+ *   db = 1/T' - 1/T[k];  a_r = -db * E_r;  x_r = exp(a_r - max_r a_r)      (IEEE round-to-nearest, no contraction)
+ *   W_r = floor(x_r * 2^32) (uint64),  C_r = W_0 + ... + W_r,  S = C_{P-1}        (exact integers)
+ *   U   = word .x of Philox4x32-10(counter (lo32(K), hi32(K), p, 6 << 28), key seed)
+ *   slot j of the population takes the state (isb_ens_select_replicas) of the smallest r with
+ *   C_r > floor((j * 2^32 + U) * S / (P * 2^32))                                (128-bit integer arithmetic)
+ *   lnQ[k][p] = max_r a_r + ln(sum_r x_r / P);  family[j] <- family[parent(j)]
+ * (r, j: indices within the population).  E_r is the energy the sweep kernel traced at the last step (isb_ssf_run's out_E).
+ *   rule: Glauber or Metropolis; order: sequential, random or checkerboard (lattices); T[k] > 0 and finite; T_next = 0: none.
+ *   out_E, out_M [nT][R] by slot (before that step's resampling); out_lnQ [nT - 1 + (T_next > 0)][n_pop];
+ *   family [R] in/out (any int32 labels, may be NULL); out_flips [R] per slot over the call.
+ * Every output may be NULL.  Two calls (T[0..a) with T_next = T[a], then T[a..b); start, step_offset and T_offset
+ * continued) equal one call of T[0..b) bit for bit.  Per-replica temperature factors must be unset (ISB_ERR_STATE).
+ * nT = 0 is a no-op. */
+int isb_ssf_run_pa(isb_ens *e, int rule, int n_pop, int64_t nT, const double *T, double T_next, int64_t steps_per_T,
+                   int order, int start, uint64_t seed, uint64_t step_offset, uint64_t T_offset, int32_t *family,
+                   double *out_E, double *out_M, double *out_lnQ, int64_t *out_flips);
 
 /* Fluctuations exactly as ISB_FLUCT_PHILOX generates them inside isb_ssf_run, for parity tests:
  * out[r*nsteps + k], r in [r0, r0+nr). rule selects the transform. prec as the model's. */

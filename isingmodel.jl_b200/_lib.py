@@ -70,6 +70,7 @@ SIGNATURES = {
     "isb_model_num_hidden": (_i, [_vp]),
     "isb_ens_create": (_i, [_vp, _i, C.POINTER(_vp)]),
     "isb_ens_clone": (_i, [_vp, C.POINTER(_vp)]),
+    "isb_ens_select_replicas": (_i, [_vp, _vp]),
     "isb_ens_destroy": (None, [_vp]),
     "isb_ens_replicas": (_i, [_vp]),
     "isb_ens_set_spins": (_i, [_vp, _vp, _i64]),
@@ -85,6 +86,7 @@ SIGNATURES = {
                               _i64]),
     "isb_ssf_run_hist": (_i, [_vp, _i, _i64, _i, _vp, _i, _i, _vp, _u64, _u64, _vp, _i64, _i64, _i64, _vp]),
     "isb_ssf_run_pt": (_i, [_vp, _i, _i, _vp, _i64, _i64, _i, _i, _u64, _u64, _u64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "isb_ssf_run_pa": (_i, [_vp, _i, _i, _i64, _vp, _d, _i64, _i, _i, _u64, _u64, _u64, _vp, _vp, _vp, _vp, _vp]),
     "isb_philox_fluct": (_i, [_vp, _i, _i, _u64, _u64, _i, _i, _i64, _vp]),
     "isb_philox_nodes": (_i, [_vp, _i, _u64, _u64, _i64, _vp]),
     "isb_philox_raw": (_i, [_vp, _vp, _vp, _i, _vp]),
@@ -553,6 +555,34 @@ class Ensemble:
                                         int(start), int(seed), int(step_offset), int(round_offset), ptr(lo), ptr(E),
                                         ptr(M), ptr(Q), ptr(acc), ptr(flips)))
         return {"level_of": lo, "E": E, "M": M, "Q": Q, "accepted": acc, "flips": flips}
+
+    def select_replicas(self, src):
+        """isb_ens_select_replicas: replica r takes the state (spins and cached fields, bit for bit) of replica src[r]."""
+        a = np.ascontiguousarray(src, dtype=np.int32).reshape(-1)
+        if a.size != self.R:
+            raise IsbError(ERR_SIZE, f"src has {a.size} entries for {self.R} replicas")
+        self._chk(load().isb_ens_select_replicas(self.handle, ptr(a)))
+
+    def ssf_run_pa(self, rule, n_pop, T, steps_per_T, *, T_next=0.0, order=ORDER_SEQUENTIAL, start=0, seed=0,
+                   step_offset=0, T_offset=0, family=None, want_E=True, want_M=False):
+        """isb_ssf_run_pa: population annealing over the temperatures T (``steps_per_T`` steps each), resampling every
+        population after each step towards the next temperature (after the last one towards ``T_next`` when > 0), all on
+        the device.  ``family`` (R int32 labels or None) follows the resampling.  Returns dict(E / M [nT][R] | None (by
+        slot, before that step's resampling), lnQ [nT - 1 + (T_next > 0)][n_pop], family[R] | None, flips[R])."""
+        Ta = np.ascontiguousarray(np.atleast_1d(T), dtype=np.float64).reshape(-1)
+        nT, n_pop = Ta.size, int(n_pop)
+        fam = None if family is None else np.array(family, dtype=np.int32).reshape(-1)
+        if fam is not None and fam.size != self.R:
+            raise IsbError(ERR_SIZE, f"family has {fam.size} entries for {self.R} replicas")
+        n_res = max(nT - 1 + (1 if T_next > 0 else 0), 0) if nT else 0
+        E = np.zeros((nT, self.R)) if want_E else None
+        M = np.zeros((nT, self.R)) if want_M else None
+        lnQ = np.zeros((n_res, max(n_pop, 0)))
+        flips = np.zeros(self.R, dtype=np.int64)
+        self._chk(load().isb_ssf_run_pa(self.handle, int(rule), n_pop, nT, ptr(Ta), float(T_next), int(steps_per_T),
+                                        int(order), int(start), int(seed), int(step_offset), int(T_offset), ptr(fam),
+                                        ptr(E), ptr(M), ptr(lnQ), ptr(flips)))
+        return {"E": E, "M": M, "lnQ": lnQ, "family": fam, "flips": flips}
 
     def bip_run(self, rule, nsteps, *, Fv=None, Fh=None, fluct_per_replica=False, seed=0, step_offset=0, T=None,
                 steps_per_T=1, trace_every=0, want_S=False):

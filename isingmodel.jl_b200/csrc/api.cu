@@ -625,6 +625,9 @@ void isb_ens_destroy(isb_ens *e) {
         cudaFree(e->hidden);
         cudaFree(e->fields);
         cudaFree(e->ifields);
+        cudaFree(e->spins2);
+        cudaFree(e->fields2);
+        cudaFree(e->ifields2);
         cudaFree(e->d_flips);
         cudaFree(e->d_counters);
         cudaFree(e->d_tscale);
@@ -1071,6 +1074,135 @@ int isb_ssf_run_pt(isb_ens *e, int rule, int n_levels, const double *levels, int
         for (int l = 0; l + 1 < L; ++l) out_accepted[l] = (int64_t)acc[l];
     e->last_near_ties = (int64_t)counters[0];
     e->last_exact_fallbacks = (int64_t)counters[1];
+    return ISB_OK;
+}
+
+int isb_ens_select_replicas(isb_ens *e, const int32_t *src) {
+    if (!e) return ISB_ERR_ARG;
+    isb_ctx *ctx = e->model->ctx;
+    ISB_LOCK(ctx);
+    const char *who = "isb_ens_select_replicas";
+    if (!general_graph(e->model)) return fail(ctx, ISB_ERR_STATE, "%s: not a general-graph ensemble", who);
+    if (!src) return fail(ctx, ISB_ERR_ARG, "%s: src is NULL", who);
+    for (int r = 0; r < e->R; ++r)
+        if (src[r] < 0 || src[r] >= e->R)
+            return fail(ctx, ISB_ERR_ARG, "%s: src[%d] = %d outside [0, %d)", who, r, src[r], e->R);
+    ISB_CUDA(ctx, cudaSetDevice(ctx->device));
+    begin_stats(e);
+    int32_t *d_src = nullptr;
+    ISB_TRY(isb::dev_reserve(ctx, isb::SCR_PA_STATE, (size_t)e->R * sizeof(int32_t), (void **)&d_src));
+    ISB_TRY(h2d(ctx, d_src, src, (size_t)e->R * sizeof(int32_t), &e->last_h2d));
+    ISB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    ISB_TRY(isb::ens_select_device(e, d_src));
+    ISB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
+    if (ce != cudaSuccess) return fail(ctx, ISB_ERR_CUDA, "%s: kernel failed: %s", who, cudaGetErrorString(ce));
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
+    e->last_ms = ms;
+    return ISB_OK;
+}
+
+int isb_ssf_run_pa(isb_ens *e, int rule, int n_pop, int64_t nT, const double *T, double T_next, int64_t steps_per_T,
+                   int order, int start, uint64_t seed, uint64_t step_offset, uint64_t T_offset, int32_t *family,
+                   double *out_E, double *out_M, double *out_lnQ, int64_t *out_flips) {
+    if (!e) return ISB_ERR_ARG;
+    isb_model *m = e->model;
+    isb_ctx *ctx = m->ctx;
+    ISB_LOCK(ctx);
+    const char *who = "isb_ssf_run_pa";
+    if (!general_graph(m)) return fail(ctx, ISB_ERR_STATE, "%s: not a general-graph ensemble", who);
+    if (rule != ISB_RULE_GLAUBER && rule != ISB_RULE_METROPOLIS)
+        return fail(ctx, ISB_ERR_ARG, "%s: rule %d has no temperature to anneal (Glauber or Metropolis only)", who, rule);
+    if (order < ISB_ORDER_SEQUENTIAL || order > ISB_ORDER_CHECKERBOARD || order == ISB_ORDER_LIST)
+        return fail(ctx, ISB_ERR_ARG, "%s: order %d is not sequential, random or checkerboard", who, order);
+    if (order == ISB_ORDER_CHECKERBOARD && !(m->kind == ISB_KIND_SPARSE || !m->fast_ok))
+        return fail(ctx, ISB_ERR_UNSUPPORTED, "%s: ISB_ORDER_CHECKERBOARD needs a periodic L x L lattice given as a sparse model", who);
+    if (e->d_tscale)
+        return fail(ctx, ISB_ERR_STATE, "%s: per-replica temperature factors are set (clear them first)", who);
+    if (n_pop < 1) return fail(ctx, ISB_ERR_ARG, "%s: n_pop = %d must be positive", who, n_pop);
+    if (e->R % n_pop != 0)
+        return fail(ctx, ISB_ERR_SIZE, "%s: R = %d replicas is not a multiple of n_pop = %d", who, e->R, n_pop);
+    const int P = e->R / n_pop;
+    if (P > (1 << 20)) return fail(ctx, ISB_ERR_UNSUPPORTED, "%s: population size %d > 2^20", who, P);
+    if (nT < 0) return fail(ctx, ISB_ERR_ARG, "%s: nT = %lld is negative", who, (long long)nT);
+    if (nT > 0 && !T) return fail(ctx, ISB_ERR_ARG, "%s: T is NULL", who);
+    if (!all_finite(T, (size_t)nT) || !std::isfinite(T_next))
+        return fail(ctx, ISB_ERR_NONFINITE, "%s: non-finite temperature", who);
+    for (int64_t k = 0; k < nT; ++k)
+        if (!(T[k] > 0.0)) return fail(ctx, ISB_ERR_ARG, "%s: T[%lld] = %g must be positive", who, (long long)k, T[k]);
+    if (T_next < 0.0) return fail(ctx, ISB_ERR_ARG, "%s: T_next = %g is negative (0: none)", who, T_next);
+    if (steps_per_T <= 0)
+        return fail(ctx, ISB_ERR_ARG, "%s: steps_per_T = %lld must be positive", who, (long long)steps_per_T);
+    if (order != ISB_ORDER_RANDOM && (start < 0 || start >= m->n))
+        return fail(ctx, ISB_ERR_ARG, "%s: start = %d outside [0, %d)", who, start, m->n);
+    ISB_CUDA(ctx, cudaSetDevice(ctx->device));
+    begin_stats(e);
+    if (nT == 0) {
+        if (out_flips) std::fill(out_flips, out_flips + e->R, (int64_t)0);
+        return ISB_OK;
+    }
+    const int64_t n_res = nT - 1 + (T_next > 0.0 ? 1 : 0);
+    std::vector<double> db((size_t)n_res);
+    for (int64_t k = 0; k < n_res; ++k) db[k] = 1.0 / (k + 1 < nT ? T[k + 1] : T_next) - 1.0 / T[k];
+
+    // device state of the call, 8-byte words: flip totals | C (CTA-local) | CTA sums of W | a | CTA maxima | CTA sums of
+    // x [R each] | population maxima [n_pop] | E [R] | lnQ [n_res][n_pop]; then int32: parent | family x 2 [R each]
+    const size_t R = (size_t)e->R, np = (size_t)n_pop;
+    const size_t words = 7 * R + np + (size_t)n_res * np;
+    char *st = nullptr;
+    ISB_TRY(isb::dev_reserve(ctx, isb::SCR_PA_STATE, 8 * words + 4 * 3 * R, (void **)&st));
+    isb::PaDevice d{};
+    d.flips_total = (unsigned long long *)st;
+    d.cloc = d.flips_total + R;
+    d.bW = d.cloc + R;
+    d.a = (double *)(d.bW + R);
+    d.bmax = d.a + R;
+    d.bx = d.bmax + R;
+    d.pmax = d.bx + R;
+    d.E = d.pmax + np;
+    d.lnQ = d.E + R;
+    d.parent = (int32_t *)(st + 8 * words);
+    if (family) {
+        d.fam[0] = d.parent + R;
+        d.fam[1] = d.fam[0] + R;
+    }
+    double *d_T = nullptr;
+    if (order == ISB_ORDER_RANDOM)
+        ISB_TRY(isb::dev_reserve(ctx, isb::SCR_NODES, (size_t)steps_per_T * sizeof(int32_t), (void **)&d.nodes));
+    ISB_TRY(isb::dev_reserve(ctx, isb::SCR_T, (size_t)nT * sizeof(double), (void **)&d_T));
+    d.T = d_T;
+    if (out_E) ISB_TRY(isb::dev_reserve(ctx, isb::SCR_E, (size_t)nT * R * sizeof(double), (void **)&d.recE));
+    if (out_M) ISB_TRY(isb::dev_reserve(ctx, isb::SCR_M, (size_t)nT * R * sizeof(double), (void **)&d.recM));
+    ISB_TRY(h2d(ctx, d_T, T, (size_t)nT * sizeof(double), &e->last_h2d));
+    if (family) ISB_TRY(h2d(ctx, d.fam[0], family, R * sizeof(int32_t), &e->last_h2d));
+    ISB_CUDA(ctx, cudaMemsetAsync(d.flips_total, 0, R * sizeof(unsigned long long), ctx->stream));
+    ISB_CUDA(ctx, cudaMemsetAsync(e->d_counters, 0, 4 * sizeof(unsigned long long), ctx->stream));
+
+    int fam_final = 0;
+    ISB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    ISB_TRY(isb::ssf_pa_run_device(e, rule, n_pop, nT, db.data(), n_res, steps_per_T, order, start, seed, step_offset,
+                                   T_offset, d, &fam_final));
+    ISB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+
+    std::vector<unsigned long long> ftot(R);
+    unsigned long long counters[4] = {0, 0, 0, 0};
+    ISB_TRY(d2h(ctx, ftot.data(), d.flips_total, R * sizeof(unsigned long long), &e->last_d2h));
+    ISB_TRY(d2h(ctx, counters, e->d_counters, sizeof counters, &e->last_d2h));
+    if (family) ISB_TRY(d2h(ctx, family, d.fam[fam_final], R * sizeof(int32_t), &e->last_d2h));
+    if (out_E) ISB_TRY(d2h(ctx, out_E, d.recE, (size_t)nT * R * sizeof(double), &e->last_d2h));
+    if (out_M) ISB_TRY(d2h(ctx, out_M, d.recM, (size_t)nT * R * sizeof(double), &e->last_d2h));
+    if (out_lnQ) ISB_TRY(d2h(ctx, out_lnQ, d.lnQ, (size_t)n_res * np * sizeof(double), &e->last_d2h));
+    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
+    if (ce != cudaSuccess) return fail(ctx, ISB_ERR_CUDA, "%s: kernel failed: %s", who, cudaGetErrorString(ce));
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
+    e->last_ms = ms;
+    for (size_t r = 0; r < R; ++r) {
+        e->last_flips += (int64_t)ftot[r];
+        if (out_flips) out_flips[r] = (int64_t)ftot[r];
+    }
+    e->last_near_ties = (int64_t)counters[0];
     return ISB_OK;
 }
 

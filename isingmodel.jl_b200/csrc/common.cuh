@@ -177,9 +177,12 @@ __host__ __device__ __forceinline__ uint32_t philox_pick(const Philox4 &p, uint3
 }
 
 // Stream domains (top 4 bits of counter word 3).
-enum : uint32_t { DOM_SSF_FLUCT = 1, DOM_SSF_NODES = 2, DOM_BIP_VISIBLE = 3, DOM_BIP_HIDDEN = 4, DOM_PT_SWAP = 5 };
+enum : uint32_t { DOM_SSF_FLUCT = 1, DOM_SSF_NODES = 2, DOM_BIP_VISIBLE = 3, DOM_BIP_HIDDEN = 4, DOM_PT_SWAP = 5,
+                  DOM_PA_RESAMPLE = 6 };
 // Replica-exchange decisions (isb_ssf_run_pt): word .x of counter (lo(K), hi(K), ladder, DOM_PT_SWAP<<28 | lo) decides the
 // swap of levels (lo, lo+1) in that ladder after absolute round K.
+// Population-annealing resampling (isb_ssf_run_pa): word .x of counter (lo(K), hi(K), population, DOM_PA_RESAMPLE<<28) is
+// the offset U of the systematic resampling of that population after absolute temperature step K.
 
 // Word assigned to step `step` of replica `replica` in a single-spin run:
 // counter = (lo(step>>2), hi(step>>2), replica, domain<<28), key = seed, word = step & 3.

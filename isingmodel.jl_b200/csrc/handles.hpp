@@ -22,7 +22,7 @@ struct isb_ctx {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    isb_devbuf scratch[17];      // grow-only device staging buffers (see isb::dev_reserve)
+    isb_devbuf scratch[18];      // grow-only device staging buffers (see isb::dev_reserve)
     // Every entry point that uses the stream, the events or the scratch buffers holds this lock for its whole
     // (synchronous) duration: calls on one context are serialised, different contexts run concurrently.
     std::recursive_mutex mtx;
@@ -83,6 +83,11 @@ struct isb_ens {
     int64_t steps_since_refresh = 0;
     int32_t *ifields = nullptr;  // fixed-point fields [R][npad] (exact integers Jint s; allocated by the first fixed-point run)
     bool ifields_ok = false;     // false: rebuilt from the spins by the next fixed-point run
+    // second set of the state buffers for isb_ens_select_replicas (gather into them, then swap the pointers); each is
+    // allocated by the first selection that moves it
+    int8_t *spins2 = nullptr;
+    void *fields2 = nullptr;
+    int32_t *ifields2 = nullptr;
     unsigned long long *d_flips = nullptr;   // [R]
     unsigned long long *d_counters = nullptr; // [0] near ties, [1] exact fallbacks of the fixed-point kernels
     double tie_eps = 0.0;
@@ -103,7 +108,7 @@ double ssf_guard_from(const double *absrowsum, const double *vals, size_t nvals,
 int dev_reserve(isb_ctx *ctx, int slot, size_t bytes, void **out);
 enum { SCR_NODES = 0, SCR_FLUCT = 1, SCR_T = 2, SCR_E = 3, SCR_M = 4, SCR_FLUCT2 = 5, SCR_OUT = 6, SCR_TMP = 7,
        SCR_TC0 = 8, SCR_TC1 = 9, SCR_S = 10, SCR_S2 = 11, SCR_HIST = 12, SCR_PT_STATE = 13, SCR_PT_E = 14, SCR_PT_M = 15,
-       SCR_PT_Q = 16 };
+       SCR_PT_Q = 16, SCR_PA_STATE = 17 };
 
 #define ISB_LOCK(ctx) std::lock_guard<std::recursive_mutex> isb_lock_guard_((ctx)->mtx)
 
@@ -155,6 +160,13 @@ int ssf_lattice_run_device(isb_ens *e, void *lat, int rule, int64_t nsteps, int 
                            uint64_t seed, uint64_t step_offset, const double *d_T, int64_t steps_per_T, int64_t trace_every,
                            double *d_E, double *d_M, int8_t *d_S);
 
+// tempering.cu: one traced Philox run of both device loops (parallel tempering and population annealing) on the dispatch
+// of isb_ssf_run: the site list of a random order, then the dense register-resident kernel for dense models up to 1024
+// sites or the neighbour-list kernel for everything else (which hands periodic lattices to the lattice kernels).  E / M
+// of the last step go to d_E / d_M [R] (steps_per_T = trace_every = nsteps).
+int ssf_traced_run_device(isb_ens *e, int rule, int64_t nsteps, int order, int32_t *d_nodes, int start, uint64_t seed,
+                          uint64_t step_offset, const double *d_T, double *d_E, double *d_M);
+
 // tempering.cu: `rounds` rounds of isb_ssf_run_pt on the context stream, no host synchronisation between rounds.  Round k
 // is one sweep launch of steps_per_round steps (traced E / M of its last step into d_Eround / d_Mround [R]), the overlap
 // kernel when d_recQ is given, then the exchange kernel (level_of, e->d_tscale, acceptance counts, flip totals, records).
@@ -162,6 +174,22 @@ int ssf_pt_run_device(isb_ens *e, int rule, int n_levels, const double *d_levels
                       int order, int start, uint64_t seed, uint64_t step_offset, uint64_t round_offset, int32_t *d_nodes,
                       const double *d_T, int32_t *d_level_of, double *d_Eround, double *d_Mround, double *d_recE,
                       double *d_recM, double *d_recQ, unsigned long long *d_accepted, unsigned long long *d_flips_total);
+
+// population.cu: isb_ens_select_replicas on the context stream (d_src: R device entries, checked by the caller), and the
+// temperature loop of isb_ssf_run_pa (buffers of PaDevice; db[k] = 1/T[k+1] - 1/T[k] per resampling, n_res of them).
+int ens_select_device(isb_ens *e, const int32_t *d_src);
+struct PaDevice {
+    const double *T;                        // [nT]
+    int32_t *nodes;                         // [steps_per_T] (random order)
+    double *recE, *recM;                    // [nT][R] records (NULL: recE -> E [R] only, no M)
+    double *E;                              // [R] energies of the step when recE is NULL
+    double *a, *bmax, *bx, *pmax, *lnQ;     // [R], [n_pop*nb] x 2, [n_pop], [n_res][n_pop]
+    unsigned long long *cloc, *bW, *flips_total;   // [R], [n_pop*nb], [R]
+    int32_t *parent, *fam[2];               // [R]; family ping-pong (NULL: no family)
+};
+int ssf_pa_run_device(isb_ens *e, int rule, int n_pop, int64_t nT, const double *db, int64_t n_res, int64_t steps_per_T,
+                      int order, int start, uint64_t seed, uint64_t step_offset, uint64_t T_offset, const PaDevice &d,
+                      int *fam_final);
 
 // bip_exact.cu
 int bip_run_exact_device(isb_ens *e, int rule, int64_t nsteps, int fluct_mode, const double *d_Fv,

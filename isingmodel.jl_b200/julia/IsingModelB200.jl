@@ -147,6 +147,28 @@ function ssf_run_pt!(e, rule, levels, rounds, steps_per_round, level_of::Vector{
                 _optr(flips, Int64)), context())
     level_of
 end
+# Replica r takes the state of replica src[r] (1-based on the Julia side, 0-based across the ABI), spins and cached
+# fields bit for bit (isb_ens_select_replicas).
+function select_replicas!(e, src)
+    s0 = Vector{Int32}(src .- 1)
+    check(ccall((:isb_ens_select_replicas, libisb), Cint, (Ens, Ptr{Int32}), e, s0), context())
+    e
+end
+# Population annealing with the temperature loop inside the library (isb_ssf_run_pa): R = n_pop * P replicas,
+# population p = replicas p*P+1 .. (p+1)*P.  `family` (Vector{Int32} labels or nothing) is updated in place.
+# E / M: R x nT (column-major == the ABI's [nT][R]), lnQ: n_pop x (nT - 1 + (T_next > 0)), flips: R.
+function ssf_run_pa!(e, rule, n_pop, T, steps_per_T; T_next = 0.0, order = ORDER_SEQUENTIAL, start = 1, seed = 0,
+                     step_offset = 0, T_offset = 0, family = nothing, E = nothing, M = nothing, lnQ = nothing,
+                     flips = nothing)
+    Tv = Vector{Float64}(T)
+    check(ccall((:isb_ssf_run_pa, libisb), Cint,
+                (Ens, Cint, Cint, Int64, Ptr{Float64}, Float64, Int64, Cint, Cint, UInt64, UInt64, UInt64, Ptr{Int32},
+                 Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}),
+                e, rule, n_pop, length(Tv), Tv, T_next, steps_per_T, order, start - 1, seed, step_offset, T_offset,
+                _optr(family, Int32), _optr(E, Float64), _optr(M, Float64), _optr(lnQ, Float64), _optr(flips, Int64)),
+          context())
+    family
+end
 # Fv / Fh: (units, steps) column-major == [steps][units].  With snapV / snapH (units x R x ntr Int8) the call is
 # isb_bip_run_snap.
 function bip_run!(e, rule, nsteps; Fv = nothing, Fh = nothing, per_replica = false, seed = 0, step_offset = 0,

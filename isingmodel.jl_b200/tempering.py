@@ -153,3 +153,76 @@ class DeviceParallelTempering:
         self.round += rounds
         self.ua.temperatureScale = self.levels[self.level].reshape(-1)
         return (out["E"], out["Q"]) if overlaps else out["E"]
+
+
+class PopulationAnnealing:
+    """Population annealing with the whole temperature loop on the device (isb_ssf_run_pa).  The replicas of ``ua``'s
+    spin system form ``populations`` independent populations of P = replicas / populations slots (population p = replicas
+    p*P .. p*P + P - 1).  After the sweeps at each temperature every population is resampled in proportion to
+    exp(-(1/T_next - 1/T) E), so that it stays an (approximately) equilibrium sample of the next temperature.
+
+    Bookkeeping kept across ``run`` calls, so that consecutive calls continue one anneal:
+      ``family``   [replicas] int32: the slot each replica's family started in (labels follow the resampling);
+      ``lnZ``      [populations]: ln Z(T_current) / Z(T_first), from ln Z_{k+1}/Z_k = ln <exp(-(1/T_{k+1} - 1/T_k) E)>;
+      ``lnZ_run``  [nT][populations]: ln Z(T[k]) / Z(T_first) at every temperature of the last run;
+      ``temperature`` the temperature the populations are at (the last one run, or ``next_temperature``);
+      ``offset`` / ``step``: the Philox step offset and the absolute temperature-step index of the next run.
+    The resampling draws from the library's counter RNG (``seed``), so the anneal is a pure function of the seed.
+    ``order``: "sequential", "random" or "checkerboard" (periodic lattices)."""
+
+    _ORDERS = {"sequential": _lib.ORDER_SEQUENTIAL, "random": _lib.ORDER_RANDOM, "checkerboard": _lib.ORDER_CHECKERBOARD}
+
+    def __init__(self, ua, *, populations=1, seed=0, order="sequential"):
+        self.ua, self.ss = ua, ua.spinSystem
+        R = self.ss.replicas
+        if populations < 1 or R % populations:
+            raise ValueError("the number of replicas must be a multiple of the number of populations")
+        if order not in self._ORDERS:
+            raise ValueError(f"order must be one of {sorted(self._ORDERS)}")
+        self.populations, self.P = int(populations), R // int(populations)
+        self.seed, self.order = int(seed), order
+        self.family = np.arange(R, dtype=np.int32)
+        self.lnZ = np.zeros(self.populations)
+        self.lnZ_run = np.zeros((0, self.populations))
+        self.temperature = None
+        self.offset = 0          # steps run so far (the Philox step offset of the next temperature step)
+        self.step = 0            # temperature steps run so far (the absolute index of the next one)
+        ua.temperatureScale = None    # every replica runs at the schedule's temperature
+
+    def run(self, temperatures, sweeps=1, *, next_temperature=None):
+        """``sweeps`` sweeps at each of ``temperatures``, each followed by a resampling towards the next temperature
+        (after the last one towards ``next_temperature``, if given).  Returns E[nT][populations][P]: the energy of every
+        slot at the end of the sweeps at each temperature, before that step's resampling."""
+        T = np.asarray(temperatures, dtype=np.float64).reshape(-1)
+        if T.size == 0:
+            return np.zeros((0, self.populations, self.P))
+        if self.temperature is not None and T[0] != self.temperature:
+            raise ValueError(f"the populations are at T = {self.temperature}, not T = {T[0]}: pass next_temperature "
+                             "to the previous run to continue at another temperature")
+        n = self.ss._host_spins.shape[1]
+        ens = self.ss._ensemble()
+        ens.set_temperature_scale(None)
+        self.ua.temperatureScale = None
+        Tn = 0.0 if next_temperature is None else float(next_temperature)
+        out = ens.ssf_run_pa(self.ua._rule, self.populations, T, sweeps * n, T_next=Tn, order=self._ORDERS[self.order],
+                             start=self.offset % n if self.order != "random" else 0, seed=self.seed,
+                             step_offset=self.offset, T_offset=self.step, family=self.family)
+        self.ss._dev_newer = True
+        self.family = out["family"]
+        path = self.lnZ + np.concatenate([np.zeros((1, self.populations)), np.cumsum(out["lnQ"], axis=0)])
+        self.lnZ_run = path[:T.size]
+        self.lnZ = path[-1]
+        self.temperature = T[-1] if next_temperature is None else Tn
+        self.offset += T.size * sweeps * n
+        self.step += T.size
+        return out["E"].reshape(T.size, self.populations, self.P)
+
+    def family_statistics(self):
+        """Per population: the number of surviving families, rho_t = P * sum(nu^2) and the family entropy
+        -sum(nu ln nu), where nu is the fraction of the population that descends from one initial replica."""
+        fams, rho, ent = (np.zeros(self.populations, dtype=np.int64), np.zeros(self.populations),
+                          np.zeros(self.populations))
+        for p, labels in enumerate(self.family.reshape(self.populations, self.P)):
+            nu = np.unique(labels, return_counts=True)[1] / self.P
+            fams[p], rho[p], ent[p] = nu.size, self.P * float((nu * nu).sum()), float(-(nu * np.log(nu)).sum())
+        return {"families": fams, "rho_t": rho, "entropy": ent}
