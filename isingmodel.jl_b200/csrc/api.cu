@@ -266,10 +266,7 @@ static bool fixed_point_couplings(const std::vector<double> &Jn, const std::vect
     const int vec = std::min(4, npad / 32);
     Jq->assign((size_t)npad * npad, 0);
     for (int i = 0; i < n; ++i)
-        for (int s = 0; s < n; ++s) {
-            const int kk = s >> 5, lane = s & 31;
-            (*Jq)[(size_t)i * npad + (size_t)(kk / vec) * (32 * vec) + lane * vec + (kk % vec)] = (int32_t)Ji[(size_t)i * n + s];
-        }
+        for (int s = 0; s < n; ++s) (*Jq)[(size_t)i * npad + isb::ssf_perm_pos(s, vec)] = (int32_t)Ji[(size_t)i * n + s];
     *q_out = q;
     *M_out = (int)Md;
     return true;
@@ -353,14 +350,13 @@ int isb_model_dense(isb_ctx *ctx, int n, const double *J, int64_t ld, const doub
         cudaMemcpyAsync(m->J64, Jn.data(), nn * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
         cudaMemcpyAsync(m->h64, hn.data(), npad * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
         if (fast) {
-            // permuted copy for the sweep kernel: site k*32+lane -> position (k/VEC)*32*VEC + lane*VEC + k%VEC
+            // permuted copy for the sweep kernel (isb::ssf_perm_pos)
             const int jsz = m->j_is_f32 ? 4 : 8;
             const int vec = std::min(16 / jsz, npl);
             std::vector<unsigned char> Jp(nn * jsz);
             for (int i = 0; i < npad; ++i)
                 for (int s = 0; s < npad; ++s) {
-                    const int k = s >> 5, lane = s & 31;
-                    const size_t pos = (size_t)i * npad + (size_t)(k / vec) * (32 * vec) + lane * vec + (k % vec);
+                    const size_t pos = (size_t)i * npad + isb::ssf_perm_pos(s, vec);
                     const double v = Jn[(size_t)i * npad + s];
                     if (m->j_is_f32)
                         reinterpret_cast<float *>(Jp.data())[pos] = (float)v;
@@ -811,6 +807,51 @@ static void begin_stats(isb_ens *e) {
     e->last_flips = e->last_near_ties = e->last_exact_fallbacks = 0;
 }
 
+// The end of a timed run, once ev1 follows its work and the copies of its results are queued: waits for them, reports a
+// failed kernel, and puts the time from ev0 to ev1 into last_ms.
+static int finish_run(isb_ens *e, const char *who) {
+    isb_ctx *ctx = e->model->ctx;
+    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
+    if (ce != cudaSuccess) return fail(ctx, ISB_ERR_CUDA, "%s: kernel failed: %s", who, cudaGetErrorString(ce));
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
+    e->last_ms = ms;
+    return ISB_OK;
+}
+
+// finish_run of a single-spin run, which also reads back its flip counts per replica (d_flips [R]: into last_flips, and
+// into out_flips when given) and its near-tie and exact-fallback counters.
+static int finish_ssf_run(isb_ens *e, const char *who, const unsigned long long *d_flips, int64_t *out_flips) {
+    isb_ctx *ctx = e->model->ctx;
+    std::vector<unsigned long long> fl((size_t)e->R);
+    unsigned long long counters[4] = {0, 0, 0, 0};
+    ISB_TRY(d2h(ctx, fl.data(), d_flips, fl.size() * sizeof(unsigned long long), &e->last_d2h));
+    ISB_TRY(d2h(ctx, counters, e->d_counters, sizeof counters, &e->last_d2h));
+    ISB_TRY(finish_run(e, who));
+    for (int r = 0; r < e->R; ++r) {
+        e->last_flips += (int64_t)fl[r];
+        if (out_flips) out_flips[r] = (int64_t)fl[r];
+    }
+    e->last_near_ties = (int64_t)counters[0];
+    e->last_exact_fallbacks = (int64_t)counters[1];
+    return ISB_OK;
+}
+
+// The checks every single-spin entry point shares: a general-graph ensemble, a known order (ISB_ORDER_CHECKERBOARD only on
+// a periodic lattice) and, for the orders that walk the sites from `start`, start in [0, n).
+static int check_ssf_run(isb_ens *e, const char *who, int order, int start) {
+    const isb_model *m = e->model;
+    isb_ctx *ctx = m->ctx;
+    if (!general_graph(m)) return fail(ctx, ISB_ERR_STATE, "%s: not a general-graph ensemble", who);
+    if (order < ISB_ORDER_SEQUENTIAL || order > ISB_ORDER_CHECKERBOARD) return fail(ctx, ISB_ERR_ARG, "%s: unknown order %d", who, order);
+    if (order == ISB_ORDER_CHECKERBOARD && !isb::sparse_model_lattice(m))
+        return fail(ctx, ISB_ERR_UNSUPPORTED,
+                    "%s: ISB_ORDER_CHECKERBOARD needs a periodic L x L lattice (L a multiple of 32) with four neighbours per site", who);
+    if ((order == ISB_ORDER_SEQUENTIAL || order == ISB_ORDER_CHECKERBOARD) && (start < 0 || start >= m->n))
+        return fail(ctx, ISB_ERR_ARG, "%s: start = %d outside [0, %d)", who, start, m->n);
+    return ISB_OK;
+}
+
 static int ssf_run_impl(isb_ens *e, int rule, int64_t nsteps, int order, const int32_t *nodes, int start, int fluct_mode,
                         const double *fluct, uint64_t seed, uint64_t step_offset, const double *Tsched, int64_t nT,
                         int64_t steps_per_T, int64_t trace_every, double *out_E, double *out_M, int64_t *out_flips,
@@ -854,12 +895,9 @@ static int ssf_run_impl(isb_ens *e, int rule, int64_t nsteps, int order, const i
     isb_ctx *ctx = m->ctx;
     ISB_LOCK(ctx);
     const char *who = "isb_ssf_run";
-    if (!general_graph(m)) return fail(ctx, ISB_ERR_STATE, "%s: not a general-graph ensemble", who);
+    ISB_TRY(check_ssf_run(e, who, order, start));
     if (rule < ISB_RULE_HOPFIELD || rule > ISB_RULE_METROPOLIS) return fail(ctx, ISB_ERR_ARG, "%s: unknown rule %d", who, rule);
     if (nsteps < 0) return fail(ctx, ISB_ERR_ARG, "%s: nsteps = %lld is negative", who, (long long)nsteps);
-    if (order < ISB_ORDER_SEQUENTIAL || order > ISB_ORDER_CHECKERBOARD) return fail(ctx, ISB_ERR_ARG, "%s: unknown order %d", who, order);
-    if (order == ISB_ORDER_CHECKERBOARD && !(m->kind == ISB_KIND_SPARSE || !m->fast_ok))
-        return fail(ctx, ISB_ERR_UNSUPPORTED, "%s: ISB_ORDER_CHECKERBOARD needs a periodic L x L lattice given as a sparse model", who);
     if (fluct_mode < ISB_FLUCT_PHILOX || fluct_mode > ISB_FLUCT_PER_REPLICA)
         return fail(ctx, ISB_ERR_ARG, "%s: unknown fluct_mode %d", who, fluct_mode);
     if (trace_every < 0) return fail(ctx, ISB_ERR_ARG, "%s: trace_every is negative", who);
@@ -871,8 +909,6 @@ static int ssf_run_impl(isb_ens *e, int rule, int64_t nsteps, int order, const i
         for (int64_t k = 0; k < nsteps; ++k)
             if (nodes[k] < 0 || nodes[k] >= m->n)
                 return fail(ctx, ISB_ERR_ARG, "%s: nodes[%lld] = %d outside [0, %d)", who, (long long)k, nodes[k], m->n);
-    } else if (order == ISB_ORDER_SEQUENTIAL || order == ISB_ORDER_CHECKERBOARD) {
-        if (start < 0 || start >= m->n) return fail(ctx, ISB_ERR_ARG, "%s: start = %d outside [0, %d)", who, start, m->n);
     }
     if (fluct_mode != ISB_FLUCT_PHILOX) {
         if (!fluct && nsteps > 0) return fail(ctx, ISB_ERR_ARG, "%s: fluctuation array is NULL", who);
@@ -921,31 +957,19 @@ static int ssf_run_impl(isb_ens *e, int rule, int64_t nsteps, int order, const i
     ISB_CUDA(ctx, cudaMemsetAsync(e->d_counters, 0, 4 * sizeof(unsigned long long), ctx->stream));
 
     ISB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    if (order == ISB_ORDER_RANDOM) {
-        ISB_TRY(isb::philox_nodes_device(ctx, m->n, seed, step_offset, nsteps, d_nodes));
-        e->last_launches += 1;
-    }
-    if (m->kind == ISB_KIND_SPARSE || !m->fast_ok)
-        ISB_TRY(isb::ssf_sparse_run_device(e, rule, nsteps, order, d_nodes, start, fluct_mode, d_fluct, seed, step_offset,
-                                           d_T, steps_per_T, (d_E || d_M || d_S) ? trace_every : 0, d_E, d_M, d_S));
-    else
-        ISB_TRY(isb::ssf_run_device(e, rule, nsteps, order, d_nodes, start, fluct_mode, d_fluct, seed, step_offset, d_T,
-                                    steps_per_T, (d_E || d_M || d_S) ? trace_every : 0, d_E, d_M, d_S));
+    ISB_TRY(isb::ssf_sweep_device(e, rule, nsteps, order, d_nodes, start, fluct_mode, d_fluct, seed, step_offset, d_T,
+                                  steps_per_T, (d_E || d_M || d_S) ? trace_every : 0, d_E, d_M, d_S));
     if (d_hist) {
         ISB_TRY(isb::config_histogram_device(ctx, d_S, ntr * e->R, m->n, d_hist));
         e->last_launches += 1;
     }
     ISB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
 
-    std::vector<unsigned long long> fl((size_t)e->R);
     std::vector<unsigned long long> hh;
     if (d_hist) {
         hh.resize((size_t)1 << m->n);
         ISB_TRY(d2h(ctx, hh.data(), d_hist, hh.size() * sizeof(unsigned long long), &e->last_d2h));
     }
-    unsigned long long counters[4] = {0, 0, 0, 0};
-    ISB_TRY(d2h(ctx, fl.data(), e->d_flips, (size_t)e->R * sizeof(unsigned long long), &e->last_d2h));
-    ISB_TRY(d2h(ctx, counters, e->d_counters, sizeof counters, &e->last_d2h));
     if (d_E) ISB_TRY(d2h(ctx, out_E, d_E, (size_t)ntr * e->R * sizeof(double), &e->last_d2h));
     if (d_M) ISB_TRY(d2h(ctx, out_M, d_M, (size_t)ntr * e->R * sizeof(double), &e->last_d2h));
     if (d_S && out_S) {
@@ -953,17 +977,7 @@ static int ssf_run_impl(isb_ens *e, int rule, int64_t nsteps, int order, const i
                                         cudaMemcpyDeviceToHost, ctx->stream));
         e->last_d2h += (int64_t)ntr * e->R * m->n;
     }
-    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
-    if (ce != cudaSuccess) return fail(ctx, ISB_ERR_CUDA, "%s: kernel failed: %s", who, cudaGetErrorString(ce));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-    e->last_ms = ms;
-    for (int r = 0; r < e->R; ++r) {
-        e->last_flips += (int64_t)fl[r];
-        if (out_flips) out_flips[r] = (int64_t)fl[r];
-    }
-    e->last_near_ties = (int64_t)counters[0];
-    e->last_exact_fallbacks = (int64_t)counters[1];
+    ISB_TRY(finish_ssf_run(e, who, e->d_flips, out_flips));
     for (size_t b = 0; b < hh.size(); ++b) hist[b] += (int64_t)hh[b];
     return ISB_OK;
 }
@@ -976,13 +990,10 @@ int isb_ssf_run_pt(isb_ens *e, int rule, int n_levels, const double *levels, int
     isb_ctx *ctx = m->ctx;
     ISB_LOCK(ctx);
     const char *who = "isb_ssf_run_pt";
-    if (!general_graph(m)) return fail(ctx, ISB_ERR_STATE, "%s: not a general-graph ensemble", who);
+    ISB_TRY(check_ssf_run(e, who, order, start));
     if (rule != ISB_RULE_GLAUBER && rule != ISB_RULE_METROPOLIS)
         return fail(ctx, ISB_ERR_ARG, "%s: rule %d has no temperature to exchange (Glauber or Metropolis only)", who, rule);
-    if (order < ISB_ORDER_SEQUENTIAL || order > ISB_ORDER_CHECKERBOARD || order == ISB_ORDER_LIST)
-        return fail(ctx, ISB_ERR_ARG, "%s: order %d is not sequential, random or checkerboard", who, order);
-    if (order == ISB_ORDER_CHECKERBOARD && !(m->kind == ISB_KIND_SPARSE || !m->fast_ok))
-        return fail(ctx, ISB_ERR_UNSUPPORTED, "%s: ISB_ORDER_CHECKERBOARD needs a periodic L x L lattice given as a sparse model", who);
+    if (order == ISB_ORDER_LIST) return fail(ctx, ISB_ERR_ARG, "%s: order %d is not sequential, random or checkerboard", who, order);
     if (n_levels < 1) return fail(ctx, ISB_ERR_ARG, "%s: n_levels = %d must be positive", who, n_levels);
     if (n_levels > 1024) return fail(ctx, ISB_ERR_UNSUPPORTED, "%s: n_levels = %d > 1024", who, n_levels);
     if (e->R % n_levels != 0)
@@ -1008,8 +1019,6 @@ int isb_ssf_run_pt(isb_ens *e, int rule, int n_levels, const double *levels, int
     if (steps_per_round <= 0)
         return fail(ctx, ISB_ERR_ARG, "%s: steps_per_round = %lld must be positive", who, (long long)steps_per_round);
     if (rounds < 0) return fail(ctx, ISB_ERR_ARG, "%s: rounds = %lld is negative", who, (long long)rounds);
-    if (order != ISB_ORDER_RANDOM && (start < 0 || start >= m->n))
-        return fail(ctx, ISB_ERR_ARG, "%s: start = %d outside [0, %d)", who, start, m->n);
     ISB_CUDA(ctx, cudaSetDevice(ctx->device));
     begin_stats(e);
     if (out_accepted) std::fill(out_accepted, out_accepted + (L - 1), (int64_t)0);
@@ -1052,28 +1061,15 @@ int isb_ssf_run_pt(isb_ens *e, int rule, int n_levels, const double *levels, int
                                    round_offset, d_nodes, d_T, d_level_of, d_Er, d_Mr, d_recE, d_recM, d_recQ, d_acc, d_ftot));
     ISB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
 
-    std::vector<unsigned long long> acc((size_t)L), ftot(R);
-    unsigned long long counters[4] = {0, 0, 0, 0};
+    std::vector<unsigned long long> acc((size_t)L);
     ISB_TRY(d2h(ctx, level_of, d_level_of, R * sizeof(int32_t), &e->last_d2h));
     ISB_TRY(d2h(ctx, acc.data(), d_acc, (size_t)L * sizeof(unsigned long long), &e->last_d2h));
-    ISB_TRY(d2h(ctx, ftot.data(), d_ftot, R * sizeof(unsigned long long), &e->last_d2h));
-    ISB_TRY(d2h(ctx, counters, e->d_counters, sizeof counters, &e->last_d2h));
     if (d_recE) ISB_TRY(d2h(ctx, out_E, d_recE, (size_t)rounds * R * sizeof(double), &e->last_d2h));
     if (d_recM) ISB_TRY(d2h(ctx, out_M, d_recM, (size_t)rounds * R * sizeof(double), &e->last_d2h));
     if (d_recQ) ISB_TRY(d2h(ctx, out_Q, d_recQ, (size_t)rounds * L * (G / 2) * sizeof(double), &e->last_d2h));
-    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
-    if (ce != cudaSuccess) return fail(ctx, ISB_ERR_CUDA, "%s: kernel failed: %s", who, cudaGetErrorString(ce));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-    e->last_ms = ms;
-    for (size_t r = 0; r < R; ++r) {
-        e->last_flips += (int64_t)ftot[r];
-        if (out_flips) out_flips[r] = (int64_t)ftot[r];
-    }
+    ISB_TRY(finish_ssf_run(e, who, d_ftot, out_flips));
     if (out_accepted)
         for (int l = 0; l + 1 < L; ++l) out_accepted[l] = (int64_t)acc[l];
-    e->last_near_ties = (int64_t)counters[0];
-    e->last_exact_fallbacks = (int64_t)counters[1];
     return ISB_OK;
 }
 
@@ -1095,12 +1091,7 @@ int isb_ens_select_replicas(isb_ens *e, const int32_t *src) {
     ISB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     ISB_TRY(isb::ens_select_device(e, d_src));
     ISB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
-    if (ce != cudaSuccess) return fail(ctx, ISB_ERR_CUDA, "%s: kernel failed: %s", who, cudaGetErrorString(ce));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-    e->last_ms = ms;
-    return ISB_OK;
+    return finish_run(e, who);
 }
 
 int isb_ssf_run_pa(isb_ens *e, int rule, int n_pop, int64_t nT, const double *T, double T_next, int64_t steps_per_T,
@@ -1111,13 +1102,10 @@ int isb_ssf_run_pa(isb_ens *e, int rule, int n_pop, int64_t nT, const double *T,
     isb_ctx *ctx = m->ctx;
     ISB_LOCK(ctx);
     const char *who = "isb_ssf_run_pa";
-    if (!general_graph(m)) return fail(ctx, ISB_ERR_STATE, "%s: not a general-graph ensemble", who);
+    ISB_TRY(check_ssf_run(e, who, order, start));
     if (rule != ISB_RULE_GLAUBER && rule != ISB_RULE_METROPOLIS)
         return fail(ctx, ISB_ERR_ARG, "%s: rule %d has no temperature to anneal (Glauber or Metropolis only)", who, rule);
-    if (order < ISB_ORDER_SEQUENTIAL || order > ISB_ORDER_CHECKERBOARD || order == ISB_ORDER_LIST)
-        return fail(ctx, ISB_ERR_ARG, "%s: order %d is not sequential, random or checkerboard", who, order);
-    if (order == ISB_ORDER_CHECKERBOARD && !(m->kind == ISB_KIND_SPARSE || !m->fast_ok))
-        return fail(ctx, ISB_ERR_UNSUPPORTED, "%s: ISB_ORDER_CHECKERBOARD needs a periodic L x L lattice given as a sparse model", who);
+    if (order == ISB_ORDER_LIST) return fail(ctx, ISB_ERR_ARG, "%s: order %d is not sequential, random or checkerboard", who, order);
     if (e->d_tscale)
         return fail(ctx, ISB_ERR_STATE, "%s: per-replica temperature factors are set (clear them first)", who);
     if (n_pop < 1) return fail(ctx, ISB_ERR_ARG, "%s: n_pop = %d must be positive", who, n_pop);
@@ -1134,8 +1122,6 @@ int isb_ssf_run_pa(isb_ens *e, int rule, int n_pop, int64_t nT, const double *T,
     if (T_next < 0.0) return fail(ctx, ISB_ERR_ARG, "%s: T_next = %g is negative (0: none)", who, T_next);
     if (steps_per_T <= 0)
         return fail(ctx, ISB_ERR_ARG, "%s: steps_per_T = %lld must be positive", who, (long long)steps_per_T);
-    if (order != ISB_ORDER_RANDOM && (start < 0 || start >= m->n))
-        return fail(ctx, ISB_ERR_ARG, "%s: start = %d outside [0, %d)", who, start, m->n);
     ISB_CUDA(ctx, cudaSetDevice(ctx->device));
     begin_stats(e);
     if (nT == 0) {
@@ -1185,25 +1171,11 @@ int isb_ssf_run_pa(isb_ens *e, int rule, int n_pop, int64_t nT, const double *T,
                                    T_offset, d, &fam_final));
     ISB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
 
-    std::vector<unsigned long long> ftot(R);
-    unsigned long long counters[4] = {0, 0, 0, 0};
-    ISB_TRY(d2h(ctx, ftot.data(), d.flips_total, R * sizeof(unsigned long long), &e->last_d2h));
-    ISB_TRY(d2h(ctx, counters, e->d_counters, sizeof counters, &e->last_d2h));
     if (family) ISB_TRY(d2h(ctx, family, d.fam[fam_final], R * sizeof(int32_t), &e->last_d2h));
     if (out_E) ISB_TRY(d2h(ctx, out_E, d.recE, (size_t)nT * R * sizeof(double), &e->last_d2h));
     if (out_M) ISB_TRY(d2h(ctx, out_M, d.recM, (size_t)nT * R * sizeof(double), &e->last_d2h));
     if (out_lnQ) ISB_TRY(d2h(ctx, out_lnQ, d.lnQ, (size_t)n_res * np * sizeof(double), &e->last_d2h));
-    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
-    if (ce != cudaSuccess) return fail(ctx, ISB_ERR_CUDA, "%s: kernel failed: %s", who, cudaGetErrorString(ce));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-    e->last_ms = ms;
-    for (size_t r = 0; r < R; ++r) {
-        e->last_flips += (int64_t)ftot[r];
-        if (out_flips) out_flips[r] = (int64_t)ftot[r];
-    }
-    e->last_near_ties = (int64_t)counters[0];
-    return ISB_OK;
+    return finish_ssf_run(e, who, d.flips_total, out_flips);
 }
 
 int isb_philox_fluct(isb_ctx *ctx, int rule, int prec, uint64_t seed, uint64_t step_offset, int r0, int nr,
@@ -1317,12 +1289,7 @@ int isb_bip_run_snap(isb_ens *e, int rule, int64_t nsteps, int fluct_mode, const
                                         cudaMemcpyDeviceToHost, ctx->stream));
         e->last_d2h += ntr * e->R * m->nh;
     }
-    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
-    if (ce != cudaSuccess) return fail(ctx, ISB_ERR_CUDA, "%s: kernel failed: %s", who, cudaGetErrorString(ce));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-    e->last_ms = ms;
-    return ISB_OK;
+    return finish_run(e, who);
 }
 
 int isb_philox_bip_fluct(isb_ctx *ctx, int rule, int prec, uint64_t seed, uint64_t step_offset, int layer, int nunits,

@@ -78,16 +78,6 @@ __device__ __forceinline__ void bulk_g2s(void *smem_dst, const void *gmem_src, u
         : "memory");
 }
 
-// Multicast variant: the bytes land at the same CTA-relative offset in every CTA of `cta_mask`, and each
-// destination CTA's mbarrier (same offset) receives the complete_tx.
-__device__ __forceinline__ void bulk_g2s_multicast(void *smem_dst, const void *gmem_src, uint32_t bytes, uint64_t *bar,
-                                                   uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(
-            smem_u32(smem_dst)),
-        "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask)
-        : "memory");
-}
 // ------------------------------------------------------------------ thread-block clusters
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
@@ -97,15 +87,6 @@ __device__ __forceinline__ uint32_t cluster_ctarank() {
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
     asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// arrive on the mbarrier at the same offset in CTA `target` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint64_t *bar, uint32_t target) {
-    asm volatile(
-        "{\n\t.reg .b32 ra;\n\t"
-        "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-        "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}" ::"r"(smem_u32(bar)),
-        "r"(target)
-        : "memory");
 }
 
 // ------------------------------------------------------------------ warp helpers

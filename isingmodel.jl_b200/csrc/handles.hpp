@@ -43,7 +43,7 @@ struct isb_model {
     bool fast_ok = false;        // N <= 1024: register-resident sweep kernel applies
     bool j_is_f32 = false;       // storage type of the permuted copy used by the sweep kernel
     double *J64 = nullptr;       // natural layout [npad][npad] (row i contiguous; symmetric)
-    void *Jperm = nullptr;       // permuted columns, double or float, [npad][npad]
+    void *Jperm = nullptr;       // permuted columns (isb::ssf_perm_pos), double or float, [npad][npad]
     double *h64 = nullptr;       // [npad]
     // near-tie guard of the single-spin kernels: 0 when every coupling and field is a small dyadic number (all sums are
     // exact), else 2^-30 of the largest row sum of |J| + |h| (see SsfParams::guard)
@@ -101,6 +101,17 @@ struct isb_ens {
 namespace isb {
 
 int fail(isb_ctx *ctx, int code, const char *fmt, ...);
+// The permuted column layout of the sweep kernel's couplings (isb_model::Jperm, and Jfix with VEC = 4): site k*32 + lane
+// of a row sits at position (k / VEC)*32*VEC + lane*VEC + k % VEC, so that a lane loads the couplings of its sites k .. k +
+// VEC - 1 with one vector load (VEC = min(16 bytes / coupling size, NPL); ssf_kernel's apply_row).
+__host__ __device__ constexpr int ssf_perm_pos(int site, int vec) {
+    const int k = site >> 5, lane = site & 31;
+    return (k / vec) * (32 * vec) + lane * vec + k % vec;
+}
+__host__ __device__ constexpr int ssf_perm_site(int pos, int vec) {   // the inverse of ssf_perm_pos
+    const int kv = pos / (32 * vec), rm = pos % (32 * vec);
+    return (kv * vec + rm % vec) * 32 + rm / vec;
+}
 // Near-tie guard of a general-graph model from its couplings (n values per row at vals[i * ld + j], or a flat list with
 // rows given by rowptr) and fields: see isb_model::guard.
 double ssf_guard_from(const double *absrowsum, const double *vals, size_t nvals, const double *h, int n);
@@ -121,9 +132,13 @@ enum { SCR_NODES = 0, SCR_FLUCT = 1, SCR_T = 2, SCR_E = 3, SCR_M = 4, SCR_FLUCT2
     } while (0)
 
 // ssf.cu
-int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_t *d_nodes, int start,
-                   int fluct_mode, const double *d_fluct, uint64_t seed, uint64_t step_offset,
-                   const double *d_T, int64_t steps_per_T, int64_t trace_every, double *d_E, double *d_M, int8_t *d_S);
+// The sweeps of every single-spin entry point (isb_ssf_run*, and each round / temperature step of isb_ssf_run_pt /
+// isb_ssf_run_pa), on arguments the entry point has checked: for ISB_ORDER_RANDOM the Philox site list into d_nodes
+// [nsteps] first, then dense models up to 1024 sites on the register-resident kernel, everything else on the
+// neighbour-list kernel (which hands periodic lattices to the lattice kernels).
+int ssf_sweep_device(isb_ens *e, int rule, int64_t nsteps, int order, int32_t *d_nodes, int start, int fluct_mode,
+                     const double *d_fluct, uint64_t seed, uint64_t step_offset, const double *d_T, int64_t steps_per_T,
+                     int64_t trace_every, double *d_E, double *d_M, int8_t *d_S);
 int ssf_ensure_fields(isb_ens *e, int sign);
 size_t ssf_field_elem_size(const isb_model *m);
 int philox_fluct_device(isb_ctx *ctx, int rule, uint64_t seed, uint64_t step_offset, int r0, int nr,
@@ -141,6 +156,7 @@ int config_histogram_device(isb_ctx *ctx, const int8_t *d_S, int64_t count, int 
 // sparse.cu
 int sparse_model_init(isb_model *m, int n, const int64_t *colptr, const int32_t *rowval, const double *nzval, int *warn);
 void sparse_model_free(isb_model *m);
+bool sparse_model_lattice(const isb_model *m);   // a periodic lattice the lattice kernels run (ISB_ORDER_CHECKERBOARD)
 void sparse_model_set_guard(isb_model *m, const double *h_host);  // near-tie guard from the stored couplings and h
 int sparse_field_device(isb_ens *e, double *d_out, int64_t ld, int nout, double hsign);
 int sparse_energy_device(isb_ens *e, double *d_E);
@@ -159,13 +175,6 @@ int lattice_side(const void *lat);
 int ssf_lattice_run_device(isb_ens *e, void *lat, int rule, int64_t nsteps, int order, int start, int fluct_mode, const double *d_fluct,
                            uint64_t seed, uint64_t step_offset, const double *d_T, int64_t steps_per_T, int64_t trace_every,
                            double *d_E, double *d_M, int8_t *d_S);
-
-// tempering.cu: one traced Philox run of both device loops (parallel tempering and population annealing) on the dispatch
-// of isb_ssf_run: the site list of a random order, then the dense register-resident kernel for dense models up to 1024
-// sites or the neighbour-list kernel for everything else (which hands periodic lattices to the lattice kernels).  E / M
-// of the last step go to d_E / d_M [R] (steps_per_T = trace_every = nsteps).
-int ssf_traced_run_device(isb_ens *e, int rule, int64_t nsteps, int order, int32_t *d_nodes, int start, uint64_t seed,
-                          uint64_t step_offset, const double *d_T, double *d_E, double *d_M);
 
 // tempering.cu: `rounds` rounds of isb_ssf_run_pt on the context stream, no host synchronisation between rounds.  Round k
 // is one sweep launch of steps_per_round steps (traced E / M of its last step into d_Eround / d_Mround [R]), the overlap

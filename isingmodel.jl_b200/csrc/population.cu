@@ -1,6 +1,6 @@
 // population.cu — population annealing for single-spin ensembles (isb_ssf_run_pa) and the replica gather under it
 // (isb_ens_select_replicas).  The sweep kernels are not touched: every temperature step is one traced isb_ssf_run of the
-// same steps (ssf_traced_run_device, shared with parallel tempering), and the resampling decides on the energies those
+// same steps (ssf_sweep_device, the sweep dispatch of isb_ssf_run), and the resampling decides on the energies those
 // kernels trace at the last step.  The resampling is a segmented multi-CTA scheme (PA_THREADS slots per CTA, up to
 // PA_THREADS CTAs per population), so populations are not limited by shared memory:
 //   pa_weight_kernel  a_r = -db E_r and the CTA maxima of a (and the per-slot flip totals)
@@ -205,8 +205,8 @@ int ssf_pa_run_device(isb_ens *e, int rule, int n_pop, int64_t nT, const double 
         const int st = (int)(((int64_t)start + t0 % n) % n);
         double *Ek = d.recE ? d.recE + k * R : d.E;
         double *Mk = d.recM ? d.recM + k * R : nullptr;
-        if (int rc = ssf_traced_run_device(e, rule, steps_per_T, order, d.nodes, st, seed, step_offset + (uint64_t)t0,
-                                           d.T + k, Ek, Mk))
+        if (int rc = ssf_sweep_device(e, rule, steps_per_T, order, d.nodes, st, ISB_FLUCT_PHILOX, nullptr, seed,
+                                      step_offset + (uint64_t)t0, d.T + k, steps_per_T, steps_per_T, Ek, Mk, nullptr))
             return rc;
         const bool resample = k < n_res;
         pa_weight_kernel<<<grid, PA_THREADS, 0, ctx->stream>>>(P, nb, resample ? -db[k] : 0.0, Ek, e->d_flips,

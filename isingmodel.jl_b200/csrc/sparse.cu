@@ -331,6 +331,8 @@ void sparse_model_set_guard(isb_model *m, const double *h_host) {
     sm->vals.clear();
 }
 
+bool sparse_model_lattice(const isb_model *m) { return m->sp && ((const SparseModel *)m->sp)->lattice; }
+
 void sparse_model_free(isb_model *m) {
     SparseModel *sm = (SparseModel *)m->sp;
     if (!sm) return;
@@ -367,8 +369,7 @@ int ssf_sparse_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const
     isb_ctx *ctx = m->ctx;
     SparseModel *sm = (SparseModel *)m->sp;
     if (nsteps <= 0) return ISB_OK;
-    if (order == ISB_ORDER_CHECKERBOARD && !sm->lattice)
-        return fail(ctx, ISB_ERR_UNSUPPORTED, "ISB_ORDER_CHECKERBOARD needs a periodic L x L lattice (L a multiple of 32) with four neighbours per site");
+    // (ISB_ORDER_CHECKERBOARD arrives on lattices only: the entry points refuse it elsewhere, see sparse_model_lattice)
     if (sm->lattice && (order == ISB_ORDER_SEQUENTIAL || order == ISB_ORDER_CHECKERBOARD))
         return ssf_lattice_run_device(e, sm->lattice, rule, nsteps, order, start, fluct_mode, d_fluct, seed, step_offset, d_T,
                                       steps_per_T, trace_every, d_E, d_M, d_S);
@@ -404,7 +405,6 @@ int ssf_sparse_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const
     p.out_E = d_E; p.out_M = d_M; p.out_S = d_S; p.ldS = m->n; p.flips = e->d_flips; p.near_ties = e->d_counters; p.tie_eps = e->tie_eps;
     p.chains_per_cta = chains;
     p.guard = m->guard;
-    if (const char *env_g = getenv("ISB_SSF_GUARD")) p.guard = atof(env_g);
     p.hsign = rule == ISB_RULE_HOPFIELD ? -1.0 : 1.0;
     const size_t smem = globalf ? 0 : per_chain * chains;
     cudaError_t ce = cudaSuccess;

@@ -14,10 +14,10 @@ namespace isb {
 
 int ssf_cold_chains(const isb_ctx *ctx, int npad, bool fixed);                // ssf_cold.cu
 cudaError_t launch_ssf_cold(const SsfParams &p, int chains, bool fixed, cudaStream_t st);
-cudaError_t launch_ssf_dd(const SsfParams &p, int npl, bool list, bool tma, int cl, int grid, int threads,
-                          size_t smem, cudaStream_t st);
-cudaError_t launch_ssf_ff(const SsfParams &p, int npl, bool list, bool tma, int cl, int grid, int threads,
-                          size_t smem, cudaStream_t st);
+cudaError_t launch_ssf_dd(const SsfParams &p, int npl, bool list, bool tma, int grid, int threads, size_t smem,
+                          cudaStream_t st);
+cudaError_t launch_ssf_ff(const SsfParams &p, int npl, bool list, bool tma, int grid, int threads, size_t smem,
+                          cudaStream_t st);
 cudaError_t launch_ssf_ii(const SsfParams &p, int npl, int grid, int threads, cudaStream_t st);
 
 size_t ssf_field_elem_size(const isb_model *m) { return m->prec == ISB_PREC_F32 ? sizeof(float) : sizeof(double); }
@@ -87,8 +87,7 @@ __global__ void __launch_bounds__(256) fixed_field_init_kernel(const int32_t *__
             for (int r = 0; r < FI_RB; ++r) up[r] += ((bw[r] >> l) & 1u) ? v : 0;
         }
     }
-    const int kv = p / (32 * vec), rm = p % (32 * vec);
-    const int site = (kv * vec + rm % vec) * 32 + rm / vec;   // inverse of the permutation of api.cu (isb_model_dense)
+    const int site = ssf_perm_site(p, vec);
 #pragma unroll
     for (int r = 0; r < FI_RB; ++r)
         if (r0 + r < R) fields[(int64_t)(r0 + r) * npad + site] = 2 * up[r] - all;   // (wrap-around: exact in range)
@@ -295,9 +294,9 @@ static int ssf_ensure_fixed_fields(isb_ens *e) {
 }
 
 // ------------------------------------------------------------------ K1 launch
-int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_t *d_nodes, int start,
-                   int fluct_mode, const double *d_fluct, uint64_t seed, uint64_t step_offset,
-                   const double *d_T, int64_t steps_per_T, int64_t trace_every, double *d_E, double *d_M, int8_t *d_S) {
+static int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_t *d_nodes, int start,
+                          int fluct_mode, const double *d_fluct, uint64_t seed, uint64_t step_offset,
+                          const double *d_T, int64_t steps_per_T, int64_t trace_every, double *d_E, double *d_M, int8_t *d_S) {
     isb_model *m = e->model;
     isb_ctx *ctx = m->ctx;
     if (!m->fast_ok)
@@ -335,28 +334,12 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
         nw = (e->R + ctas - 1) / ctas;
         ctas = (e->R + nw - 1) / nw;
     }
-    const char *env_nw = getenv("ISB_SSF_CHAINS_PER_CTA");
-    if (env_nw) {
-        nw = std::max(1, std::min(max_chains, atoi(env_nw)));
-        ctas = (e->R + nw - 1) / nw;
-    }
-    bool tma = getenv("ISB_SSF_NOTMA") == nullptr;
-    int NG = (int)((ctx->smem_optin - 2048) / ((size_t)SSF_G * rowb));
-    NG = std::min(NG, 8);
-    if (const char *env_ng = getenv("ISB_SSF_NG")) NG = std::max(1, std::min(NG, atoi(env_ng)));   // fewer ring slots = more L1 (A/B runs)
-    if (NG < 2) tma = false;
+    const int NG = std::min(8, (int)((ctx->smem_optin - 2048) / ((size_t)SSF_G * rowb)));
     // the fixed-point path has no streaming kernel: with 4 KiB rows the plain kernel (rows from L1 / L2) was faster than a
     // TMA ring at every acceptance of the C2 anneal (38 % down to 0.1 %; profiles/ssf_fixed_ab_b200.json)
-    if (fixed) tma = false;
-    const size_t smem = tma ? (size_t)NG * SSF_G * rowb + (size_t)(3 * NG + 2) * sizeof(uint64_t) + 16 : 0;
-    // thread-block clusters: one multicast J-row stream per cluster of `cl` CTAs (L2 -> SM traffic / cl)
-    int cl = 1;  // measured on B200: the per-SM ingest of the row stream is the limit, multicast does not lift it
-    const char *env_cl = getenv("ISB_SSF_CLUSTER");
-    if (env_cl && tma) {
-        const int v = atoi(env_cl);
-        cl = (v == 2 || v == 4) ? v : 1;
-    }
-    if (cl > 1) ctas = (ctas + cl - 1) / cl * cl;  // padding CTAs own no chains but take part in the protocol
+    const bool tma = NG >= 2 && !fixed;
+    // ring | full and empty barrier per slot, epoch and go barrier | epoch flips and mode
+    const size_t smem = tma ? (size_t)NG * SSF_G * rowb + (size_t)(2 * NG + 2) * sizeof(uint64_t) + 16 : 0;
 
     SsfParams p{};
     p.J = fixed ? (const void *)m->Jfix : m->Jperm;
@@ -396,12 +379,10 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
     p.NG = NG;
     p.keys = philox_keys(seed);
     p.guard = m->guard;
-    if (const char *env_g = getenv("ISB_SSF_GUARD")) p.guard = atof(env_g);   // 0 disables the near-tie guard (A/B measurements)
     p.J64 = m->J64;
     p.ld64 = m->npad;
     p.hsign = rule == ISB_RULE_HOPFIELD ? -1.0 : 1.0;
     p.od_ratio = 0.8f;
-    if (const char *env_od = getenv("ISB_SSF_OD_RATIO")) p.od_ratio = (float)atof(env_od);
 
     p.fluct_pitch = nsteps;
     const int threads = 32 * (nw + 1);
@@ -433,8 +414,8 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
         if (mode == 0) return launch_ssf_cold(q, cold_chains, fixed, ctx->stream);
         const size_t sm = use_tma ? smem : 0;
         if (fixed) return launch_ssf_ii(q, npl, ctas, threads, ctx->stream);
-        return hd ? launch_ssf_dd(q, npl, list, use_tma, use_tma ? cl : 1, ctas, threads, sm, ctx->stream)
-                  : launch_ssf_ff(q, npl, list, use_tma, use_tma ? cl : 1, ctas, threads, sm, ctx->stream);
+        return hd ? launch_ssf_dd(q, npl, list, use_tma, ctas, threads, sm, ctx->stream)
+                  : launch_ssf_ff(q, npl, list, use_tma, ctas, threads, sm, ctx->stream);
     };
     // Adaptive delivery across launches.  The streaming kernel (TMA ring, adaptive epochs) wins while more than about one
     // flip in five is accepted; below that the plain kernel — every chain reads the rows of its own flips from L2, no
@@ -460,7 +441,7 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
         min_work = 0.0;
     }
     seg = (seg + unit - 1) / unit * unit;
-    bool segment = (tma || fixed) && !list && cl == 1 && unit > 0 && nsteps > 2 * seg && (double)e->R * m->n >= min_work;
+    bool segment = (tma || fixed) && !list && unit > 0 && nsteps > 2 * seg && (double)e->R * m->n >= min_work;
     if (const char *env_sg = getenv("ISB_SSF_SEGMENT")) segment = segment && atoi(env_sg) != 0;
     double thr = fixed ? 2.0 : 0.2;   // accepted flips per attempt above which the streaming kernel is the faster one
     if (const char *env_th = getenv("ISB_SSF_SEG_THR")) thr = atof(env_th);
@@ -513,10 +494,25 @@ int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const int32_
         if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
     }
     if (ce != cudaSuccess)
-        return fail(ctx, ISB_ERR_CUDA, "ssf_kernel launch failed: %s (grid %d x %d threads, %zu B smem, cluster %d)",
-                    cudaGetErrorString(ce), ctas, threads, smem, cl);
+        return fail(ctx, ISB_ERR_CUDA, "ssf_kernel launch failed: %s (grid %d x %d threads, %zu B smem)",
+                    cudaGetErrorString(ce), ctas, threads, smem);
     e->steps_since_refresh += nsteps;
     return ISB_OK;
+}
+
+int ssf_sweep_device(isb_ens *e, int rule, int64_t nsteps, int order, int32_t *d_nodes, int start, int fluct_mode,
+                     const double *d_fluct, uint64_t seed, uint64_t step_offset, const double *d_T, int64_t steps_per_T,
+                     int64_t trace_every, double *d_E, double *d_M, int8_t *d_S) {
+    isb_model *m = e->model;
+    if (order == ISB_ORDER_RANDOM) {
+        if (int rc = philox_nodes_device(m->ctx, m->n, seed, step_offset, nsteps, d_nodes)) return rc;
+        e->last_launches += 1;
+    }
+    if (m->kind == ISB_KIND_SPARSE || !m->fast_ok)
+        return ssf_sparse_run_device(e, rule, nsteps, order, d_nodes, start, fluct_mode, d_fluct, seed, step_offset, d_T,
+                                     steps_per_T, trace_every, d_E, d_M, d_S);
+    return ssf_run_device(e, rule, nsteps, order, d_nodes, start, fluct_mode, d_fluct, seed, step_offset, d_T, steps_per_T,
+                          trace_every, d_E, d_M, d_S);
 }
 
 }  // namespace isb

@@ -7,56 +7,36 @@
 namespace isb {
 
 template <typename K>
-static cudaError_t launch_kernel(K kern, int cluster, const SsfParams &p, int grid, int threads, size_t smem, cudaStream_t st) {
+static cudaError_t launch_kernel(K kern, const SsfParams &p, int grid, int threads, size_t smem, cudaStream_t st) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    if (cluster > 1) {
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)grid);
-        cfg.blockDim = dim3((unsigned)threads);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)cluster;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        return cudaLaunchKernelEx(&cfg, kern, p);
-    }
     kern<<<grid, threads, smem, st>>>(p);
     return cudaGetLastError();
 }
 
 template <typename HT, typename JT, int NPL>
-static cudaError_t launch_one(const SsfParams &p, bool list, bool tma, int cl, int grid, int threads, size_t smem,
-                              cudaStream_t st) {
-    auto go = [&](auto kern, int cluster) { return launch_kernel(kern, cluster, p, grid, threads, smem, st); };
-    if (tma && cl == 2)
-        return list ? go(ssf_kernel<HT, JT, NPL, true, true, 2>, 2) : go(ssf_kernel<HT, JT, NPL, false, true, 2>, 2);
-    if (tma && cl == 4)
-        return list ? go(ssf_kernel<HT, JT, NPL, true, true, 4>, 4) : go(ssf_kernel<HT, JT, NPL, false, true, 4>, 4);
+static cudaError_t launch_one(const SsfParams &p, bool list, bool tma, int grid, int threads, size_t smem, cudaStream_t st) {
+    auto go = [&](auto kern) { return launch_kernel(kern, p, grid, threads, smem, st); };
     if constexpr (std::is_same<HT, double>::value) {
         if (p.guard > 0.0) {   // couplings from a small non-dyadic alphabet: the instantiation with the near-tie guard
-            if (list) return tma ? go(ssf_kernel<HT, JT, NPL, true, true, 1, true>, 1) : go(ssf_kernel<HT, JT, NPL, true, false, 1, true>, 1);
-            return tma ? go(ssf_kernel<HT, JT, NPL, false, true, 1, true>, 1) : go(ssf_kernel<HT, JT, NPL, false, false, 1, true>, 1);
+            if (list) return tma ? go(ssf_kernel<HT, JT, NPL, true, true, true>) : go(ssf_kernel<HT, JT, NPL, true, false, true>);
+            return tma ? go(ssf_kernel<HT, JT, NPL, false, true, true>) : go(ssf_kernel<HT, JT, NPL, false, false, true>);
         }
     }
-    if (list) return tma ? go(ssf_kernel<HT, JT, NPL, true, true>, 1) : go(ssf_kernel<HT, JT, NPL, true, false>, 1);
-    return tma ? go(ssf_kernel<HT, JT, NPL, false, true>, 1) : go(ssf_kernel<HT, JT, NPL, false, false>, 1);
+    if (list) return tma ? go(ssf_kernel<HT, JT, NPL, true, true>) : go(ssf_kernel<HT, JT, NPL, true, false>);
+    return tma ? go(ssf_kernel<HT, JT, NPL, false, true>) : go(ssf_kernel<HT, JT, NPL, false, false>);
 }
 
 template <typename HT, typename JT>
-static cudaError_t launch_pair(const SsfParams &p, int npl, bool list, bool tma, int cl, int grid, int threads,
-                               size_t smem, cudaStream_t st) {
+static cudaError_t launch_pair(const SsfParams &p, int npl, bool list, bool tma, int grid, int threads, size_t smem,
+                               cudaStream_t st) {
     switch (npl) {
-        case 1: return launch_one<HT, JT, 1>(p, list, tma, cl, grid, threads, smem, st);
-        case 2: return launch_one<HT, JT, 2>(p, list, tma, cl, grid, threads, smem, st);
-        case 4: return launch_one<HT, JT, 4>(p, list, tma, cl, grid, threads, smem, st);
-        case 8: return launch_one<HT, JT, 8>(p, list, tma, cl, grid, threads, smem, st);
-        case 16: return launch_one<HT, JT, 16>(p, list, tma, cl, grid, threads, smem, st);
-        case 32: return launch_one<HT, JT, 32>(p, list, tma, cl, grid, threads, smem, st);
+        case 1: return launch_one<HT, JT, 1>(p, list, tma, grid, threads, smem, st);
+        case 2: return launch_one<HT, JT, 2>(p, list, tma, grid, threads, smem, st);
+        case 4: return launch_one<HT, JT, 4>(p, list, tma, grid, threads, smem, st);
+        case 8: return launch_one<HT, JT, 8>(p, list, tma, grid, threads, smem, st);
+        case 16: return launch_one<HT, JT, 16>(p, list, tma, grid, threads, smem, st);
+        case 32: return launch_one<HT, JT, 32>(p, list, tma, grid, threads, smem, st);
         default: return cudaErrorInvalidValue;
     }
 }

@@ -2,7 +2,7 @@
 namespace isb {
 // The fixed-point path (SsfParams::fix_q): sequential order, plain kernel (rows from L1 / L2; see ssf_run_device).
 cudaError_t launch_ssf_ii(const SsfParams &p, int npl, int grid, int threads, cudaStream_t st) {
-    auto go = [&](auto kern) { return launch_kernel(kern, 1, p, grid, threads, 0, st); };
+    auto go = [&](auto kern) { return launch_kernel(kern, p, grid, threads, 0, st); };
     switch (npl) {
         case 1: return go(ssf_kernel<int32_t, int32_t, 1, false, false>);
         case 2: return go(ssf_kernel<int32_t, int32_t, 2, false, false>);

@@ -28,10 +28,7 @@
 
 namespace isb {
 
-#ifndef ISB_SSF_G
-#define ISB_SSF_G 8
-#endif
-constexpr int SSF_G = ISB_SSF_G;  // rows of J per ring slot (a power of two; 8 measured best: A/B builds with -DISB_SSF_G=2|4|16)
+constexpr int SSF_G = 8;  // rows of J per ring slot (a power of two; 8 measured best against 2, 4 and 16: DESIGN §7)
 
 struct SsfParams {
     const void *J;  // permuted couplings [npad][ldj] (double or float)
@@ -186,14 +183,10 @@ __device__ __forceinline__ void fixed_thresholds(double fts, double hh, double q
     hi = a + M;
 }
 
-// CL > 1: the CTAs of a thread-block cluster (same GPC) walk the same row sequence, so the leader CTA's
-// producer issues each J row ONCE as a multicast bulk copy that lands in every CTA's ring (one L2 read for CL
-// SMs).  Followers arm their own full barriers and tell the leader (remote mbarrier arrive) when their slot is free.
 // GUARD: the near-tie guard (SsfParams::guard) is compiled in — a separate instantiation, because its rare slow path
 // costs the hot loop registers (measured: 195 -> 232 ms on the C2 schedule when it is merely present).
-template <typename HT, typename JT, int NPL, bool LIST, bool TMA, int CL = 1, bool GUARD = false>
+template <typename HT, typename JT, int NPL, bool LIST, bool TMA, bool GUARD = false>
 __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(const SsfParams p) {
-    static_assert(CL == 1 || TMA, "clusters only make sense with the TMA ring");
     // int32 fields and couplings: the fixed-point path (sequential order, plain kernel, no traces, no tie audit; see SsfParams)
     constexpr bool FIXED = std::is_same<HT, int32_t>::value;
     static_assert(!FIXED || (std::is_same<JT, int32_t>::value && !LIST && !TMA && !GUARD), "fixed-point: plain sequential sweeps only");
@@ -208,12 +201,10 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
     JT *ring = reinterpret_cast<JT *>(smem_raw);
     uint64_t *full_bar = reinterpret_cast<uint64_t *>(smem_raw + (size_t)p.NG * G * ROWB);
     uint64_t *empty_bar = full_bar + p.NG;
-    uint64_t *peer_bar = empty_bar + p.NG;  // leader only: followers' "slot armed and free" arrivals
-    uint64_t *ep_bar = peer_bar + p.NG;     // consumers -> producer: "epoch finished" (count = chains of this CTA)
+    uint64_t *ep_bar = empty_bar + p.NG;    // consumers -> producer: "epoch finished" (count = chains of this CTA)
     uint64_t *go_bar = ep_bar + 1;          // producer -> consumers: "mode of the next epoch decided"
     unsigned int *ep_flips = reinterpret_cast<unsigned int *>(go_bar + 1);  // flips of the CTA in the current epoch
     volatile int *ep_mode = reinterpret_cast<volatile int *>(ep_flips + 1); // 1 = streamed, 0 = on demand
-    const uint32_t crank = CL > 1 ? cluster_ctarank() : 0u;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int nw = p.nw;
@@ -227,7 +218,6 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
             for (int s = 0; s < NG; ++s) {
                 mbar_init(&full_bar[s], 1);
                 mbar_init(&empty_bar[s], (uint32_t)(nactive > 0 ? nactive : 1));
-                if constexpr (CL > 1) mbar_init(&peer_bar[s], CL - 1);
             }
             mbar_init(ep_bar, (uint32_t)(nactive > 0 ? nactive : 1));
             mbar_init(go_bar, 1);
@@ -235,19 +225,15 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
             *ep_mode = 1;
             mbar_fence_init();
         }
-        if constexpr (CL > 1)
-            cluster_sync_all();  // every CTA's barriers are initialised before any remote arrive / multicast
-        else
-            __syncthreads();
+        __syncthreads();
     }
 
     // ------------------------------------------------------------------ producer warp
     if (warp == nw) {
         if constexpr (TMA) {
             if (lane == 0) {
-                // Adaptive delivery is decided per CTA; inside a cluster all CTAs must stream the same epochs, so
-                // clusters always stream.
-                const bool adaptive = CL == 1 && p.od_ratio > 0.f && nactive > 0;
+                // adaptive delivery is decided per CTA
+                const bool adaptive = p.od_ratio > 0.f && nactive > 0;
                 int site = p.start;
                 int slot = 0;
                 uint32_t ph = 0;  // (slot, ph) of the next streamed group, kept incrementally (no 64-bit divisions)
@@ -282,25 +268,15 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
                         const int64_t left = esteps - q * G;
                         const int rows = left < G ? (int)left : G;
                         mbar_arrive_expect_tx(&full_bar[slot], (uint32_t)(rows * ROWB));
-                        if (CL > 1 && crank != 0) {
-                            mbar_arrive_remote(&peer_bar[slot], 0);  // armed and free: the leader may multicast into it
-                        } else {
-                            if constexpr (CL > 1) mbar_wait(&peer_bar[slot], ph);
-                            for (int g = 0; g < rows; ++g) {
-                                int i;
-                                if constexpr (LIST) {
-                                    i = __ldg(&p.nodes[t0 + q * G + g]);
-                                } else {
-                                    i = site;
-                                    if (++site == p.n) site = 0;
-                                }
-                                if constexpr (CL > 1)
-                                    bulk_g2s_multicast(ring + ((size_t)slot * G + g) * NPAD, Jg + (int64_t)i * p.ldj,
-                                                       ROWB, &full_bar[slot], (uint16_t)((1u << CL) - 1u));
-                                else
-                                    bulk_g2s(ring + ((size_t)slot * G + g) * NPAD, Jg + (int64_t)i * p.ldj, ROWB,
-                                             &full_bar[slot]);
+                        for (int g = 0; g < rows; ++g) {
+                            int i;
+                            if constexpr (LIST) {
+                                i = __ldg(&p.nodes[t0 + q * G + g]);
+                            } else {
+                                i = site;
+                                if (++site == p.n) site = 0;
                             }
+                            bulk_g2s(ring + ((size_t)slot * G + g) * NPAD, Jg + (int64_t)i * p.ldj, ROWB, &full_bar[slot]);
                         }
                         if (++slot == NG) {
                             slot = 0;
@@ -353,7 +329,7 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
     int ep_len = SSF_EPOCH;  // length of the current epoch (on-demand epochs are longer)
     uint32_t ep_idx = 0;
     unsigned int ep_nflips = 0;
-    const bool adaptive = TMA && CL == 1 && p.od_ratio > 0.f;
+    const bool adaptive = TMA && p.od_ratio > 0.f;
 
     auto release_held = [&]() {
         if (held) {
@@ -677,8 +653,6 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
         }
     }
     }  // consumer warp
-    // no CTA of the cluster may retire while a peer can still multicast into its ring or arrive on its barriers
-    if constexpr (CL > 1) cluster_sync_all();
 }
 
 }  // namespace isb

@@ -1,7 +1,7 @@
 // tempering.cu — device-resident parallel tempering for single-spin ensembles (isb_ssf_run_pt): the round loop over the
-// existing sweep launchers, the replica-exchange kernel and the replica-overlap kernel, and the traced sweep dispatch it
-// shares with population annealing (population.cu).  The sweep kernels are not touched: every round is exactly one
-// isb_ssf_run of the same steps, and the exchange decides on the energies those kernels trace at the last step of the round.
+// sweep dispatch of isb_ssf_run (ssf_sweep_device), the replica-exchange kernel and the replica-overlap kernel.  The sweep
+// kernels are not touched: every round is exactly one traced isb_ssf_run of the same steps, and the exchange decides on the
+// energies those kernels trace at the last step of the round.
 #include <algorithm>
 
 #include "common.cuh"
@@ -79,22 +79,6 @@ __global__ void pt_overlap_kernel(int L, int n, const int8_t *__restrict__ spins
     }
 }
 
-int ssf_traced_run_device(isb_ens *e, int rule, int64_t nsteps, int order, int32_t *d_nodes, int start, uint64_t seed,
-                          uint64_t step_offset, const double *d_T, double *d_E, double *d_M) {
-    isb_model *m = e->model;
-    if (order == ISB_ORDER_RANDOM) {
-        if (int rc = philox_nodes_device(m->ctx, m->n, seed, step_offset, nsteps, d_nodes)) return rc;
-        e->last_launches += 1;
-    }
-    // the dispatch of isb_ssf_run: dense models up to 1024 sites on the register-resident kernel, everything else on
-    // the neighbour-list kernel (which hands periodic lattices to the lattice kernels)
-    return (m->kind == ISB_KIND_SPARSE || !m->fast_ok)
-               ? ssf_sparse_run_device(e, rule, nsteps, order, d_nodes, start, ISB_FLUCT_PHILOX, nullptr, seed, step_offset,
-                                       d_T, nsteps, nsteps, d_E, d_M, nullptr)
-               : ssf_run_device(e, rule, nsteps, order, d_nodes, start, ISB_FLUCT_PHILOX, nullptr, seed, step_offset, d_T,
-                                nsteps, nsteps, d_E, d_M, nullptr);
-}
-
 int ssf_pt_run_device(isb_ens *e, int rule, int n_levels, const double *d_levels, int64_t rounds, int64_t steps_per_round,
                       int order, int start, uint64_t seed, uint64_t step_offset, uint64_t round_offset, int32_t *d_nodes,
                       const double *d_T, int32_t *d_level_of, double *d_Eround, double *d_Mround, double *d_recE,
@@ -108,7 +92,8 @@ int ssf_pt_run_device(isb_ens *e, int rule, int n_levels, const double *d_levels
         const int64_t t0 = k * steps_per_round;
         const uint64_t so = step_offset + (uint64_t)t0;
         const int st = (int)(((int64_t)start + t0 % n) % n);
-        if (int rc = ssf_traced_run_device(e, rule, steps_per_round, order, d_nodes, st, seed, so, d_T, d_Eround, d_Mround))
+        if (int rc = ssf_sweep_device(e, rule, steps_per_round, order, d_nodes, st, ISB_FLUCT_PHILOX, nullptr, seed, so, d_T,
+                                      steps_per_round, steps_per_round, d_Eround, d_Mround, nullptr))
             return rc;
         if (d_recQ) {
             pt_overlap_kernel<<<dim3(L, G / 2), 256, 0, ctx->stream>>>(L, m->n, e->spins, e->lds, d_level_of,
