@@ -451,10 +451,21 @@ static int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const
     double thr_cold = fixed ? 0.06 : 0.03;
     if (const char *env_tc = getenv("ISB_SSF_COLD_THR")) thr_cold = atof(env_tc);
     if (cold_chains < 16) thr_cold = -1.0;
-    int forced = -1;          // ISB_SSF_MODE = 0 | 1 | 2: one launch of that kernel (A/B runs and tests)
+    // ISB_SSF_MODE = 0 | 1 | 2: one launch of that kernel (A/B runs and tests).  A mode the run cannot take is an error, so
+    // that a test which forces a kernel never passes on another one.
+    int forced = -1;
     if (const char *env_md = getenv("ISB_SSF_MODE")) {
         forced = atoi(env_md);
-        if (forced < 0 || forced > 2 || (forced == 0 && cold_chains < 1) || (forced == 2 && !tma)) forced = -1;
+        if (forced < 0 || forced > 2)
+            return fail(ctx, ISB_ERR_ARG, "ISB_SSF_MODE=%s: expected 0 (cold), 1 (plain) or 2 (streaming)", env_md);
+        if (forced == 0 && cold_chains < 1)
+            return fail(ctx, ISB_ERR_ARG,
+                        "ISB_SSF_MODE=0: no cold kernel for this run (it needs sequential order, no traces, no tie audit, and "
+                        "either fixed point with Npad %% 128 == 0 or Float64 without the near-tie guard with Npad %% 64 == 0; "
+                        "Npad = %d, %s)", m->npad, fixed ? "fixed point" : (hd ? "Float64" : "Float32"));
+        if (forced == 2 && !tma)
+            return fail(ctx, ISB_ERR_ARG, "ISB_SSF_MODE=2: no streaming kernel for this run (%s)",
+                        fixed ? "the fixed-point path has none" : "the ring does not fit in shared memory");
     }
     if (forced >= 0) {
         ce = launch(0, nsteps, forced);

@@ -197,13 +197,16 @@ def test_ssf_segmented_run_equals_the_oracle(ctx, orc, synth, monkeypatch, thr, 
         assert np.array_equal(M, out["M"][:, r]) and _close(out["E"][:, r], E)
 
 
+@pytest.mark.parametrize("fixed", ["1", "0"])
 @pytest.mark.parametrize("rule,per_rep,start", [(1, True, 5), (2, False, 0), (0, False, 77)])
-@pytest.mark.parametrize("thr,thr_cold", [("0.2", "0.04"), ("2", "2"), ("0.5", "0.25")])
-def test_ssf_cold_kernel_in_segmented_runs(ctx, orc, synth, monkeypatch, thr, thr_cold, rule, per_rep, start):
+@pytest.mark.parametrize("thr,thr_cold", [(None, None), ("2", "2"), ("0.5", "0.25")])
+def test_ssf_cold_kernel_in_segmented_runs(ctx, orc, synth, monkeypatch, thr, thr_cold, rule, per_rep, start, fixed):
     """The third kernel of a segmented run (csrc/ssf_cold.cu: fields in shared memory, 28 chains per SM), chosen when the
-    previous segment accepted few flips and the run has no traces: thresholds of the product, "cold from the second
-    segment on", and a mix that alternates streaming / plain / cold launches.  The cached fields pass from kernel to
-    kernel, so every replica must still equal the oracle's single run bit for bit."""
+    previous segment accepted few flips and the run has no traces.  Untraced sequential runs take the fixed-point kernels
+    (plain and cold, product thresholds 2.0 / 0.06); with ISB_SSF_FIXED=0 they take the Float64 ones (streaming, plain and
+    cold, product thresholds 0.2 / 0.03).  Thresholds: the product's, "cold from the second segment on", and a mix that
+    alternates the kernels.  The cached fields pass from kernel to kernel, so every replica must still equal the oracle's
+    single run bit for bit."""
     L = _lib()
     N, R, sweeps = 128, 90, 37
     nsteps = sweeps * N + 51
@@ -212,9 +215,11 @@ def test_ssf_cold_kernel_in_segmented_runs(ctx, orc, synth, monkeypatch, thr, th
     gen = synth.logistic if rule == 1 else synth.exponential
     fl = None if rule == 0 else gen(84, (R, nsteps) if per_rep else nsteps)
     T = synth.geometric_schedule(3.0, 0.03, sweeps + 1)
+    monkeypatch.setenv("ISB_SSF_FIXED", fixed)
     monkeypatch.setenv("ISB_SSF_SEG_MIN", str(3 * N))
-    monkeypatch.setenv("ISB_SSF_SEG_THR", thr)
-    monkeypatch.setenv("ISB_SSF_COLD_THR", thr_cold)
+    if thr is not None:
+        monkeypatch.setenv("ISB_SSF_SEG_THR", thr)
+        monkeypatch.setenv("ISB_SSF_COLD_THR", thr_cold)
     e = L.Ensemble(L.Model.dense(ctx, J, h, L.PREC_F64), R)
     e.set_spins(S0)
     out = e.ssf_run(rule, nsteps, start=start, fluct=fl, fluct_per_replica=per_rep, T=T, steps_per_T=N)

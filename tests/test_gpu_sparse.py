@@ -131,18 +131,22 @@ def test_dense_model_above_1024_sites(ctx, orc, synth):
     assert _close(e.energy(), np.array([orc.energy(J, h, S[r]) for r in range(R)]))
 
 
-@pytest.mark.parametrize("path,rule", [("dense", 2), ("dense", 1), ("sparse", 2), ("sparse", 1)])
+@pytest.mark.parametrize("path,rule", [("dense", 2), ("dense", 1), ("sparse", 2), ("sparse", 1), ("f32", 1)])
 def test_energy_distribution_matches_exact_result(ctx, synth, path, rule):
     """Independent RNG (in-kernel Philox): the mean energy of the 16 x 16 torus at T = 2.269 sampled by 4096
     chains of sequential sweeps agrees with Kaufman's exact finite-size value (tolerance: 5 standard errors
-    estimated from the replica scatter + 0.1 % for the residual equilibration bias)."""
+    estimated from the replica scatter + 0.1 % for the residual equilibration bias).  Path f32: the dense Float32 kernels
+    (float couplings and fields), which must sample the Boltzmann distribution of the float couplings (here exact)."""
     import scipy.sparse as sp
     from exact_ising import mean_energy
     L_, T, R = 16, 2.269, 4096
     N = L_ * L_
     L = _lib()
     J = synth.lattice_J(L_)
-    model = L.Model.dense(ctx, J, np.zeros(N), L.PREC_AUTO) if path == "dense" else L.Model.sparse(ctx, sp.csc_matrix(J), np.zeros(N))
+    if path == "sparse":
+        model = L.Model.sparse(ctx, sp.csc_matrix(J), np.zeros(N))
+    else:
+        model = L.Model.dense(ctx, J, np.zeros(N), L.PREC_F32 if path == "f32" else L.PREC_AUTO)
     e = L.Ensemble(model, R)
     e.set_spins(synth.spins(3, R, N))
     e.ssf_run(rule, 600 * N, seed=11, T=np.array([T]), steps_per_T=600 * N)            # equilibrate
