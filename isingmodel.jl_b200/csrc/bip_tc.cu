@@ -11,12 +11,13 @@
 //                W is stored as P bf16 terms W = W1 + W2 + W3 (P = 3: 24 mantissa bits, fp32-exact split;
 //                P = 1: W rounded to bf16, exact when W is bf16-representable, e.g. small integers);
 //   D          = fp32 accumulators in TMEM (2 stages x 256 columns), all P terms accumulate into the same D.
-// Warp-specialised persistent kernel, one CTA per SM, by default in CTA pairs (cta_group::2: the two CTAs of a
-// cluster run one M = 256 MMA, each loading its own 128 replicas of A and half of the coupling tile):
-//   warp 0 = TMA producer (cp.async.bulk.tensor, 128B swizzle, smem ring of 6 (pairs) / 4 slots, mbarrier complete_tx)
+// Warp-specialised persistent kernel, one CTA per SM, in CTA pairs (cta_group::2: the two CTAs of a cluster run one
+// M = 256 MMA, each loading its own 128 replicas of A and half of the coupling tile, so every SM pulls half of the
+// coupling bytes from L2; single CTAs were measured slower on every workload, DESIGN §3):
+//   warp 0 = TMA producer (cp.async.bulk.tensor, 128B swizzle, smem ring of 6 slots, mbarrier complete_tx)
 //   warp 1 = MMA issuer (tcgen05.mma.kind::f16 by one elected lane of the leader CTA, tcgen05.commit frees the slot)
 //   warp 2 = TMEM allocator
-//   warps 4-19 = epilogue: tcgen05.ld the accumulators, draw the noise (Philox4x32-10, same words as the
+//   warps 4-15 = epilogue: tcgen05.ld the accumulators, draw the noise (Philox4x32-10, same words as the
 //                Float64 path), apply the rule, write the new layer as bf16 (next GEMM's operand),
 //                overlapping the next tile's MMAs; the canonical int8 spins are refreshed per run / trace point.
 // The producer and issuer warps run their loops warp-uniformly and pick the issuing lane with elect.sync, so that
@@ -54,31 +55,19 @@ constexpr int TC_BK = 64;       // K elements per stage, 16-bit operands (128 by
 constexpr int TC_BK8 = 128;     // K elements per stage, int8 digit planes (the same 128 bytes)
 constexpr int TC_PMAX = 4;      // coupling terms / digit planes
 constexpr int TC_BN_MAX = 256;  // units per tile (UMMA N), runtime BN <= 256, multiple of 16
-constexpr int TC_STAGES = 4;     // smem ring slots, single CTAs (16 KiB of A + 32 KiB of B each)
-#ifndef ISB_TC_STAGES2
-#define ISB_TC_STAGES2 6
-#endif
-constexpr int TC_STAGES2 = ISB_TC_STAGES2;  // CTA pairs: a slot holds 16 KiB of A + half a B tile (16 KiB)
-constexpr int TC_A_BYTES = TC_BM * TC_BK * 2;          // 16 KiB
-constexpr int TC_B_BYTES = TC_BN_MAX * TC_BK * 2;      // 32 KiB
+constexpr int TC_STAGES = 6;     // smem ring slots
+constexpr int TC_A_BYTES = TC_BM * TC_BK * 2;            // 16 KiB: this CTA's 128 replicas
+constexpr int TC_B_BYTES = TC_BN_MAX / 2 * TC_BK * 2;    // 16 KiB: this CTA's half of the coupling tile
 constexpr int TC_STAGE_BYTES = TC_A_BYTES + TC_B_BYTES;
-#ifndef ISB_TC_EPI_WARPS
-#define ISB_TC_EPI_WARPS 12
-#endif
-#ifndef ISB_TC_CW
-#define ISB_TC_CW 16
-#endif
-constexpr int TC_EPI_WARPS = ISB_TC_EPI_WARPS;  // a multiple of 4: equal shares of the four TMEM lane quadrants
-constexpr int TC_CW = ISB_TC_CW;                // accumulator columns (units) per epilogue chunk: 8 or 16
-static_assert(TC_EPI_WARPS % 4 == 0 && (TC_CW == 8 || TC_CW == 16), "epilogue shape");
+constexpr int TC_EPI_WARPS = 12;  // a multiple of 4: equal shares of the four TMEM lane quadrants
+constexpr int TC_CW = 16;         // accumulator columns (units) per epilogue chunk
+static_assert(TC_EPI_WARPS % 4 == 0, "epilogue shape");
 constexpr int TC_THREADS = 32 * (4 + TC_EPI_WARPS);
 constexpr int TC_HALVES = TC_EPI_WARPS / 4;     // epilogue warps per TMEM lane quadrant
 constexpr int TC_GW = TC_CW * TC_HALVES;        // accumulator columns the epilogue warps cover per round
 constexpr int TC_SIG_MAX = 32;                  // chain-resident mode: progress barriers per layer
 constexpr size_t TC_SMEM = (size_t)TC_STAGES * TC_STAGE_BYTES + 1024 /*alignment slack*/ + 1024 /*barriers*/;
 static_assert((2 * TC_STAGES + 8 + 2 * TC_SIG_MAX) * 8 <= 1024, "barrier block");
-static_assert((2 * TC_STAGES2 + 8 + 2 * TC_SIG_MAX) * 8 <= 1024, "barrier block");
-static_assert(TC_STAGES2 * (TC_A_BYTES + TC_B_BYTES / 2) <= TC_STAGES * TC_STAGE_BYTES, "pair ring fits the same smem");
 
 struct TcModel {
     int P = 1;
@@ -146,14 +135,16 @@ struct TcParams {
     // `nsteps_seg` full steps (hidden then visible) on them without leaving the SM — chains are independent, so
     // no grid-wide synchronisation exists; only the CTA's own producer waits for its own epilogue.
     int persist, layer, m_tiles, rows_per_cta, nsteps_seg;
-    // cg == 2: CTA pairs (cta_group::2).  The two CTAs of a cluster run one M = 256 MMA together: CTA `rank` owns the
-    // replicas [m0 + 128 rank, + 128) of the pair's tile and loads the rows [rank bn/2, + bn/2) of the coupling tile,
-    // so every SM ingests half of W per tile.  m_tiles counts tiles of 128 cg replicas.
+    // cg = 2 always: the CTAs run in pairs (cta_group::2).  The two CTAs of a cluster run one M = 256 MMA together: CTA
+    // `rank` owns the replicas [m0 + 128 rank, + 128) of the pair's tile and loads the rows [rank bn/2, + bn/2) of the
+    // coupling tile, so every SM ingests half of W per tile.  m_tiles counts tiles of 128 cg replicas.
     int cg;
     // chain-resident mode: the epilogue publishes its progress through the layer it is writing (one mbarrier per
     // tile and per round of TC_GW columns, sig_gpt[layer] rounds per tile), and the producer of the next half-step
-    // waits K block by K block instead of for the whole layer.  The last `sig_fine` tiles of a half-step publish
-    // after every round (one proxy fence each), the earlier tiles once at their end.
+    // waits K block by K block instead of for the whole layer.  The last `sig_fine` tiles of a half-step (always 1)
+    // publish after every round (one proxy fence each), the earlier tiles once at their end.
+    // cg and sig_fine are parameters rather than constants because folding either one into the kernel changes the
+    // register allocation and schedule of the instantiations that were measured.
     int sig_gpt[2], sig_fine;
     int r_off;               // global replica index of row 0 (a run may hold a slice of the replicas): Philox only
     uint32_t fmt;            // operand format: 0 bf16 terms, 1 fp16 terms, 2 int8 digit planes (selects the instantiation)
@@ -221,23 +212,9 @@ struct TcJobIter {
 };
 
 // ------------------------------------------------------------------ PTX wrappers (tcgen05 / TMA)
-__device__ __forceinline__ void tma_load_2d(void *smem_dst, const CUtensorMap *map, int c0, int c1, uint64_t *bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
-            smem_u32(smem_dst)),
-        "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_3d(void *smem_dst, const CUtensorMap *map, int c0, int c1, int c2, uint64_t *bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
-            smem_u32(smem_dst)),
-        "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-// 2-CTA variants (CG = 2, the two CTAs of a cluster on one TPC): each CTA loads its own A rows and HALF of the B
-// tile; the bytes of both CTAs complete on the leader's (cluster rank 0) full barrier, whose address `leader_bar`
-// is a shared::cluster address obtained with mapa.
+// All of them act for a CTA pair (the two CTAs of a cluster on one TPC): each CTA loads its own A rows and HALF of
+// the B tile; the bytes of both CTAs complete on the leader's (cluster rank 0) full barrier, whose address
+// `leader_bar` is a shared::cluster address obtained with mapa.
 __device__ __forceinline__ uint32_t mapa_rank0(const void *smem_ptr) {
     uint32_t ra;
     asm volatile("mapa.shared::cluster.u32 %0, %1, 0;" : "=r"(ra) : "r"(smem_u32(smem_ptr)));
@@ -249,38 +226,27 @@ __device__ __forceinline__ uint32_t mapa_rank0(const void *smem_ptr) {
 __device__ __forceinline__ void mbar_arrive_cluster_addr(uint32_t cluster_addr) {
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
-__device__ __forceinline__ void tma_load_2d_cg2(void *smem_dst, const CUtensorMap *map, int c0, int c1, uint32_t leader_bar) {
+__device__ __forceinline__ void tma_load_2d(void *smem_dst, const CUtensorMap *map, int c0, int c1, uint32_t leader_bar) {
     asm volatile(
         "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
             smem_u32(smem_dst)),
         "l"(map), "r"(leader_bar), "r"(c0), "r"(c1)
         : "memory");
 }
-__device__ __forceinline__ void tma_load_3d_cg2(void *smem_dst, const CUtensorMap *map, int c0, int c1, int c2, uint32_t leader_bar) {
+__device__ __forceinline__ void tma_load_3d(void *smem_dst, const CUtensorMap *map, int c0, int c1, int c2, uint32_t leader_bar) {
     asm volatile(
         "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
             smem_u32(smem_dst)),
         "l"(map), "r"(leader_bar), "r"(c0), "r"(c1), "r"(c2)
         : "memory");
 }
-template <int CG>
 __device__ __forceinline__ void tmem_alloc(uint32_t *smem_slot, uint32_t ncols) {
-    if constexpr (CG == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_slot)), "r"(ncols)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    } else {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_slot)), "r"(ncols)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_slot)), "r"(ncols)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
 }
-template <int CG>
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-    if constexpr (CG == 1)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-    else
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
 // true in exactly one (converged) lane of the warp
 __device__ __forceinline__ bool elect_one() {
@@ -294,66 +260,32 @@ __device__ __forceinline__ bool elect_one() {
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-template <int CG>
+// issued by the leader CTA only: M = 256 (128 rows of A per CTA), each CTA holds half of B's rows
 __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-    if constexpr (CG == 1)
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "setp.ne.b32 p, %4, 0;\n\t"
-            "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-            "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-            : "memory");
-    else  // issued by the leader CTA only: M = 256 (128 rows of A per CTA), each CTA holds half of B's rows
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "setp.ne.b32 p, %4, 0;\n\t"
-            "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-            "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-            : "memory");
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
+        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
+        : "memory");
 }
 // kind::i8: A, B signed 8-bit, D = int32 accumulators, K = 32 per instruction (the same 32 operand bytes per row)
-template <int CG>
 __device__ __forceinline__ void umma_i8(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-    if constexpr (CG == 1)
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "setp.ne.b32 p, %4, 0;\n\t"
-            "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-            "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-            : "memory");
-    else
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "setp.ne.b32 p, %4, 0;\n\t"
-            "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-            "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-            : "memory");
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
+        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
+        : "memory");
 }
-// CG = 2: the arrive is multicast to the barrier at the same offset in both CTAs of the pair
-template <int CG>
+// the arrive is multicast to the barrier at the same offset in both CTAs of the pair
 __device__ __forceinline__ void umma_commit(uint64_t *bar) {
-    if constexpr (CG == 1)
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-                     : "memory");
-    else
-        asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                         smem_u32(bar)),
-                     "h"((uint16_t)3)
-                     : "memory");
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-                 : "r"(taddr)
+    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+                     smem_u32(bar)),
+                 "h"((uint16_t)3)
                  : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-#ifdef ISB_TC_PROBE_NO_LDTM   // timing probe only: how much of a chunk is the tcgen05.ld latency?
-#pragma unroll
-    for (int j = 0; j < 16; ++j) v[j] = taddr * 2654435761u + (uint32_t)j * 40503u;
-    return;
-#endif
     asm volatile(
         "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
         : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
@@ -364,11 +296,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
 }
 // the same load without the wait: several loads in flight, one tmem_ld_wait() before the first use
 __device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t (&v)[16]) {
-#ifdef ISB_TC_PROBE_NO_LDTM
-#pragma unroll
-    for (int j = 0; j < 16; ++j) v[j] = taddr * 2654435761u + (uint32_t)j * 40503u;
-    return;
-#endif
     asm volatile(
         "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
         : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
@@ -454,32 +381,10 @@ __device__ __forceinline__ float ex2_approx(float x) {
 }
 __device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
 
-// Waits of the tcgen05 kernel.  Single CTAs: every completion is local and the suspending try_wait (20 us hint)
-// leaves the issue slots to the epilogue warps.  CTA pairs: the barriers complete through the peer (remote arrives,
-// multicast commits, the peer's TMA bytes) and the suspended waiters were measured to wake late (the pair kernel ran
-// at half the single-CTA rate), so pairs poll.
-template <int CG>
-__device__ __forceinline__ void tc_wait(uint64_t *bar, uint32_t parity) {
-#ifdef ISB_TC_PAIR_SLEEP
-    mbar_wait_sleep(bar, parity);
-#else
-    if constexpr (CG == 2)
-        mbar_wait(bar, parity);
-    else
-        mbar_wait_sleep(bar, parity);
-#endif
-}
-
-// The producer and the MMA issuer are one thread each: they poll (two threads' issue slots are nothing), so that the
-// dependency chain epilogue -> producer -> TMA -> MMA of a half-step boundary carries no wake-up latency.
-template <int CG>
-__device__ __forceinline__ void tc_wait1(uint64_t *bar, uint32_t parity) {
-#ifdef ISB_TC_SLEEP_ALL
-    tc_wait<CG>(bar, parity);
-#else
-    mbar_wait(bar, parity);
-#endif
-}
+// Every wait of the kernel polls (mbar_wait).  The barriers complete through the peer CTA (remote arrives, multicast
+// commits, the peer's TMA bytes), and suspended waits (a try_wait time hint) gained nothing there (DESIGN §3).  The
+// producer and the MMA issuer are one thread each: polling costs two threads' issue slots, and the dependency chain
+// epilogue -> producer -> TMA -> MMA of a half-step boundary carries no wake-up latency.
 
 struct TcMaps {
     CUtensorMap A[2];     // input spin matrix of layer update [1] (visible layer) and [0] (hidden layer)
@@ -488,14 +393,14 @@ struct TcMaps {
 
 // FMT: operand format (0 bf16 terms, 1 fp16 terms of the pre-scaled couplings, 2 int8 digit planes); a template
 // parameter, so that the bf16 instantiations keep their code (and registers) exactly.
-template <bool EXTF, int CG, int FMT>
+template <bool EXTF, int FMT>
 __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_constant__ TcMaps maps, const TcParams p) {
     constexpr bool F16 = FMT == 1;
     constexpr bool I8 = FMT == 2;
     constexpr int BK = I8 ? TC_BK8 : TC_BK;                   // K elements per ring slot (128 bytes either way)
     constexpr uint32_t ONE2 = F16 ? 0x3C003C00u : 0x3F803F80u;  // two packed +1 of the operand format
-    constexpr int NST = CG == 2 ? TC_STAGES2 : TC_STAGES;     // ring slots
-    constexpr int STB = TC_A_BYTES + TC_B_BYTES / CG;         // bytes per slot
+    constexpr int NST = TC_STAGES;                            // ring slots
+    constexpr int STB = TC_STAGE_BYTES;                       // bytes per slot
     extern __shared__ unsigned char smem_dyn[];
     unsigned char *smem = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem + (size_t)TC_STAGES * TC_STAGE_BYTES);
@@ -507,46 +412,32 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
     uint64_t *sig_bar = bars + 2 * NST + 8;  // [2][TC_SIG_MAX] chain-resident mode: epilogue -> producer progress
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int crank = CG == 2 ? (int)cluster_ctarank() : 0;  // rank in the CTA pair; 0 = leader (issues the MMAs)
+    const int crank = (int)cluster_ctarank();  // rank in the CTA pair; 0 = leader (issues the MMAs)
     const bool leader = crank == 0;
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < NST; ++s) {
-#ifdef ISB_TC_PAIR_NOARRIVE  // A/B probe: only the leader arrives (with both CTAs' byte count)
-            mbar_init(&full_bar[s], 1);
-#else
-            mbar_init(&full_bar[s], CG);   // pair: the leader's barrier takes one arrive per CTA and both CTAs' bytes
-#endif
+            mbar_init(&full_bar[s], 2);   // the leader's barrier takes one arrive per CTA and both CTAs' bytes
             mbar_init(&empty_bar[s], 1);
         }
         for (int a = 0; a < 2; ++a) mbar_init(&tfull_bar[a], 1);
         for (int a = 0; a < 2; ++a)
-            mbar_init(&tempty_bar[a], CG * TC_EPI_WARPS);  // pair: the epilogue warps of both CTAs release the leader's
+            mbar_init(&tempty_bar[a], 2 * TC_EPI_WARPS);  // the epilogue warps of both CTAs release the leader's
         if (p.persist)
             for (int i = 0; i < 2 * TC_SIG_MAX; ++i) mbar_init(&sig_bar[i], TC_EPI_WARPS);
         mbar_fence_init();
     }
-    if (warp == 2) tmem_alloc<CG>(tmem_slot, 512);
+    if (warp == 2) tmem_alloc(tmem_slot, 512);
     tc_fence_before();
-    // pair: no remote arrive, multicast commit or 2-CTA MMA may touch the peer before its barriers / TMEM exist
-    if constexpr (CG == 2)
-        cluster_sync_all();
-    else
-        __syncthreads();
+    // no remote arrive, multicast commit or 2-CTA MMA may touch the peer before its barriers / TMEM exist
+    cluster_sync_all();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     TcJobIter jobs;
     jobs.init(p, crank);
     TcJob job;
 
-    // ISB_TC_REGSPLIT (16 sampling warps): the four service warps (TMA producer, MMA issuer, TMEM allocator, spare) hand
-    // registers to the sampling warps (launch: 96 per thread).  The two setmaxnreg sit at the head of code paths that
-    // only meet again at the kernel's last barrier, so that ptxas budgets each path separately.
     if (warp < 4) {
-#ifdef ISB_TC_REGSPLIT
-    static_assert(TC_EPI_WARPS == 16, "register split is sized for 16 sampling warps");
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(ISB_TC_REGS_SERVICE) : "memory");
-#endif
     if (warp == 0) {
         // ================================================================ TMA producer
         // (the whole warp walks the loop, one elected lane issues: see the MMA issuer below)
@@ -562,13 +453,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
                 const int pl = 1 - job.layer;   // the layer sampled by the previous half-step = this one's input
                 const uint32_t dep_par = (uint32_t)((job.hs >> 1) - (job.layer == 1 ? 1 : 0)) & 1u;
                 int waited = -1;
-                const int bnc = L.bn_mma / CG;  // rows of the coupling tile this CTA loads
+                const int bnc = L.bn_mma / 2;  // rows of the coupling tile this CTA loads
                 const uint32_t tx = (uint32_t)(TC_A_BYTES + bnc * 128);
-#ifdef ISB_TC_PROBE_K1  // timing probe only: one K block per tile = the epilogue's cost without the contraction
-                const int num_kb = 1;
-#else
                 const int num_kb = L.num_kb;
-#endif
                 // 16-bit terms: K block outer, term inner (all terms accumulate into one accumulator).  int8 digit
                 // planes: one stacked coupling tile per K block (all planes in one MMA).
                 const int n_inner = I8 ? 1 : p.P;
@@ -579,30 +466,22 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
                         const int ul = min(kb * BK + BK - 1, p.L[pl].nout - 1);
                         const int idx = (ul / p.L[pl].bn) * p.sig_gpt[pl] + (ul % p.L[pl].bn) / TC_GW;
                         if (idx > waited) {
-                            tc_wait1<CG>(&sig_bar[pl * TC_SIG_MAX + idx], dep_par);
+                            mbar_wait(&sig_bar[pl * TC_SIG_MAX + idx], dep_par);
                             waited = idx;
                         }
                     }
                     for (int ti = 0; ti < n_inner; ++ti) {
                         const int t = ti;
-                        tc_wait1<CG>(&empty_bar[s], ph ^ 1u);
+                        mbar_wait(&empty_bar[s], ph ^ 1u);
                         unsigned char *sa = smem + (size_t)s * STB;
                         if (elect_one()) {
-                            if constexpr (CG == 1) {
-                                mbar_arrive_expect_tx(&full_bar[s], tx);
-                                tma_load_3d(sa, &maps.A[job.layer], kr * BK, job.m0, kq, &full_bar[s]);
-                                tma_load_2d(sa + TC_A_BYTES, &maps.B[job.layer][t], kb * BK, job.n_blk * L.bn_mma, &full_bar[s]);
-                            } else {
-                                const uint32_t lbar = mapa_rank0(&full_bar[s]);
-                                if (leader)
-                                    mbar_arrive_expect_tx(&full_bar[s], 2u * tx);
-#ifndef ISB_TC_PAIR_NOARRIVE
-                                else
-                                    mbar_arrive_cluster_addr(lbar);
-#endif
-                                tma_load_3d_cg2(sa, &maps.A[job.layer], kr * BK, job.m0, kq, lbar);
-                                tma_load_2d_cg2(sa + TC_A_BYTES, &maps.B[job.layer][t], kb * BK, job.n_blk * L.bn_mma + crank * bnc, lbar);
-                            }
+                            const uint32_t lbar = mapa_rank0(&full_bar[s]);
+                            if (leader)
+                                mbar_arrive_expect_tx(&full_bar[s], 2u * tx);
+                            else
+                                mbar_arrive_cluster_addr(lbar);
+                            tma_load_3d(sa, &maps.A[job.layer], kr * BK, job.m0, kq, lbar);
+                            tma_load_2d(sa + TC_A_BYTES, &maps.B[job.layer][t], kb * BK, job.n_blk * L.bn_mma + crank * bnc, lbar);
                         }
                         __syncwarp();
                         if (++s == NST) {
@@ -617,37 +496,31 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
                 }
                 }
             }
-            if constexpr (CG == 2) {
-                // the leader's commits also arrive on this CTA's empty barriers: do not retire (or let the peer retire)
-                // before the last of them has landed
-                for (int i = 0; i < NST; ++i) {
-                    tc_wait1<CG>(&empty_bar[s], ph ^ 1u);
-                    if (++s == NST) {
-                        s = 0;
-                        ph ^= 1u;
-                    }
+            // the leader's commits also arrive on this CTA's empty barriers: do not retire (or let the peer retire)
+            // before the last of them has landed
+            for (int i = 0; i < NST; ++i) {
+                mbar_wait(&empty_bar[s], ph ^ 1u);
+                if (++s == NST) {
+                    s = 0;
+                    ph ^= 1u;
                 }
             }
         }
     } else if (warp == 1) {
-        // ================================================================ MMA issuer (pair: the leader CTA's only)
+        // ================================================================ MMA issuer (the leader CTA's only)
         // The WHOLE warp walks this loop and one elected lane issues: with warp-uniform control flow the smem
         // descriptors, TMEM and barrier addresses stay in uniform registers.  (Under `if (lane == 0)` ptxas wrapped every
         // tcgen05 instruction in an ELECT / R2UR.BROADCAST / BRA.U.ANY loop: 112 instructions per K block, 890 cycles for
         // 512 cycles of MMA — the issuing thread, not the operand feed, bounded the contraction.)
-        if (CG == 1 || leader) {
+        if (leader) {
             uint32_t tl = 0;
             int s = 0;            // ring slot and its phase, kept incrementally
             uint32_t ph = 0;
             const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
             while (jobs.next(p, job)) {
                 const TcLayer &L = p.L[job.layer];
-                const uint32_t idesc = I8 ? umma_idesc_i8(TC_BM * CG, L.bn_mma) : umma_idesc_bf16(TC_BM * CG, L.bn_mma, F16 ? 1u : 0u);
-#ifdef ISB_TC_PROBE_K1
-                const int num_kb = 1;
-#else
+                const uint32_t idesc = I8 ? umma_idesc_i8(2 * TC_BM, L.bn_mma) : umma_idesc_bf16(2 * TC_BM, L.bn_mma, F16 ? 1u : 0u);
                 const int num_kb = L.num_kb;
-#endif
                 const int a = tl & 1;
                 // one accumulator stage per tile: all K blocks x terms (16-bit), or the stacked planes (int8), into it
                 const int iters = I8 ? num_kb : num_kb * p.P;
@@ -657,11 +530,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
                 const int i_tail = L.kb_per_blk == L.num_kb ? iters - (I8 ? 1 : p.P) : iters;   // first iteration of the last K block
                 const int nk_tail = min(4, (L.kin - (num_kb - 1) * BK + BK / 4 - 1) / (BK / 4));
                 {
-                    tc_wait1<CG>(&tempty_bar[a], ((tl >> 1) & 1) ^ 1);  // epilogue has drained this accumulator
+                    mbar_wait(&tempty_bar[a], ((tl >> 1) & 1) ^ 1);  // epilogue has drained this accumulator
                     const uint32_t d_tmem = tmem_u + (uint32_t)(a * TC_BN_MAX);
                     tc_fence_after();
                     for (int i = 0; i < iters; ++i) {
-                        tc_wait1<CG>(&full_bar[s], ph);
+                        mbar_wait(&full_bar[s], ph);
                         tc_fence_after();
                         const unsigned char *sa = smem + (size_t)s * STB;
                         const uint64_t adesc = umma_desc_sw128(sa);
@@ -672,19 +545,19 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
 #pragma unroll
                                 for (int k = 0; k < 4; ++k) {  // 4 x 32 operand bytes per slot row: advance 2 descriptor units along K
                                     if constexpr (I8)
-                                        umma_i8<CG>(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (i | k) ? 1u : 0u);
+                                        umma_i8(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (i | k) ? 1u : 0u);
                                     else
-                                        umma_bf16<CG>(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (i | k) ? 1u : 0u);
+                                        umma_bf16(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (i | k) ? 1u : 0u);
                                 }
                             } else {
                                 for (int k = 0; k < nk; ++k) {
                                     if constexpr (I8)
-                                        umma_i8<CG>(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (i | k) ? 1u : 0u);
+                                        umma_i8(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (i | k) ? 1u : 0u);
                                     else
-                                        umma_bf16<CG>(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (i | k) ? 1u : 0u);
+                                        umma_bf16(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (i | k) ? 1u : 0u);
                                 }
                             }
-                            umma_commit<CG>(&empty_bar[s]);  // slot free (in both CTAs of a pair) when these MMAs have read it
+                            umma_commit(&empty_bar[s]);  // slot free (in both CTAs) when these MMAs have read it
                         }
                         __syncwarp();
                         if (++s == NST) {
@@ -693,16 +566,13 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
                         }
                     }
                 }
-                if (elect_one()) umma_commit<CG>(&tfull_bar[a]);  // accumulator complete (each CTA: its 128 replicas x bn units)
+                if (elect_one()) umma_commit(&tfull_bar[a]);  // accumulator complete (each CTA: its 128 replicas x bn units)
                 __syncwarp();
                 ++tl;
             }
         }
     }
     } else {
-#ifdef ISB_TC_REGSPLIT
-        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(ISB_TC_REGS_SAMPLE) : "memory");
-#endif
         // ================================================================ epilogue (sampling rule)
         const int ew = warp - 4;
         const int quad = warp & 3;          // TMEM lane quadrant this warp may read: lanes 32*(warpid % 4) ..
@@ -751,10 +621,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
                 //   u (1 + e^{-2x/T}) > 1,  u = (w + 1/2) 2^-32    <=>    (float)w (1 + 2^{cE x}) > 2^32
                 // (x = acc + bias: FADD; cE x: FMUL; the left side: one FFMA; the compare and the sign packing run on the
                 // ALU pipe, the conversion and the exponential on the XU).
-                fast_hs = !EXTF && CW == 16 && p.rule == ISB_BIP_SCA && L.npeer == 0 && !__any_sync(0xFFFFFFFFu, !(Tf > 0.f));
+                fast_hs = !EXTF && p.rule == ISB_BIP_SCA && L.npeer == 0 && !__any_sync(0xFFFFFFFFu, !(Tf > 0.f));
             }
             TC_TIME(tw0);
-            tc_wait<CG>(&tfull_bar[a], (tl >> 1) & 1);
+            mbar_wait(&tfull_bar[a], (tl >> 1) & 1);
             tc_fence_after();
             TC_TIME(tw1);
             const int gpt = p.sig_gpt[LY];
@@ -764,7 +634,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
             const int tile_u0 = job.n_blk * L.bn;
             const int nfull = fastp ? min(L.bn, L.nout - tile_u0) / CW : 0;   // chunks the fast path takes
             const float *bias_t = L.bias_f + tile_u0;
-            __nv_bfloat16 *out_t = reinterpret_cast<__nv_bfloat16 *>(L.out_bf) + (int64_t)(row_ok ? r : job.m0) * L.ldo + tile_u0;
             const uint32_t taddr_t = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(a * TC_BN_MAX);
             const uint32_t pc2 = (uint32_t)(r + p.r_off), pc3 = (L.domain << 28) | (uint32_t)((L.u_off + tile_u0) >> 2);
             if constexpr (I8) {
@@ -774,11 +643,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
               const int8_t *in8 = L.in_diag ? L.in_diag + (int64_t)rr * L.ld_in + tile_u0 : nullptr;
               const uint32_t tq = taddr_t;          // plane t of the tile: columns [t * bn, (t + 1) * bn) of stage a
               const uint32_t pstride = (uint32_t)L.bn;
-#ifdef ISB_TC_PROBE_NO_EPI  // timing probe only: the contraction without the sampling epilogue
-              for (int g = 0; false;) {
-#else
               for (int g = 0; g * TC_HALVES < nchunks; ++g) {
-#endif
                 const int c = g * TC_HALVES + hrot;
                 if (c < nfull) {
                   // fast path (SCA, in-kernel noise, T > 0, 16 real units): field in float — every plane sum is an exact
@@ -822,22 +687,14 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
                   Philox4 blk[4];
 #pragma unroll
                   for (int q = 0; q < 4; ++q)
-#ifdef ISB_TC_PROBE_NO_PHILOX  // timing probe only: how much of a half-step is the noise generation?
-                      blk[q] = Philox4{(uint32_t)step_abs * 2654435761u + pc2, (pc3 + (uint32_t)(c * 4 + q)) * 40503u, pc2 << 7, keys.k0[3]};
-#else
                       blk[q] = philox4x32_10k((uint32_t)step_abs, (uint32_t)(step_abs >> 32), pc2, pc3 + (uint32_t)(c * 4 + q), keys);
-#endif
                   uint32_t wb[4] = {0x01010101u, 0x01010101u, 0x01010101u, 0x01010101u};
 #pragma unroll
                   for (int j = 0; j < 16; ++j) {
                       const float wf = (float)philox_pick(blk[j >> 2], (uint32_t)(j & 3));
                       if (fmaf(wf, ex2_approx(cE * xf[j]), wf) > 4294967296.0f) wb[j >> 2] |= 0xFEu << (8 * (j & 3));
                   }
-#ifdef ISB_TC_PROBE_NO_STORE   // timing probe only: the sampled spins are (almost) never stored
-                  if (row_ok && (wb[0] ^ (wb[1] << 1) ^ (wb[2] << 2) ^ (wb[3] << 3)) == 0x12345678u) *reinterpret_cast<uint4 *>(out8 + c * 16) = make_uint4(wb[0], wb[1], wb[2], wb[3]);
-#else
                   if (row_ok) *reinterpret_cast<uint4 *>(out8 + c * 16) = make_uint4(wb[0], wb[1], wb[2], wb[3]);
-#endif
                 } else if (c < nchunks && tile_u0 + c * 16 < L.nout) do {   // (chunks of padding units: nothing to do)
                   // general path: the field in double, EXACT (every term is a multiple of the quantum q0)
                   double xd[16];
@@ -903,11 +760,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
                 }
               }
             } else {
-#ifdef ISB_TC_PROBE_NO_EPI  // timing probe only: the contraction without the sampling epilogue
-            for (int g = 0; false;) {
-#else
+            __nv_bfloat16 *out_t = reinterpret_cast<__nv_bfloat16 *>(L.out_bf) + (int64_t)(row_ok ? r : job.m0) * L.ldo + tile_u0;
             for (int g = 0; g * TC_HALVES < nchunks; ++g) {
-#endif
               const int c = g * TC_HALVES + hrot;
               if (c < nfull) {
                 uint32_t v[16];
@@ -938,11 +792,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
                 }
               } else if (c < nchunks) do {
                 uint32_t v[CW];
-                const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(a * TC_BN_MAX + c * CW);
-                if constexpr (CW == 16)
-                    tmem_ld16(taddr, reinterpret_cast<uint32_t(&)[16]>(v));
-                else
-                    tmem_ld8(taddr, reinterpret_cast<uint32_t(&)[8]>(v));
+                tmem_ld16(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(a * TC_BN_MAX + c * CW), v);
                 const int u0 = job.n_blk * L.bn + c * CW;
                 if (!row_ok || u0 >= L.nout) break;
                 __nv_bfloat16 *ob = reinterpret_cast<__nv_bfloat16 *>(L.out_bf) + (int64_t)r * L.ldo + u0;
@@ -996,12 +846,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
 #pragma unroll
                     for (int q = 0; q < CW / 4; ++q) {
                         // == philox_unit_block(seed, domain, r, step, unit >> 2) with the round keys hoisted
-#ifdef ISB_TC_PROBE_NO_PHILOX  // timing probe only: how much of a half-step is the noise generation?
-                        blk[q] = Philox4{(uint32_t)step_abs * 2654435761u + (uint32_t)r, (uint32_t)(u0 + q) * 40503u, (uint32_t)r << 7, keys.k0[3]};
-#else
                         blk[q] = philox4x32_10k((uint32_t)step_abs, (uint32_t)(step_abs >> 32), (uint32_t)(r + p.r_off),
                                                 (L.domain << 28) | (uint32_t)(((L.u_off + u0) >> 2) + q), keys);
-#endif
                     }
 #pragma unroll
                     for (int q = 0; q < CW / 4; ++q) {
@@ -1056,7 +902,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
             __syncwarp();
             if (lane == 0) {
                 uint64_t *tb = &tempty_bar[a];
-                if (CG == 2 && !leader)
+                if (!leader)
                     mbar_arrive_cluster_addr(mapa_rank0(tb));
                 else
                     mbar_arrive(tb);
@@ -1115,13 +961,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) bip_tc_kernel(const __grid_cons
 #endif
     }
     tc_fence_before();
-    if constexpr (CG == 2)
-        cluster_sync_all();  // neither CTA frees its TMEM or retires while the pair's MMAs / remote arrives can be in flight
-    else
-        __syncthreads();
+    cluster_sync_all();  // neither CTA frees its TMEM or retires while the pair's MMAs / remote arrives can be in flight
     if (warp == 2) {
         tc_fence_after();
-        tmem_dealloc<CG>(tmem_base, 512);
+        tmem_dealloc(tmem_base, 512);
     }
 }
 
@@ -1263,12 +1106,10 @@ static int pick_bn(int nout, int bn_max = TC_BN_MAX) {
 
 // Row pitch (elements) of a K-major bf16 operand with k valid columns.  A TMA box reads 128-256 rows at this pitch at
 // once: a pitch that is a multiple of 1 KiB would put all of them on a few L2 slices, so such pitches get one more
-// 128-byte line (ISB_TC_PAD=0 disables the padding, for A/B measurements).
+// 128-byte line.
 static int tc_pitch(int k, int esz = 2) {
     int ld = (k + 15) / 16 * 16;
-    bool pad = true;
-    if (const char *env = getenv("ISB_TC_PAD")) pad = atoi(env) != 0;
-    if (pad && (ld * esz) % 1024 == 0) ld += 128 / esz;
+    if ((ld * esz) % 1024 == 0) ld += 128 / esz;
     return ld;
 }
 
@@ -1320,10 +1161,6 @@ static bool prec_is_i8(int prec) { return prec == ISB_PREC_I8X2 || prec == ISB_P
 // on config 4: 512 hidden units as 7 tiles of 80 beat 8 tiles of 64 by 3 % although they pad the layer to 560) — so
 // minimise tiles x (N + 160) over the multiples of 16.
 static int i8_pick_bn(int nout, int P) {
-    if (const char *env = getenv("ISB_I8_BN")) {
-        const int v = atoi(env);
-        if (v >= 16 && v % 16 == 0 && v * P <= TC_BN_MAX) return v;
-    }
     int best = 16;
     long best_cost = 0;
     for (int bn = 16; bn * P <= TC_BN_MAX; bn += 16) {
@@ -1551,7 +1388,7 @@ void bip_tc_ens_free(isb_ens *e) {
 }
 
 // Coupling tensor maps of orientation `orient` (1: Wt, hidden update; 0: Wn, visible update) whose box holds `bn`
-// rows of W (the tile width, or half of it when a CTA pair shares the tile)
+// rows of W (half the tile width: each CTA of a pair loads half of the tile)
 static int get_maps_b(isb_ctx *ctx, TcModel *t, int orient, int bn, CUtensorMap out[TC_PMAX]) {
     const int dflt = (orient == 1 ? t->bn_h : t->bn_v) * (t->i8 ? t->P : 1);
     const int esz = t->i8 ? 1 : 2;
@@ -1601,18 +1438,9 @@ static void fill_layer(TcLayer &L, int nout, int kin, int bn, void *out_bf, int6
     L.npeer = 0;
 }
 
-// CTA pairs (cta_group::2, the default) or single CTAs (ISB_TC_CG=1)?  Pairs halve the coupling bytes every SM pulls
-// from L2 and reads from shared memory per MMA.  Measured on B200 (bf16x1 / bf16x3, TFLOP/s algorithmic): C3 1340 / 472
-// with single CTAs, 1453 / 504 with pairs; C4 651 / 325 vs 670 / 391.  Results are bit-identical.
-static int tc_cta_group() {
-    int cg = 2;
-    if (const char *env = getenv("ISB_TC_CG")) cg = atoi(env) == 1 ? 1 : 2;
-    return cg;
-}
-
-template <bool EXTF, int CG, int FMT>
+template <bool EXTF, int FMT>
 static int launch_tc_inst(isb_ctx *ctx, const TcMaps &maps, const TcParams &p, int grid) {
-    ISB_CUDA(ctx, cudaFuncSetAttribute(bip_tc_kernel<EXTF, CG, FMT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM));
+    ISB_CUDA(ctx, cudaFuncSetAttribute(bip_tc_kernel<EXTF, FMT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3(TC_THREADS);
@@ -1620,27 +1448,20 @@ static int launch_tc_inst(isb_ctx *ctx, const TcMaps &maps, const TcParams &p, i
     cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CG;
+    attr[0].val.clusterDim.x = 2;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = CG > 1 ? 1 : 0;
-    ISB_CUDA(ctx, cudaLaunchKernelEx(&cfg, bip_tc_kernel<EXTF, CG, FMT>, maps, p));
+    cfg.numAttrs = 1;
+    ISB_CUDA(ctx, cudaLaunchKernelEx(&cfg, bip_tc_kernel<EXTF, FMT>, maps, p));
     return ISB_OK;
 }
 
-// grid = CTAs (a multiple of p.cg)
+// grid = CTAs (even: CTA pairs)
 static int launch_tc(isb_ctx *ctx, const TcMaps &maps, const TcParams &p, int grid, bool extf) {
-    if (p.fmt == 2) {
-        if (p.cg == 2) return extf ? launch_tc_inst<true, 2, 2>(ctx, maps, p, grid) : launch_tc_inst<false, 2, 2>(ctx, maps, p, grid);
-        return extf ? launch_tc_inst<true, 1, 2>(ctx, maps, p, grid) : launch_tc_inst<false, 1, 2>(ctx, maps, p, grid);
-    }
-    if (p.fmt == 1) {
-        if (p.cg == 2) return extf ? launch_tc_inst<true, 2, 1>(ctx, maps, p, grid) : launch_tc_inst<false, 2, 1>(ctx, maps, p, grid);
-        return extf ? launch_tc_inst<true, 1, 1>(ctx, maps, p, grid) : launch_tc_inst<false, 1, 1>(ctx, maps, p, grid);
-    }
-    if (p.cg == 2) return extf ? launch_tc_inst<true, 2, 0>(ctx, maps, p, grid) : launch_tc_inst<false, 2, 0>(ctx, maps, p, grid);
-    return extf ? launch_tc_inst<true, 1, 0>(ctx, maps, p, grid) : launch_tc_inst<false, 1, 0>(ctx, maps, p, grid);
+    if (p.fmt == 2) return extf ? launch_tc_inst<true, 2>(ctx, maps, p, grid) : launch_tc_inst<false, 2>(ctx, maps, p, grid);
+    if (p.fmt == 1) return extf ? launch_tc_inst<true, 1>(ctx, maps, p, grid) : launch_tc_inst<false, 1>(ctx, maps, p, grid);
+    return extf ? launch_tc_inst<true, 0>(ctx, maps, p, grid) : launch_tc_inst<false, 0>(ctx, maps, p, grid);
 }
 
 // Steps [k0, k0 + nseg) of a run: one chain-resident launch when the replicas fill the SMs, else 2 * nseg
@@ -1652,37 +1473,26 @@ static int launch_steps(isb_ens *e, int rule, int fluct_mode, const double *d_Fv
     isb_ctx *ctx = m->ctx;
     TcModel *t = (TcModel *)m->tc;
     TcEns *s = (TcEns *)e->tc;
-    const int cg = tc_cta_group();
-    const int m_tiles = (e->R + TC_BM * cg - 1) / (TC_BM * cg);
+    const int m_tiles = (e->R + 2 * TC_BM - 1) / (2 * TC_BM);   // tiles of a CTA pair's 256 replicas
     const bool extf = fluct_mode != ISB_FLUCT_PHILOX;
     // chain-resident mode pays off when every SM gets a (nearly) full 128-row block of replicas to itself
-    int rows = (e->R + ctx->num_sms - 1) / ctx->num_sms;
-    rows = std::min(rows, TC_BM);
-    bool persist = rows >= 96;
+    bool persist = (e->R + ctx->num_sms - 1) / ctx->num_sms >= 96;
+    // ISB_TC_PERSIST=0|1 forces a launch mode (the tests run both on the same ensemble)
     if (const char *env = getenv("ISB_TC_PERSIST")) persist = atoi(env) != 0 && e->R >= 1;
-    // A CTA's time per step does not depend on how many of its 128 tile rows hold replicas, and these runs are POWER-capped
-    // (C4: ~1000 W, 1.75 GHz of 1.965): full tiles on fewer SMs do the same work per cycle with fewer SMs drawing power —
-    // 16384 chains as 128 CTAs x 128 rows instead of 148 x 111 measured 0.313 -> 0.326 of the bf16 burst rate at 1.84 GHz.
-    // ISB_TC_ROWS overrides (A/B runs; 0 = spread over all SMs).
-    if (persist) {
-        int want = TC_BM;
-        if (const char *env = getenv("ISB_TC_ROWS")) want = atoi(env);
-        if (want >= rows && want <= TC_BM) rows = want;
-    }
     // tile widths: least padding per CTA in chain-resident mode, fewest (waves x width) otherwise
     // (int8 digit planes: the tile width is part of the stacked storage order, fixed when the model was built)
     const int sp = t->i8 ? t->P : 1;
-    const int bn_h = (persist || t->i8) ? t->bn_h : pick_bn_waves(m->nh, m_tiles, ctx->num_sms / cg);
-    const int bn_v = (persist || t->i8) ? t->bn_v : pick_bn_waves(m->nv, m_tiles, ctx->num_sms / cg);
+    const int bn_h = (persist || t->i8) ? t->bn_h : pick_bn_waves(m->nh, m_tiles, ctx->num_sms / 2);
+    const int bn_v = (persist || t->i8) ? t->bn_v : pick_bn_waves(m->nv, m_tiles, ctx->num_sms / 2);
     TcMaps maps;
     maps.A[1] = s->mapSv;
     maps.A[0] = s->mapSh;
-    int rcm = get_maps_b(ctx, t, 1, bn_h * sp / cg, maps.B[1]);
+    int rcm = get_maps_b(ctx, t, 1, bn_h * sp / 2, maps.B[1]);
     if (rcm) return rcm;
-    rcm = get_maps_b(ctx, t, 0, bn_v * sp / cg, maps.B[0]);
+    rcm = get_maps_b(ctx, t, 0, bn_v * sp / 2, maps.B[0]);
     if (rcm) return rcm;
     TcParams p{};
-    p.cg = cg;
+    p.cg = 2;
     const int bk = t->i8 ? TC_BK8 : TC_BK;
     fill_layer(p.L[1], m->nh, m->nv, bn_h, s->Sh, t->i8 ? e->ldh : t->ldkh, m->bb64, t->bias_hf, d_Fh, DOM_BIP_HIDDEN, bk, sp);
     fill_layer(p.L[0], m->nv, m->nh, bn_v, s->Sv, t->i8 ? e->lds : t->ldkv, m->hb64, t->bias_vf, d_Fv, DOM_BIP_VISIBLE, bk, sp);
@@ -1697,9 +1507,8 @@ static int launch_steps(isb_ens *e, int rule, int fluct_mode, const double *d_Fv
         p.i8_sf[term] = (float)p.i8_sd[term];
     }
     // plane recombination of the fast sampling path (i8_field16): pairs are exact up to K = 65000, all three planes of
-    // 24-bit couplings when the model's row L1 norms allow it; ISB_I8_COMB = 0 | 1 forces the simpler forms (A/B runs)
+    // 24-bit couplings when the model's row L1 norms allow it
     p.i8_comb = std::max(m->nv, m->nh) <= 65000 ? ((t->P == 3 && t->i8_wide) ? 2 : 1) : 0;
-    if (const char *env = getenv("ISB_I8_COMB")) p.i8_comb = std::min(p.i8_comb, std::max(0, atoi(env)));
     p.R = e->R;
     p.P = t->P;
     p.rule = rule;
@@ -1720,12 +1529,15 @@ static int launch_steps(isb_ens *e, int rule, int fluct_mode, const double *d_Fv
     if (persist) {
         p.persist = 1;
         p.sig_fine = 1;
-        if (const char *env = getenv("ISB_TC_FINE")) p.sig_fine = std::max(0, atoi(env));
-        p.rows_per_cta = rows;
+        // A CTA's time per step does not depend on how many of its 128 tile rows hold replicas, and these runs are
+        // POWER-capped (C4: ~1000 W, 1.75 GHz of 1.965): full tiles on fewer SMs do the same work per cycle with fewer
+        // SMs drawing power — 16384 chains as 128 CTAs x 128 rows instead of 148 x 111 measured 0.313 -> 0.326 of the
+        // bf16 burst rate at 1.84 GHz.
+        p.rows_per_cta = TC_BM;
         p.nsteps_seg = (int)nseg;
         p.k0 = k0;
         p.step_abs0 = step_offset + (uint64_t)k0;
-        const int grid = ((e->R + rows - 1) / rows + cg - 1) / cg * cg;  // an odd last CTA gets a peer without replicas
+        const int grid = ((e->R + TC_BM - 1) / TC_BM + 1) / 2 * 2;  // an odd last CTA gets a peer without replicas
         int rc = launch_tc(ctx, maps, p, grid, extf);
         if (rc) return rc;
         e->last_launches += 1;
@@ -1737,7 +1549,7 @@ static int launch_steps(isb_ens *e, int rule, int fluct_mode, const double *d_Fv
             p.layer = layer;
             p.k0 = k;
             p.step_abs0 = step_offset + (uint64_t)k;
-            const int grid = std::min(p.L[layer].n_tiles * p.m_tiles, ctx->num_sms / cg) * cg;
+            const int grid = std::min(p.L[layer].n_tiles * p.m_tiles, ctx->num_sms / 2) * 2;
             int rc = launch_tc(ctx, maps, p, grid, extf);
             if (rc) return rc;
             e->last_launches += 1;
@@ -1884,11 +1696,10 @@ int shard_halfstep_device(isb_model *m, int R, int replica_offset, int layer, in
     int rc = make_map_a(ctx, &maps.A[layer], in_full, m->shard_G, R, m->shard_nb, m->shard_nb, esz);
     if (rc) return rc;
     maps.A[1 - layer] = maps.A[layer];
-    const int cg = tc_cta_group();
-    const int m_tiles = (R + TC_BM * cg - 1) / (TC_BM * cg);
+    const int m_tiles = (R + 2 * TC_BM - 1) / (2 * TC_BM);
     const int sp = t->i8 ? t->P : 1;   // int8: the tile width is part of the stacked storage order
-    const int bn = t->i8 ? t->bn_h : pick_bn_waves(m->shard_nb, m_tiles, ctx->num_sms / cg);
-    rc = get_maps_b(ctx, t, 1, bn * sp / cg, maps.B[1]);  // W is symmetric: one orientation serves both half-steps
+    const int bn = t->i8 ? t->bn_h : pick_bn_waves(m->shard_nb, m_tiles, ctx->num_sms / 2);
+    rc = get_maps_b(ctx, t, 1, bn * sp / 2, maps.B[1]);  // W is symmetric: one orientation serves both half-steps
     if (rc) return rc;
     for (int i = 0; i < TC_PMAX; ++i) maps.B[0][i] = maps.B[1][i];
     TcParams p{};
@@ -1911,7 +1722,6 @@ int shard_halfstep_device(isb_model *m, int R, int replica_offset, int layer, in
         p.i8_sf[term] = (float)p.i8_sd[term];
     }
     p.i8_comb = (int64_t)m->shard_nb * m->shard_G <= 65000 ? 1 : 0;   // (row L1 norms of generated rows are not known here: no all-int32 form)
-    if (const char *env = getenv("ISB_I8_COMB")) p.i8_comb = std::min(p.i8_comb, std::max(0, atoi(env)));
     p.L[1 - layer] = p.L[layer];
     p.R = R;
     p.r_off = replica_offset;
@@ -1928,9 +1738,9 @@ int shard_halfstep_device(isb_model *m, int R, int replica_offset, int layer, in
     p.step_abs0 = step_abs;
     p.persist = 0;
     p.layer = layer;
-    p.cg = cg;
+    p.cg = 2;
     p.m_tiles = m_tiles;
-    const int grid = std::min(p.L[layer].n_tiles * p.m_tiles, ctx->num_sms / cg) * cg;
+    const int grid = std::min(p.L[layer].n_tiles * p.m_tiles, ctx->num_sms / 2) * 2;
     return launch_tc(ctx, maps, p, grid, false);
 }
 

@@ -40,33 +40,12 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity) {
         : "memory");
     return ok != 0;
 }
-// The same with a suspend-time hint (20 us): the waiting thread sleeps instead of polling, which leaves the
-// issue slots to the working warps (measured: +3-4 % on the tcgen05 kernels, -2 % on the sweep kernel, whose
-// chains wait for rows only briefly — so only the former use it).
-__device__ __forceinline__ bool mbar_try_wait_sleep(uint64_t *bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, 0x4E20;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
 // Bounded wait: a protocol bug traps (context error) instead of hanging the GPU.
 __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
     if (mbar_try_wait(bar, parity)) return;
     uint32_t spins = 0;
     while (!mbar_try_wait(bar, parity)) {
         if (++spins > (1u << 22)) __trap();
-    }
-}
-__device__ __forceinline__ void mbar_wait_sleep(uint64_t *bar, uint32_t parity) {
-    if (mbar_try_wait(bar, parity)) return;
-    uint32_t spins = 0;
-    while (!mbar_try_wait_sleep(bar, parity)) {
-        if (++spins > (1u << 20)) __trap();
     }
 }
 // 1-D bulk copy global -> shared, completion signalled on an mbarrier (SASS: UBLKCP).

@@ -1,7 +1,7 @@
 #!/bin/bash
 # Builds an A/B variant of libising_b200.so with extra nvcc flags into scratch_ab/lib_<tag>.so (git-ignored, ships to
 # the GPU box); select it at run time with ISING_B200_LIB=$PWD/scratch_ab/lib_<tag>.so.
-#   scripts/build_variant.sh st4 -DISB_TC_STAGES2=4
+#   scripts/build_variant.sh timing -DISB_TC_TIMING
 set -eu
 tag=$1; shift
 root=$(cd "$(dirname "$0")/.." && pwd)

@@ -68,15 +68,14 @@ def test_i8_trajectories_bit_exact(ctx, orc, synth, monkeypatch, nv, nh, rule, R
     for r in rows:
         s, t, _ = orc.bip_run(rule, Weff, h, b, S0[r], T0[r], nsteps, Fv if shared else Fv[r], Fh if shared else Fh[r], T)
         assert np.array_equal(s, S[r]) and np.array_equal(t, Tm[r]), f"replica {r}"
-    # launch modes and CTA grouping give the same bits
-    for cg, ps in (("1", "0"), ("2", "0")):
-        monkeypatch.setenv("ISB_TC_CG", cg)
+    # both launch modes give the same bits
+    for ps in ("0", "1"):
         monkeypatch.setenv("ISB_TC_PERSIST", ps)
         e2 = L.Ensemble(m, R)
         e2.set_spins(S0)
         e2.set_hidden(T0)
         e2.bip_run(rule, nsteps, Fv=Fv, Fh=Fh, fluct_per_replica=not shared, T=T)
-        assert np.array_equal(e2.get_spins(), S) and np.array_equal(e2.get_hidden(), Tm), (cg, ps)
+        assert np.array_equal(e2.get_spins(), S) and np.array_equal(e2.get_hidden(), Tm), ps
 
 
 @pytest.mark.parametrize("rule", [0, 1])

@@ -500,8 +500,8 @@ def test_bip_tc_philox_matches_f64_path(ctx, synth):
 
 def test_bip_tc_fp16_terms(ctx, synth, monkeypatch):
     """ISB_PREC_FP16X2 / _FP16X1: fp16 terms of the power-of-two pre-scaled couplings.  Integer W is exact in one fp16
-    term, so the trajectory must equal the Float64 path's bit for bit (T = 0 and caller-supplied noise, single CTAs
-    and pairs, both launch modes); for Gaussian W the two-term split represents W to 2^-24 of max|W| (as good as W
+    term, so the trajectory must equal the Float64 path's bit for bit (T = 0 and caller-supplied noise, both launch
+    modes); for Gaussian W the two-term split represents W to 2^-24 of max|W| (as good as W
     rounded to float), so with the same noise words almost every chain follows the Float64 trajectory, exactly as
     with three bf16 terms."""
     L = _lib()
@@ -518,16 +518,14 @@ def test_bip_tc_fp16_terms(ctx, synth, monkeypatch):
         e.bip_run(0, 3, **kw)
         ref[kw_name] = (e.get_spins(), e.get_hidden())
         for prec in (L.PREC_FP16X1, L.PREC_FP16X2):
-            for cg, persist in (("1", "0"), ("2", "0"), ("2", "1")):
-                monkeypatch.setenv("ISB_TC_CG", cg)
+            for persist in ("0", "1"):
                 monkeypatch.setenv("ISB_TC_PERSIST", persist)
                 e = L.Ensemble(L.Model.bipartite(ctx, W, h, b, prec), R)
                 e.set_spins(S0)
                 e.set_hidden(T0)
                 e.bip_run(0, 3, **kw)
-                assert np.array_equal(e.get_spins(), ref[kw_name][0]), (kw_name, prec, cg, persist)
-                assert np.array_equal(e.get_hidden(), ref[kw_name][1]), (kw_name, prec, cg, persist)
-    monkeypatch.delenv("ISB_TC_CG")
+                assert np.array_equal(e.get_spins(), ref[kw_name][0]), (kw_name, prec, persist)
+                assert np.array_equal(e.get_hidden(), ref[kw_name][1]), (kw_name, prec, persist)
     monkeypatch.delenv("ISB_TC_PERSIST")
     W, h, b = synth.bipartite_W(nv, nh, 127, 0.1)
     En = {}
@@ -547,10 +545,11 @@ def test_bip_tc_fp16_terms(ctx, synth, monkeypatch):
         L.Model.shard_sk(ctx, 256, 2, 0, 1, 1.0, prec=L.PREC_FP16X2)
 
 
-@pytest.mark.parametrize("R,nv,nh", [(300, 160, 96), (19500, 96, 80), (1000, 784, 512)])
+@pytest.mark.parametrize("R,nv,nh", [(300, 160, 96), (19500, 96, 80), (1000, 784, 512), (130, 784, 512), (1, 24, 17)])
 def test_bip_tc_chain_resident_equals_per_half_step_launches(ctx, synth, monkeypatch, R, nv, nh):
     """The chain-resident persistent kernel (one launch for all steps, each CTA keeps its replicas) must give
-    exactly what the one-launch-per-half-step path gives: same tiles, same K order, same noise words."""
+    exactly what the one-launch-per-half-step path gives: same tiles, same K order, same noise words.  R = 130 / R = 1
+    leave the second CTA of a pair (almost) without replicas."""
     L = _lib()
     W, h, b = synth.bipartite_W(nv, nh, 101, 0.2)
     S0, T0 = synth.spins(102, R, nv), synth.spins(103, R, nh)
@@ -558,21 +557,17 @@ def test_bip_tc_chain_resident_equals_per_half_step_launches(ctx, synth, monkeyp
     T = synth.geometric_schedule(1.5, 0.4, nsteps)
     for rule in (0, 1):
         res = []
-        # chain-resident mode with progress published per tile ("0"), per round of columns in the last tile ("1")
-        # and in every tile ("99")
-        for persist, fine in (("0", "1"), ("1", "0"), ("1", "1"), ("1", "99")):
+        for persist in ("0", "1"):
             monkeypatch.setenv("ISB_TC_PERSIST", persist)
-            monkeypatch.setenv("ISB_TC_FINE", fine)
             e = L.Ensemble(L.Model.bipartite(ctx, W, h, b, L.PREC_BF16X3), R)
             e.set_spins(S0)
             e.set_hidden(T0)
             E = e.bip_run(rule, nsteps, seed=42, step_offset=7, T=T, trace_every=2)
             res.append((e.get_spins(), e.get_hidden(), E, e.last_stats()["launches"]))
-        for other in res[1:]:
-            assert np.array_equal(res[0][0], other[0]) and np.array_equal(res[0][1], other[1])
-            assert np.array_equal(res[0][2], other[2])
-            assert other[3] < res[0][3]  # fewer launches in chain-resident mode
-    monkeypatch.delenv("ISB_TC_FINE")
+        half_steps, resident = res
+        assert np.array_equal(half_steps[0], resident[0]) and np.array_equal(half_steps[1], resident[1])
+        assert np.array_equal(half_steps[2], resident[2])
+        assert resident[3] < half_steps[3]  # fewer launches in chain-resident mode
     # caller-supplied fluctuations through the chain-resident kernel vs the oracle-checked exact path at T = 0
     monkeypatch.setenv("ISB_TC_PERSIST", "1")
     if R <= 1000:
@@ -590,32 +585,41 @@ def test_bip_tc_chain_resident_equals_per_half_step_launches(ctx, synth, monkeyp
 
 
 @pytest.mark.parametrize("R,nv,nh", [(300, 160, 96), (130, 784, 512), (1, 24, 17), (19500, 96, 80)])
-def test_bip_tc_cta_pairs_equal_single_ctas(ctx, synth, monkeypatch, R, nv, nh):
-    """cta_group::2 (two CTAs share one M = 256 MMA, each loads half of the coupling tile) must reproduce the
-    single-CTA kernel bit for bit: same K order, same noise words; in both launch modes, for both rules, with
-    in-kernel and caller-supplied noise.  R = 130 / R = 1 leave the second CTA of a pair (almost) without replicas."""
+def test_bip_tc_cta_pairs_equal_f64_path(ctx, synth, monkeypatch, R, nv, nh):
+    """The tensor-core kernel runs in CTA pairs (cta_group::2: two CTAs share one M = 256 MMA, each loads half of the
+    coupling tile).  Integer couplings are exact in bf16 terms and on the int8 grid, so the pair kernel must reproduce
+    the Float64 path bit for bit in spins, hidden layer and traced energies: in both launch modes, for both rules, with
+    caller-supplied noise at T > 0 and with in-kernel Philox noise at T = 0 (where the noise drops out).  R = 130 / R = 1
+    leave the second CTA of a pair (almost) without replicas."""
     L = _lib()
-    W, h, b = synth.bipartite_W(nv, nh, 111, 0.2)
+    W = np.round(synth.gaussian(111, nv * nh).reshape(nv, nh) * 1.5)
+    h, b = np.round(synth.gaussian(115, nv)), np.round(synth.gaussian(116, nh))
     S0, T0 = synth.spins(112, R, nv), synth.spins(113, R, nh)
     nsteps = 4
-    T = synth.geometric_schedule(1.5, 0.4, nsteps)
     Fv, Fh = synth.logistic(114, (nsteps, nv), 1), synth.logistic(114, (nsteps, nh), 2)
-    for prec in (L.PREC_BF16X3, L.PREC_BF16X1):
-        m = L.Model.bipartite(ctx, W, h, b, prec)
-        for rule in (0, 1):
-            for kw in (dict(seed=42, step_offset=7), dict(Fv=Fv, Fh=Fh)):
-                res = []
-                for cg, persist in (("1", "0"), ("2", "0"), ("2", "1")):
-                    monkeypatch.setenv("ISB_TC_CG", cg)
+    runs = (dict(Fv=Fv, Fh=Fh, T=synth.geometric_schedule(1.5, 0.4, nsteps)),
+            dict(seed=42, step_offset=7, T=np.zeros(nsteps)))
+
+    def run(m, rule, kw):
+        e = L.Ensemble(m, R)
+        e.set_spins(S0)
+        e.set_hidden(T0)
+        E = e.bip_run(rule, nsteps, trace_every=2, **kw)
+        return e.get_spins(), e.get_hidden(), E
+
+    ref_model = L.Model.bipartite(ctx, W, h, b, L.PREC_F64)
+    models = {prec: L.Model.bipartite(ctx, W, h, b, prec) for prec in (L.PREC_BF16X3, L.PREC_BF16X1, L.PREC_I8X3)}
+    for m in models.values():
+        assert np.array_equal(m.effective_couplings(), W)
+    for rule in (0, 1):
+        for i, kw in enumerate(runs):
+            ref = run(ref_model, rule, kw)
+            for prec, m in models.items():
+                for persist in ("0", "1"):
                     monkeypatch.setenv("ISB_TC_PERSIST", persist)
-                    e = L.Ensemble(m, R)
-                    e.set_spins(S0)
-                    e.set_hidden(T0)
-                    E = e.bip_run(rule, nsteps, T=T, trace_every=2, **kw)
-                    res.append((e.get_spins(), e.get_hidden(), E))
-                for other in res[1:]:
-                    assert np.array_equal(res[0][0], other[0]) and np.array_equal(res[0][1], other[1])
-                    assert np.array_equal(res[0][2], other[2])
+                    S, Tm, E = run(m, rule, kw)
+                    assert np.array_equal(S, ref[0]) and np.array_equal(Tm, ref[1]), (rule, i, prec, persist)
+                    assert np.array_equal(E, ref[2]), (rule, i, prec, persist)
 
 
 # ---------------------------------------------------------------- edge cases
