@@ -248,6 +248,40 @@ int isb_ssf_run_pa(isb_ens *e, int rule, int n_pop, int64_t nT, const double *T,
                    int order, int start, uint64_t seed, uint64_t step_offset, uint64_t T_offset, int32_t *family,
                    double *out_E, double *out_M, double *out_lnQ, int64_t *out_flips);
 
+/* Swendsen-Wang cluster sweeps of an ensemble of a SPARSE model (isb_model_sparse: any graph, periodic lattices included;
+ * n <= 16384 sites, ISB_ERR_UNSUPPORTED above; dense and bipartite ensembles: ISB_ERR_STATE).  Energy convention as
+ * everywhere: E = -sum_{i<j} J_ij s_i s_j - sum_i h_i s_i.  Sweep k of the call (absolute index K = sweep_offset + k) of
+ * replica r runs at T_r(k) = Tsched[k / sweeps_per_T] * scale[r] (the isb_ens_set_temperature_scale factors, 1 when unset),
+ * the product isb_ssf_run forms:
+ *   bonds     the pairs (i, j), i < j, J_ij != 0 after the constructor's symmetrisation, numbered e = 0, 1, ... in order
+ *             of i, then j (row i of the stored CSR, columns > i).  Bond e is active when J_ij s_i s_j > 0 and
+ *             u(w_e) < 1 - exp(-2|J_ij| / T_r(k)), w_e = word e & 3 of Philox4x32-10(counter (lo32 K, hi32 K, r,
+ *             7 << 28 | e >> 2), key seed), u(w) = (w + 1/2) 2^-32; exp in double, IEEE round-to-nearest, no contraction;
+ *   clusters  the connected components of the active bonds; the ROOT of a cluster is its smallest site;
+ *   fields    on a grid, so that the cluster sums are exact and independent of order: e_h = the smallest integer with
+ *             max|h| <= 2^e_h, q = 2^(e_h - 30), hq_i = rint(h_i / q) (every hq_i = 0 when h = 0).  The chain samples the
+ *             Boltzmann distribution of the fields q hq, which differ from h by at most 2^-31 max|h| each;
+ *   flips     for cluster C with root rho: S_C = sum_{i in C} hq_i s_i (exact int64), x = 2 q S_C / T_r(k),
+ *             P = 1 / (1 + exp(x)); every spin of C flips when u(z) < P, z = word rho & 3 of Philox4x32-10(counter
+ *             (lo32 K, hi32 K, r, 8 << 28 | rho >> 2), key seed).  P = 1/2 exactly when h = 0.  This is the heat-bath
+ *             choice of each cluster's orientation given its bonds: detailed balance holds with fields and with couplings
+ *             of either sign.
+ * The device's double exp and a replay's may differ by an ulp: a decision can differ only when u falls between the two,
+ * with probability of order 2^-53 per decision.
+ *   out_E, out_M   [nsweeps / trace_every][R]: energy (in double, exact for dyadic J and h; its summation order differs from
+ *                  isb_ens_energy) and magnetisation after the flips of every trace_every-th sweep;
+ *   out_csq        same shape: sum over that sweep's clusters of |C|^2, the improved estimator of the susceptibility
+ *                  (chi = <sum |C|^2> / N at h = 0);
+ *   out_flips      [R]: spins flipped during the call.
+ * Every output may be NULL.  ISB_ERR_ARG: nsweeps < 0, sweeps_per_T < 1, trace_every < 0 or, when nsweeps > 0, no schedule
+ * (nT < 1), a schedule shorter than nsweeps (nT * sweeps_per_T < nsweeps) or a temperature T_r(k) <= 0 the call would use;
+ * ISB_ERR_NONFINITE: a non-finite one.  An error leaves the ensemble unchanged; nsweeps = 0 is a no-op.  The result is
+ * bit-identical from run to run and does not depend on the launch configuration; two calls (sweep_offset and schedule
+ * continued) equal one call.  The cached fields of the single-spin kernels are rebuilt by the next isb_ssf_run. */
+int isb_sw_run(isb_ens *e, int64_t nsweeps, uint64_t seed, uint64_t sweep_offset, const double *Tsched, int64_t nT,
+               int64_t sweeps_per_T, int64_t trace_every, double *out_E, double *out_M, int64_t *out_csq,
+               int64_t *out_flips);
+
 /* Fluctuations exactly as ISB_FLUCT_PHILOX generates them inside isb_ssf_run, for parity tests:
  * out[r*nsteps + k], r in [r0, r0+nr). rule selects the transform. prec as the model's. */
 int isb_philox_fluct(isb_ctx *ctx, int rule, int prec, uint64_t seed, uint64_t step_offset,

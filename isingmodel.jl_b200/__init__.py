@@ -7,8 +7,9 @@ There is no CPU fallback: without the built library or without a CUDA device eve
 """
 from . import _lib  # noqa: F401
 from . import SpinSystems, SingleSpinFlip, OnBipartiteGraph, MultiSpinFlip, SamplingHelper  # noqa: F401
-from . import sharding, rowshard, tempering  # noqa: F401
+from . import sharding, rowshard, tempering, cluster  # noqa: F401
+from .cluster import SwendsenWang  # noqa: F401
 from ._lib import IsbError, build, context  # noqa: F401
 
 __all__ = ["SpinSystems", "SingleSpinFlip", "MultiSpinFlip", "OnBipartiteGraph", "SamplingHelper", "sharding", "rowshard", "tempering",
-           "IsbError", "build", "context"]
+           "cluster", "SwendsenWang", "IsbError", "build", "context"]

@@ -87,6 +87,7 @@ SIGNATURES = {
     "isb_ssf_run_hist": (_i, [_vp, _i, _i64, _i, _vp, _i, _i, _vp, _u64, _u64, _vp, _i64, _i64, _i64, _vp]),
     "isb_ssf_run_pt": (_i, [_vp, _i, _i, _vp, _i64, _i64, _i, _i, _u64, _u64, _u64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "isb_ssf_run_pa": (_i, [_vp, _i, _i, _i64, _vp, _d, _i64, _i, _i, _u64, _u64, _u64, _vp, _vp, _vp, _vp, _vp]),
+    "isb_sw_run": (_i, [_vp, _i64, _u64, _u64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp]),
     "isb_philox_fluct": (_i, [_vp, _i, _i, _u64, _u64, _i, _i, _i64, _vp]),
     "isb_philox_nodes": (_i, [_vp, _i, _u64, _u64, _i64, _vp]),
     "isb_philox_raw": (_i, [_vp, _vp, _vp, _i, _vp]),
@@ -583,6 +584,22 @@ class Ensemble:
                                         int(order), int(start), int(seed), int(step_offset), int(T_offset), ptr(fam),
                                         ptr(E), ptr(M), ptr(lnQ), ptr(flips)))
         return {"E": E, "M": M, "lnQ": lnQ, "family": fam, "flips": flips}
+
+    def sw_run(self, nsweeps, T, *, sweeps_per_T=1, trace_every=0, seed=0, sweep_offset=0, want_E=True, want_M=True,
+               want_csq=True):
+        """isb_sw_run: ``nsweeps`` Swendsen-Wang sweeps of every replica (sparse models), sweep k at T[k // sweeps_per_T]
+        times the replica's temperature factor.  Returns dict(E / M [ntr][R] float64 | None, csq [ntr][R] int64 | None
+        (sum of |C|^2 over the clusters of the traced sweep), flips[R]); ntr = nsweeps // trace_every."""
+        nsweeps = int(nsweeps)
+        Ta = np.ascontiguousarray(np.atleast_1d(T), dtype=np.float64).reshape(-1)
+        ntr = nsweeps // trace_every if trace_every > 0 else 0
+        E = np.zeros((ntr, self.R)) if (ntr and want_E) else None
+        M = np.zeros((ntr, self.R)) if (ntr and want_M) else None
+        csq = np.zeros((ntr, self.R), dtype=np.int64) if (ntr and want_csq) else None
+        flips = np.zeros(self.R, dtype=np.int64)
+        self._chk(load().isb_sw_run(self.handle, nsweeps, int(seed), int(sweep_offset), ptr(Ta), Ta.size, int(sweeps_per_T),
+                                    int(trace_every), ptr(E), ptr(M), ptr(csq), ptr(flips)))
+        return {"E": E, "M": M, "csq": csq, "flips": flips}
 
     def bip_run(self, rule, nsteps, *, Fv=None, Fh=None, fluct_per_replica=False, seed=0, step_offset=0, T=None,
                 steps_per_T=1, trace_every=0, want_S=False):

@@ -1178,6 +1178,82 @@ int isb_ssf_run_pa(isb_ens *e, int rule, int n_pop, int64_t nT, const double *T,
     return finish_ssf_run(e, who, d.flips_total, out_flips);
 }
 
+int isb_sw_run(isb_ens *e, int64_t nsweeps, uint64_t seed, uint64_t sweep_offset, const double *Tsched, int64_t nT,
+               int64_t sweeps_per_T, int64_t trace_every, double *out_E, double *out_M, int64_t *out_csq,
+               int64_t *out_flips) {
+    if (!e) return ISB_ERR_ARG;
+    isb_model *m = e->model;
+    isb_ctx *ctx = m->ctx;
+    ISB_LOCK(ctx);
+    const char *who = "isb_sw_run";
+    if (m->kind != ISB_KIND_SPARSE) return fail(ctx, ISB_ERR_STATE, "%s: not an ensemble of a sparse model", who);
+    if (m->n > isb::SW_MAX_N)
+        return fail(ctx, ISB_ERR_UNSUPPORTED, "%s: n = %d sites > %d (the labels live in shared memory)", who, m->n,
+                    isb::SW_MAX_N);
+    if (nsweeps < 0) return fail(ctx, ISB_ERR_ARG, "%s: nsweeps = %lld is negative", who, (long long)nsweeps);
+    if (sweeps_per_T < 1) return fail(ctx, ISB_ERR_ARG, "%s: sweeps_per_T = %lld must be positive", who, (long long)sweeps_per_T);
+    if (trace_every < 0) return fail(ctx, ISB_ERR_ARG, "%s: trace_every is negative", who);
+    const int64_t nused = (nsweeps + sweeps_per_T - 1) / sweeps_per_T;   // schedule entries the call reads
+    if (nsweeps > 0) {
+        if (!Tsched || nT < 1) return fail(ctx, ISB_ERR_ARG, "%s: a temperature schedule is required", who);
+        if (nused > nT)
+            return fail(ctx, ISB_ERR_ARG, "%s: schedule of %lld entries x %lld sweeps is shorter than %lld sweeps", who,
+                        (long long)nT, (long long)sweeps_per_T, (long long)nsweeps);
+        if (!all_finite(Tsched, (size_t)nused)) return fail(ctx, ISB_ERR_NONFINITE, "%s: non-finite temperature", who);
+        double tmin = Tsched[0], tmax = Tsched[0];
+        for (int64_t k = 0; k < nused; ++k) {
+            if (!(Tsched[k] > 0.0))
+                return fail(ctx, ISB_ERR_ARG, "%s: Tsched[%lld] = %g must be positive", who, (long long)k, Tsched[k]);
+            tmin = std::min(tmin, Tsched[k]);
+            tmax = std::max(tmax, Tsched[k]);
+        }
+        if (e->d_tscale) {   // the temperatures the replicas run at: Tsched[k] * scale[r]
+            std::vector<double> sc((size_t)e->R);
+            ISB_CUDA(ctx, cudaSetDevice(ctx->device));
+            ISB_TRY(d2h(ctx, sc.data(), e->d_tscale, sc.size() * sizeof(double), nullptr));
+            ISB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            for (int r = 0; r < e->R; ++r) {
+                const double lo = tmin * sc[r], hi = tmax * sc[r];
+                if (!std::isfinite(lo) || !std::isfinite(hi))
+                    return fail(ctx, ISB_ERR_NONFINITE, "%s: non-finite temperature of replica %d", who, r);
+                if (!(lo > 0.0) || !(hi > 0.0))
+                    return fail(ctx, ISB_ERR_ARG, "%s: replica %d runs at a temperature <= 0 (factor %g)", who, r, sc[r]);
+            }
+        }
+    }
+    ISB_CUDA(ctx, cudaSetDevice(ctx->device));
+    begin_stats(e);
+    if (nsweeps == 0) {
+        if (out_flips) std::fill(out_flips, out_flips + e->R, (int64_t)0);
+        return ISB_OK;
+    }
+    ISB_TRY(isb::sw_model_prepare(m));
+
+    const size_t R = (size_t)e->R;
+    const int64_t ntr = trace_every > 0 ? nsweeps / trace_every : 0;
+    double *d_T = nullptr, *d_E = nullptr, *d_M = nullptr;
+    int64_t *d_csq = nullptr;
+    ISB_TRY(isb::dev_reserve(ctx, isb::SCR_T, (size_t)nused * sizeof(double), (void **)&d_T));
+    ISB_TRY(h2d(ctx, d_T, Tsched, (size_t)nused * sizeof(double), &e->last_h2d));
+    if (ntr > 0 && out_E) ISB_TRY(isb::dev_reserve(ctx, isb::SCR_E, (size_t)ntr * R * sizeof(double), (void **)&d_E));
+    if (ntr > 0 && out_M) ISB_TRY(isb::dev_reserve(ctx, isb::SCR_M, (size_t)ntr * R * sizeof(double), (void **)&d_M));
+    if (ntr > 0 && out_csq)
+        ISB_TRY(isb::dev_reserve(ctx, isb::SCR_SW_CSQ, (size_t)ntr * R * sizeof(int64_t), (void **)&d_csq));
+    ISB_CUDA(ctx, cudaMemsetAsync(e->d_counters, 0, 4 * sizeof(unsigned long long), ctx->stream));
+    // the spins change under the cached fields of the single-spin kernels
+    e->fields_rule_sign = 0;
+    e->ifields_ok = false;
+
+    ISB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    ISB_TRY(isb::sw_run_device(e, nsweeps, seed, sweep_offset, d_T, sweeps_per_T, trace_every, d_E, d_M, d_csq));
+    ISB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+
+    if (d_E) ISB_TRY(d2h(ctx, out_E, d_E, (size_t)ntr * R * sizeof(double), &e->last_d2h));
+    if (d_M) ISB_TRY(d2h(ctx, out_M, d_M, (size_t)ntr * R * sizeof(double), &e->last_d2h));
+    if (d_csq) ISB_TRY(d2h(ctx, out_csq, d_csq, (size_t)ntr * R * sizeof(int64_t), &e->last_d2h));
+    return finish_ssf_run(e, who, e->d_flips, out_flips);
+}
+
 int isb_philox_fluct(isb_ctx *ctx, int rule, int prec, uint64_t seed, uint64_t step_offset, int r0, int nr,
                      int64_t nsteps, double *out) {
     (void)prec;

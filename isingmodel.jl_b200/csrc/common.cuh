@@ -138,11 +138,14 @@ __host__ __device__ __forceinline__ uint32_t philox_pick(const Philox4 &p, uint3
 
 // Stream domains (top 4 bits of counter word 3).
 enum : uint32_t { DOM_SSF_FLUCT = 1, DOM_SSF_NODES = 2, DOM_BIP_VISIBLE = 3, DOM_BIP_HIDDEN = 4, DOM_PT_SWAP = 5,
-                  DOM_PA_RESAMPLE = 6 };
+                  DOM_PA_RESAMPLE = 6, DOM_SW_BOND = 7, DOM_SW_FLIP = 8 };
 // Replica-exchange decisions (isb_ssf_run_pt): word .x of counter (lo(K), hi(K), ladder, DOM_PT_SWAP<<28 | lo) decides the
 // swap of levels (lo, lo+1) in that ladder after absolute round K.
 // Population-annealing resampling (isb_ssf_run_pa): word .x of counter (lo(K), hi(K), population, DOM_PA_RESAMPLE<<28) is
 // the offset U of the systematic resampling of that population after absolute temperature step K.
+// Swendsen-Wang sweeps (isb_sw_run): word e & 3 of counter (lo(K), hi(K), replica, DOM_SW_BOND<<28 | e >> 2) decides bond e
+// in absolute sweep K, word rho & 3 of counter (lo(K), hi(K), replica, DOM_SW_FLIP<<28 | rho >> 2) the flip of the cluster
+// whose smallest site is rho.
 
 // Word assigned to step `step` of replica `replica` in a single-spin run:
 // counter = (lo(step>>2), hi(step>>2), replica, domain<<28), key = seed, word = step & 3.

@@ -22,7 +22,7 @@ struct isb_ctx {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    isb_devbuf scratch[18];      // grow-only device staging buffers (see isb::dev_reserve)
+    isb_devbuf scratch[19];      // grow-only device staging buffers (see isb::dev_reserve)
     // Every entry point that uses the stream, the events or the scratch buffers holds this lock for its whole
     // (synchronous) duration: calls on one context are serialised, different contexts run concurrently.
     std::recursive_mutex mtx;
@@ -119,7 +119,7 @@ double ssf_guard_from(const double *absrowsum, const double *vals, size_t nvals,
 int dev_reserve(isb_ctx *ctx, int slot, size_t bytes, void **out);
 enum { SCR_NODES = 0, SCR_FLUCT = 1, SCR_T = 2, SCR_E = 3, SCR_M = 4, SCR_FLUCT2 = 5, SCR_OUT = 6, SCR_TMP = 7,
        SCR_TC0 = 8, SCR_TC1 = 9, SCR_S = 10, SCR_S2 = 11, SCR_HIST = 12, SCR_PT_STATE = 13, SCR_PT_E = 14, SCR_PT_M = 15,
-       SCR_PT_Q = 16, SCR_PA_STATE = 17 };
+       SCR_PT_Q = 16, SCR_PA_STATE = 17, SCR_SW_CSQ = 18 };
 
 #define ISB_LOCK(ctx) std::lock_guard<std::recursive_mutex> isb_lock_guard_((ctx)->mtx)
 
@@ -169,6 +169,27 @@ int ssf_sparse_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const
 #include <utility>
 #include <vector>
 namespace isb {
+// isb_model::sp of a sparse model (kind SPARSE), built by sparse_model_init
+struct SparseModel {
+    int64_t nnz = 0;
+    int *rowptr = nullptr;   // [n+1]
+    int *col = nullptr;      // [nnz] ascending within a row
+    double *val = nullptr;   // [nnz]
+    int maxdeg = 0;
+    void *lattice = nullptr;  // periodic square lattice recognised: sequential sweeps run in lattice.cu
+    std::vector<double> ars;  // row sums of |J| (near-tie guard, completed with |h| by the caller)
+    std::vector<double> vals;
+    // Swendsen-Wang sweeps (cluster.cu), built by the first isb_sw_run on the model: the bonds (i, j), i < j, J_ij != 0,
+    // in the order of row i then column j, as i << 16 | j and J_ij; the fields on the grid q * hq (hq_i = rint(h_i / q))
+    bool sw_ready = false;
+    int64_t sw_nbonds = 0;
+    uint32_t *sw_pair = nullptr;  // [nbonds]
+    double *sw_J = nullptr;       // [nbonds]
+    int32_t *sw_hq = nullptr;     // [n]
+    double sw_q = 1.0;
+    bool sw_has_h = false;
+};
+
 void *lattice_detect(isb_ctx *ctx, int n, const std::vector<std::vector<std::pair<int, double>>> &rows);
 void lattice_free(void *lat);
 int lattice_side(const void *lat);
@@ -199,6 +220,16 @@ struct PaDevice {
 int ssf_pa_run_device(isb_ens *e, int rule, int n_pop, int64_t nT, const double *db, int64_t n_res, int64_t steps_per_T,
                       int order, int start, uint64_t seed, uint64_t step_offset, uint64_t T_offset, const PaDevice &d,
                       int *fam_final);
+
+// cluster.cu: Swendsen-Wang sweeps of a sparse ensemble (isb_sw_run), on arguments the entry point has checked.
+constexpr int SW_MAX_N = 16384;
+struct SparseModel;
+int sw_model_prepare(isb_model *m);   // the bond list and the field grid (once per model; caller holds the context lock)
+void sw_model_free(SparseModel *sm);
+// one launch: nsweeps sweeps, T_r(k) = d_T[k / sweeps_per_T] * tscale[r]; traces [nsweeps / trace_every][R] (NULL: not
+// recorded), flips per replica into e->d_flips
+int sw_run_device(isb_ens *e, int64_t nsweeps, uint64_t seed, uint64_t sweep_offset, const double *d_T,
+                  int64_t sweeps_per_T, int64_t trace_every, double *d_E, double *d_M, int64_t *d_csq);
 
 // bip_exact.cu
 int bip_run_exact_device(isb_ens *e, int rule, int64_t nsteps, int fluct_mode, const double *d_Fv,

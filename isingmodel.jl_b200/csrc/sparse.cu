@@ -19,17 +19,6 @@
 
 namespace isb {
 
-struct SparseModel {
-    int64_t nnz = 0;
-    int *rowptr = nullptr;   // [n+1]
-    int *col = nullptr;      // [nnz] ascending within a row
-    double *val = nullptr;   // [nnz]
-    int maxdeg = 0;
-    void *lattice = nullptr;  // periodic square lattice recognised: sequential sweeps run in lattice.cu
-    std::vector<double> ars;  // row sums of |J| (near-tie guard, completed with |h| by the caller)
-    std::vector<double> vals;
-};
-
 struct SpParams {
     const int *rowptr;
     const int *col;
@@ -339,6 +328,7 @@ void sparse_model_free(isb_model *m) {
     cudaFree(sm->rowptr);
     cudaFree(sm->col);
     cudaFree(sm->val);
+    sw_model_free(sm);
     lattice_free(sm->lattice);
     delete sm;
     m->sp = nullptr;

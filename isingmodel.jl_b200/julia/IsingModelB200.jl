@@ -169,6 +169,20 @@ function ssf_run_pa!(e, rule, n_pop, T, steps_per_T; T_next = 0.0, order = ORDER
           context())
     family
 end
+# Swendsen-Wang cluster sweeps of a sparse ensemble (isb_sw_run): sweep k at T[k ÷ sweeps_per_T + 1] (a scalar T: every
+# sweep) times the replica's temperature factor.  E / M / csq: R x (nsweeps ÷ trace_every) (column-major == the ABI's
+# [ntr][R]; csq = sum of |C|^2 over the clusters of the traced sweep), flips: R.
+function sw_run!(e, nsweeps, T; seed = 0, sweep_offset = 0, sweeps_per_T = 1, trace_every = 0, E = nothing, M = nothing,
+                 csq = nothing, flips = nothing)
+    Tv = T isa Real ? [Float64(T)] : Vector{Float64}(T)
+    spT = T isa Real ? max(nsweeps, 1) : sweeps_per_T
+    check(ccall((:isb_sw_run, libisb), Cint,
+                (Ens, Int64, UInt64, UInt64, Ptr{Float64}, Int64, Int64, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64},
+                 Ptr{Int64}),
+                e, nsweeps, seed, sweep_offset, Tv, length(Tv), spT, trace_every, _optr(E, Float64), _optr(M, Float64),
+                _optr(csq, Int64), _optr(flips, Int64)), context())
+    e
+end
 # Fv / Fh: (units, steps) column-major == [steps][units].  With snapV / snapH (units x R x ntr Int8) the call is
 # isb_bip_run_snap.
 function bip_run!(e, rule, nsteps; Fv = nothing, Fh = nothing, per_replica = false, seed = 0, step_offset = 0,
