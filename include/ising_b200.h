@@ -327,8 +327,8 @@ int isb_philox_bip_fluct(isb_ctx *ctx, int rule, int prec, uint64_t seed, uint64
  * (src/OnBipartiteGraph.jl:30-43) on the embedding W = (J + qI)/2, h/2, h/2, sigma = tau = s (demo.jl:82-90),
  * with W too large for one GPU.  Rank `block` of `n_blocks` owns the output units
  * [block*nb, (block+1)*nb), nb = n / n_blocks, of BOTH half-steps (W is symmetric) and holds only W[block rows, :].
- * The spin matrices live in CALLER-OWNED device buffers (the host layer allocates them with its tensor library
- * and all-gathers them over NCCL / NVLink between half-steps):
+ * The spin matrices live in CALLER-OWNED device buffers (the caller allocates them and gathers the sampled blocks
+ * of every rank between half-steps; isb_shard_run_* below does both):
  *   full layer  : bf16 [n_blocks][R][nb]   (block-major, +1/-1)        — the K operand of a half-step
  *   own block   : bf16 [R][nb], one buffer per layer                    — what this rank samples (on entry it
  *                 holds the block's previous values, which MomentumAnnealing multiplies into the noise)
@@ -353,19 +353,10 @@ int isb_model_shard_block(const isb_model *m); /* nb, 0 for other models */
 /* One half-step of this rank's block (layer 1: hidden from the full visible layer, 0: visible from the full
  * hidden layer): own <- sgn+(2 (W[block,:] . in + bias) - F T [.* own]) for all R replicas.  All pointers are
  * DEVICE pointers on the context's device; the kernel is enqueued on the context's stream (isb_set_stream). */
-/* R replicas whose global indices start at replica_offset (the host layer may split the replicas into groups
- * and pipeline one group's exchange under the other group's GEMM: chains are independent). */
+/* R replicas whose global indices start at replica_offset (isb_shard_run_* splits the replicas into two groups and
+ * hides one group's exchange under the other group's GEMM: chains are independent). */
 int isb_shard_halfstep_dev(isb_model *m, int R, int replica_offset, int layer, int rule,
-                           const void *in_full_bf16, void *out_block_bf16, uint64_t seed, uint64_t step_abs,
-                           double T);
-/* The same half-step with the all-gather FUSED into the sampling epilogue: every sampled 16-unit run is also
- * stored, tile by tile while the next tile's MMAs run, straight into the gathered matrices of up to 7 peer GPUs
- * through peer-mapped (NVLink) device pointers.  peer_blocks_bf16[q] is the address, in THIS process, of the
- * [R][nb] slab of peer q's gathered layer that belongs to this rank (block-major layout: base_q + block*R*nb).
- * The caller separates half-steps with a cross-GPU barrier instead of an all-gather. */
-int isb_shard_halfstep_fused_dev(isb_model *m, int R, int replica_offset, int layer, int rule,
-                                 const void *in_full_bf16, void *out_block_bf16, int n_peers,
-                                 void *const *peer_blocks_bf16, uint64_t seed, uint64_t step_abs, double T);
+                           const void *in_full, void *out_block, uint64_t seed, uint64_t step_abs, double T);
 
 /* The step loop of the row-sharded SCA inside the library (no torch, no Python on the path): one run object per rank
  * owns the gathered spin matrices and this rank's blocks, splits the replicas into two groups and hides one group's

@@ -100,7 +100,6 @@ SIGNATURES = {
     "isb_sk_rows": (_i, [_vp, _i, _u64, _i, _i, _vp]),
     "isb_model_shard_block": (_i, [_vp]),
     "isb_shard_halfstep_dev": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _u64, _u64, _d]),
-    "isb_shard_halfstep_fused_dev": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _i, _vp, _u64, _u64, _d]),
     "isb_shard_run_create": (_i, [_vp, _i, _i, C.POINTER(_vp)]),
     "isb_shard_run_destroy": (None, [_vp]),
     "isb_nccl_unique_id": (_i, [_vp]),
@@ -300,14 +299,6 @@ class Model:
         """isb_shard_halfstep_dev with raw device pointers (ints)."""
         check(load().isb_shard_halfstep_dev(self.handle, int(R), int(replica_offset), int(layer), int(rule), _vp(in_full_ptr),
                                             _vp(out_block_ptr), int(seed), int(step_abs), float(T)), self.ctx.handle)
-
-    def shard_halfstep_fused(self, R, layer, rule, in_full_ptr, out_block_ptr, peer_ptrs, seed, step_abs, T,
-                             replica_offset=0):
-        """isb_shard_halfstep_fused_dev: peer_ptrs = device addresses of this rank's slab in each peer's matrix."""
-        arr = (C.c_void_p * max(1, len(peer_ptrs)))(*[int(x) for x in peer_ptrs])
-        check(load().isb_shard_halfstep_fused_dev(self.handle, int(R), int(replica_offset), int(layer), int(rule), _vp(in_full_ptr),
-                                                  _vp(out_block_ptr), len(peer_ptrs), C.cast(arr, _vp), int(seed),
-                                                  int(step_abs), float(T)), self.ctx.handle)
 
     def effective_couplings(self):
         """The couplings exactly as the kernels use them (isb_model_effective_couplings): [nv][nh]."""

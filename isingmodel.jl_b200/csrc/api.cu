@@ -1462,28 +1462,18 @@ int isb_sk_rows(isb_ctx *ctx, int n, uint64_t seed, int row0, int nrows, double 
     return ISB_OK;
 }
 
-int isb_shard_halfstep_dev(isb_model *m, int R, int replica_offset, int layer, int rule, const void *in_full_bf16,
-                           void *out_block_bf16, uint64_t seed, uint64_t step_abs, double T) {
-    return isb_shard_halfstep_fused_dev(m, R, replica_offset, layer, rule, in_full_bf16, out_block_bf16, 0, nullptr, seed,
-                                        step_abs, T);
-}
-
-int isb_shard_halfstep_fused_dev(isb_model *m, int R, int replica_offset, int layer, int rule, const void *in_full_bf16,
-                                 void *out_block_bf16, int n_peers, void *const *peer_blocks_bf16, uint64_t seed,
-                                 uint64_t step_abs, double T) {
+int isb_shard_halfstep_dev(isb_model *m, int R, int replica_offset, int layer, int rule, const void *in_full,
+                           void *out_block, uint64_t seed, uint64_t step_abs, double T) {
     if (!m) return ISB_ERR_ARG;
     isb_ctx *ctx = m->ctx;
     ISB_LOCK(ctx);
     const char *who = "isb_shard_halfstep_dev";
     if (m->kind != ISB_KIND_SHARD) return fail(ctx, ISB_ERR_STATE, "%s: not a row-sharded model", who);
-    if (!in_full_bf16 || !out_block_bf16 || R <= 0 || replica_offset < 0 || (layer != 0 && layer != 1) || n_peers < 0 ||
-        n_peers > 7 || (n_peers > 0 && !peer_blocks_bf16) || (rule != ISB_BIP_SCA && rule != ISB_BIP_MA) || !std::isfinite(T))
+    if (!in_full || !out_block || R <= 0 || replica_offset < 0 || (layer != 0 && layer != 1) ||
+        (rule != ISB_BIP_SCA && rule != ISB_BIP_MA) || !std::isfinite(T))
         return fail(ctx, ISB_ERR_ARG, "%s: bad argument", who);
-    for (int q = 0; q < n_peers; ++q)
-        if (!peer_blocks_bf16[q]) return fail(ctx, ISB_ERR_ARG, "%s: NULL peer pointer", who);
     ISB_CUDA(ctx, cudaSetDevice(ctx->device));
-    return isb::shard_halfstep_device(m, R, replica_offset, layer, rule, in_full_bf16, out_block_bf16, n_peers,
-                                      peer_blocks_bf16, seed, step_abs, T);
+    return isb::shard_halfstep_device(m, R, replica_offset, layer, rule, in_full, out_block, seed, step_abs, T);
 }
 
 // ------------------------------------------------------------------ instrumentation

@@ -122,8 +122,8 @@ struct TcLayer {
     const float *bias_f;     // [nout rounded up to 16] the same in float (Philox mode)
     const double *F;         // external fluctuations (f64) or NULL
     uint32_t domain;         // Philox stream of this layer
-    // fused all-gather (row-sharded SCA): the sampled block is also stored straight into every peer GPU's
-    // gathered matrix through NVLink-mapped pointers (same [R][ldo] addressing as out_bf), tile by tile
+    // peer stores of the sampled block: always 0 since the fused row-sharded half-step was removed.  Kept with the epilogue's
+    // peer-store loops: without them ptxas reschedules the int8 kernel, measured 0.7 % slower on C3 (DESIGN §7)
     int npeer;
     void *peer[7];
 };
@@ -1688,7 +1688,7 @@ int shard_model_init(isb_model *m, const double *Wrows, uint64_t seed, double q,
 int shard_elem_size(const isb_model *m) { return ((const TcModel *)m->tc)->i8 ? 1 : 2; }
 
 int shard_halfstep_device(isb_model *m, int R, int replica_offset, int layer, int rule, const void *in_full, void *out_block,
-                          int n_peers, void *const *peer_blocks, uint64_t seed, uint64_t step_abs, double T) {
+                          uint64_t seed, uint64_t step_abs, double T) {
     isb_ctx *ctx = m->ctx;
     TcModel *t = (TcModel *)m->tc;
     TcMaps maps;
@@ -1709,8 +1709,6 @@ int shard_halfstep_device(isb_model *m, int R, int replica_offset, int layer, in
     p.L[layer].u_off = m->shard_g * m->shard_nb;
     p.L[layer].num_kb = m->nv / bk;
     p.L[layer].kb_per_blk = m->shard_nb / bk;
-    p.L[layer].npeer = n_peers;
-    for (int q = 0; q < n_peers; ++q) p.L[layer].peer[q] = peer_blocks[q];
     if (t->i8) {  // the diagonal of W: unit u's own input spin sits in this rank's slab of the gathered input layer
         p.L[layer].diag_f = t->diag_f;
         p.L[layer].diag_d = t->diag_d;

@@ -249,7 +249,7 @@ void bip_tc_ens_free(isb_ens *e);
 int shard_model_init(isb_model *m, const double *Wrows /*[nb][n] or NULL*/, uint64_t seed, double q, double wmax);
 int bip_tc_effective_couplings(isb_model *m, double *W_host_rowmajor_vh);
 int shard_halfstep_device(isb_model *m, int R, int replica_offset, int layer, int rule, const void *in_full, void *out_block,
-                          int n_peers, void *const *peer_blocks, uint64_t seed, uint64_t step_abs, double T);
+                          uint64_t seed, uint64_t step_abs, double T);
 int shard_elem_size(const isb_model *m);  // bytes per +-1 of the spin matrices of a row-sharded model (1 int8, 2 bf16)
 int sk_rows_device(isb_ctx *ctx, int n, uint64_t seed, int row0, int nrows, double *d_out);
 int bip_run_tc_device(isb_ens *e, int rule, int64_t nsteps, int fluct_mode, const double *d_Fv,

@@ -461,7 +461,7 @@ int isb_shard_run_steps(isb_shard_run *s, int rule, int64_t nsteps, const double
                     gr.pending[src] = false;
                 }
                 void *own = s->G == 1 ? gr.full[layer] : gr.blk[layer];   // a single block samples in place
-                ISB_TRY(isb::shard_halfstep_device(m, gr.R, gr.r0, layer, rule, gr.full[src], own, 0, nullptr, seed,
+                ISB_TRY(isb::shard_halfstep_device(m, gr.R, gr.r0, layer, rule, gr.full[src], own, seed,
                                                    step_offset + (uint64_t)k, T));
                 s->launches += 1;
                 if (s->G == 1) continue;

@@ -4,23 +4,10 @@ The MultiSpinFlip SCA of an N-spin model is the bipartite SCA (reference: src/On
 embedding W = (J + qI)/2, sigma = tau = s (demo.jl:82-90).  When W does not fit one GPU, rank g owns the output
 units [g*nb, (g+1)*nb) of both half-steps and W[block rows, :]; after every half-step the freshly sampled
 [R][nb] blocks are exchanged into the block-major [G][R][nb] matrix that is the next half-step's K operand.
-torch is plumbing here: device buffers, streams, and the collective.
 
-Exchange modes (``exchange=``), all bit-identical, measured on 8 x B200 at N = 65536, R = 1024 (ms per half-step,
-bf16x1 / bf16x3; the MMA-only target is 0.81 / 2.43):
-  "copy"      (default) two replica groups; every rank pushes its freshly sampled block into all ranks' gathered
-              matrices with the COPY ENGINES (symmetric memory, cudaMemcpyAsync on a side stream, then a
-              cross-GPU barrier) while the other group's GEMM owns the SMs: the exchange hides     0.92 / 2.88
-  "nccl"      one ncclAllGather after every half-step kernel (fallback)                          1.11 / 3.11
-  "pipelined" the replicas are split into two groups and one group's all-gather runs on NCCL's stream under
-              the other group's GEMM (chains are independent).  NCCL's CTAs and the persistent GEMM CTAs (one
-              per SM, all of its shared memory) contend for the SMs: slower                       1.42 / 4.00
-  "fused"     the sampling epilogue stores every sampled run straight into all peers' gathered matrices
-              (symmetric memory, NVLink stores) and a cross-GPU barrier replaces the all-gather: the 32-byte
-              peer stores stall the epilogue warps: slower                                        1.67 / 3.51
-
-The library's noise is indexed by global (replica, step, unit), so the result depends neither on G nor on the
-grouping: with ``emulate_blocks=G`` one process plays all G ranks in turn on one GPU (parity tests).
+Multi-GPU runs go through ``ShardRunSCA``, whose step loop and exchange live in the library (isb_shard_run_*).
+``RowShardedSCA`` plays all G row blocks in turn in one process on one GPU: the library's noise is indexed by global
+(replica, step, unit), so the trajectory does not depend on G, and the tests use it as the reference for G > 1.
 """
 from __future__ import annotations
 
@@ -29,231 +16,77 @@ import numpy as np
 from . import _lib
 
 
-class _Group:
-    """One slice of the replicas with its own gathered matrices and in-flight collective."""
-
-    def __init__(self, r0, R, G, nb, nblocks_local, dev, torch, symm=None, dist_group=None, dtype=None):
-        bf = dtype if dtype is not None else torch.bfloat16   # +-1 in the operand format of the model (bf16 or int8)
-        self.r0, self.R = r0, R
-        self.hv = self.hh = None
-        if symm is not None:
-            self.full_v = symm.empty((G, R, nb), dtype=bf, device=dev)
-            self.full_h = symm.empty((G, R, nb), dtype=bf, device=dev)
-            self.hv = symm.rendezvous(self.full_v, dist_group)
-            self.hh = symm.rendezvous(self.full_h, dist_group)
-            self.full_v.zero_()
-            self.full_h.zero_()
-        else:
-            self.full_v = torch.zeros((G, R, nb), dtype=bf, device=dev)
-            self.full_h = torch.zeros((G, R, nb), dtype=bf, device=dev)
-        # this rank's freshly sampled blocks, one per layer (they also hold the block's previous values)
-        self.blk_v = [torch.ones((R, nb), dtype=bf, device=dev) for _ in range(nblocks_local)]
-        self.blk_h = [torch.ones((R, nb), dtype=bf, device=dev) for _ in range(nblocks_local)]
-        self.pending = {0: None, 1: None}  # in-flight all-gather producing full_v (layer 0) / full_h (layer 1)
-
-
 class RowShardedSCA:
-    def __init__(self, n: int, R: int, *, seed: int | None = None, q: float = 1.0, W=None, h=None, rule=_lib.BIP_SCA,
-                 prec=_lib.PREC_BF16X3, emulate_blocks: int | None = None, device: int | None = None, group=None,
-                 exchange: str | None = None, fused: bool | None = None):
+    def __init__(self, n: int, R: int, *, emulate_blocks: int, seed: int | None = None, q: float = 1.0, W=None, h=None,
+                 rule=_lib.BIP_SCA, prec=_lib.PREC_BF16X3, device: int | None = None):
         import torch
-        import torch.distributed as dist
 
-        self.torch, self.dist, self.group = torch, dist, group
+        self.torch = torch
         self.n, self.R, self.rule = int(n), int(R), rule
-        self.distributed = emulate_blocks is None and dist.is_available() and dist.is_initialized() \
-            and dist.get_world_size(group) > 1
-        if emulate_blocks is not None:
-            self.G, self.blocks = int(emulate_blocks), list(range(int(emulate_blocks)))
-        elif self.distributed:
-            self.G, self.blocks = dist.get_world_size(group), [dist.get_rank(group)]
-        else:
-            self.G, self.blocks = 1, [0]
+        self.G = int(emulate_blocks)
         if self.n % self.G:
             raise ValueError("n must be divisible by the number of blocks")
         self.nb = self.n // self.G
-        if fused is not None and exchange is None:  # older spelling
-            exchange = "fused" if fused else "nccl"
-        if exchange is None:
-            exchange = "copy"
-        if not self.distributed:
-            exchange = "local"
-        if exchange in ("pipelined", "copy") and self.R < 256:
-            exchange = "nccl"
-        self.exchange = exchange
         self.ctx = _lib.context(device)
         self.dev = torch.device("cuda", self.ctx.device)
         torch.cuda.set_device(self.dev)
         self.ctx.set_stream(torch.cuda.current_stream(self.dev).cuda_stream)
-        # operand format of the spin matrices: int8 +-1 for the int8 digit-plane models (half the bytes to exchange)
+        # operand format of the spin matrices: int8 +-1 for the int8 digit-plane models, else bf16
         self.dtype = torch.int8 if prec in _lib.I8_PRECS else torch.bfloat16
-        self.esz = 1 if prec in _lib.I8_PRECS else 2
         self.models = []
         wmax = 0.0
         if W is not None and prec in _lib.I8_PRECS:
-            # the fixed-point grid must be the same on every rank: the largest off-diagonal |W| of the whole matrix
+            # the fixed-point grid must be the same for every block: the largest off-diagonal |W| of the whole matrix
             Wa = np.abs(np.asarray(W, dtype=np.float64))
             wmax = float((Wa - np.diag(np.diag(Wa))).max())
-        for g in self.blocks:
+        for g in range(self.G):
             if W is not None:
                 Wg = np.asarray(W, dtype=np.float64)[g * self.nb:(g + 1) * self.nb, :]
                 hb = None if h is None else 0.5 * np.asarray(h, dtype=np.float64)[g * self.nb:(g + 1) * self.nb]
                 self.models.append(_lib.Model.shard_rows(self.ctx, self.n, self.G, g, Wg, hb, hb, prec, wmax=wmax))
             else:
                 self.models.append(_lib.Model.shard_sk(self.ctx, self.n, self.G, g, int(seed), q, prec))
-        symm = None
-        self.fused = False
-        self.cstream = None
-        if exchange == "copy":
-            try:
-                import torch.distributed._symmetric_memory as symm_mem
-                symm = symm_mem
-                self.cstream = torch.cuda.Stream(device=self.dev)
-            except Exception as exc:  # pragma: no cover
-                self.fused_error = repr(exc)
-                self.exchange = exchange = "nccl"
-        if exchange == "fused" and 2 <= self.G <= 8:
-            try:
-                import torch.distributed._symmetric_memory as symm_mem
-                symm = symm_mem
-                self.fused = True
-            except Exception as exc:  # pragma: no cover - depends on the torch build
-                self.fused_error = repr(exc)
-                self.exchange = exchange = "nccl"
-        grp = group if group is not None else (dist.group.WORLD if self.distributed else None)
-        if exchange in ("pipelined", "copy"):
-            half = (self.R // 2 + 127) // 128 * 128   # whole 128-replica tiles in the first group
-            slices = [(0, half), (half, self.R - half)]
-        else:
-            slices = [(0, self.R)]
-        try:
-            self.groups = [_Group(r0, Rg, self.G, self.nb, len(self.blocks), self.dev, torch, symm, grp, self.dtype)
-                           for r0, Rg in slices if Rg > 0]
-        except Exception as exc:  # pragma: no cover - symmetric memory unavailable on this driver
-            if not self.fused and self.cstream is None:
-                raise
-            self.cstream = None
-            self.fused, self.fused_error, self.exchange = False, repr(exc), "nccl"
-            self.groups = [_Group(0, self.R, self.G, self.nb, len(self.blocks), self.dev, torch, dtype=self.dtype)]
-        self.launches = 0
-        self.gather_bytes = 0
+        # the visible and hidden layers, block-major [G][R][nb]; block g samples in place into its slab
+        self.full_v = torch.zeros((self.G, self.R, self.nb), dtype=self.dtype, device=self.dev)
+        self.full_h = torch.zeros((self.G, self.R, self.nb), dtype=self.dtype, device=self.dev)
 
-    # ---- state
     def set_spins(self, S):
         """S: (R, n) int8 +-1; the embedding starts from sigma = tau = s."""
-        torch = self.torch
-        self._drain()
-        S = torch.as_tensor(np.ascontiguousarray(S, dtype=np.int8), device=self.dev)
-        for gr in self.groups:
-            full = S[gr.r0:gr.r0 + gr.R].view(gr.R, self.G, self.nb).permute(1, 0, 2).contiguous().to(self.dtype)
-            gr.full_v.copy_(full)
-            gr.full_h.copy_(full)
-            for i, g in enumerate(self.blocks):
-                gr.blk_v[i].copy_(full[g])
-                gr.blk_h[i].copy_(full[g])
-        if self.fused or self.cstream is not None:
-            # no peer may store into this rank's matrices before they hold the initial configuration
-            torch.cuda.synchronize(self.dev)
-            self.dist.barrier(group=self.group)
+        S = self.torch.as_tensor(np.ascontiguousarray(S, dtype=np.int8), device=self.dev)
+        full = S.view(self.R, self.G, self.nb).permute(1, 0, 2).to(self.dtype)
+        self.full_v.copy_(full)
+        self.full_h.copy_(full)
 
-    def _drain(self):
-        for gr in self.groups:
-            for layer in (0, 1):
-                if gr.pending[layer] is not None:
-                    self._wait(gr.pending[layer])
-                    gr.pending[layer] = None
-
-    def _wait(self, pending):
-        """Make the compute stream wait for an in-flight exchange (an NCCL work object or a CUDA event)."""
-        if hasattr(pending, "wait") and not isinstance(pending, self.torch.cuda.Event):
-            pending.wait()
-        else:
-            self.torch.cuda.current_stream(self.dev).wait_event(pending)
-
-    def _layer(self, which):
-        self._drain()
-        torch = self.torch
-        parts = []
-        for gr in self.groups:
-            full = gr.full_v if which == 0 else gr.full_h
-            s = (full > 0).to(torch.int8) * 2 - 1
-            parts.append(s.permute(1, 0, 2).reshape(gr.R, self.n))
-        return torch.cat(parts, 0).cpu().numpy()
+    def _layer(self, full):
+        s = (full > 0).to(self.torch.int8) * 2 - 1
+        return s.permute(1, 0, 2).reshape(self.R, self.n).cpu().numpy()
 
     def get_spins(self):
-        """(R, n) int8 visible layer (identical on every rank after the exchange)."""
-        return self._layer(0)
+        """(R, n) int8 visible layer."""
+        return self._layer(self.full_v)
 
     def get_hidden(self):
-        return self._layer(1)
-
-    # ---- one half-step of one replica group: every owned block samples its units, then the blocks are exchanged
-    def _half(self, gr, layer, seed, step_abs, T):
-        src, dst = (gr.full_v, gr.full_h) if layer == 1 else (gr.full_h, gr.full_v)
-        src_layer = 0 if layer == 1 else 1
-        if gr.pending[src_layer] is not None:   # the gathered input of this half-step (stream-level wait)
-            self._wait(gr.pending[src_layer])
-            gr.pending[src_layer] = None
-        if self.fused:
-            g, hdl = self.blocks[0], (gr.hh if layer == 1 else gr.hv)
-            slab = g * gr.R * self.nb * self.esz  # byte offset of this rank's block in every gathered matrix
-            peers = [int(ptr) + slab for q, ptr in enumerate(hdl.buffer_ptrs) if q != hdl.rank]
-            self.models[0].shard_halfstep_fused(gr.R, layer, self.rule, src.data_ptr(), dst.data_ptr() + slab, peers,
-                                                seed, step_abs, T, replica_offset=gr.r0)
-            self.launches += 1
-            self.gather_bytes += (self.G - 1) * gr.R * self.nb * self.esz
-            hdl.barrier(channel=0)  # all peers' stores have landed before anyone reads the layer
-            return
-        blk = gr.blk_h if layer == 1 else gr.blk_v
-        for i, m in enumerate(self.models):
-            m.shard_halfstep(gr.R, layer, self.rule, src.data_ptr(), blk[i].data_ptr(), seed, step_abs, T,
-                             replica_offset=gr.r0)
-            self.launches += 1
-        if self.cstream is not None:
-            # copy-engine exchange on the side stream: push this rank's block into every rank's gathered matrix
-            torch = self.torch
-            hdl = gr.hh if layer == 1 else gr.hv
-            g = self.blocks[0]
-            ready = torch.cuda.Event()
-            ready.record(torch.cuda.current_stream(self.dev))
-            with torch.cuda.stream(self.cstream):
-                self.cstream.wait_event(ready)
-                for q in range(self.G):
-                    peer = hdl.get_buffer(q, (self.G, gr.R, self.nb), self.dtype)
-                    peer[g].copy_(blk[0], non_blocking=True)
-                hdl.barrier(channel=0)
-                done = torch.cuda.Event()
-                done.record(self.cstream)
-            gr.pending[layer] = done
-            self.gather_bytes += (self.G - 1) * blk[0].numel() * self.esz
-        elif self.distributed:
-            # the one real exchange step of this path: [R][nb] per rank -> [G][R][nb] everywhere.  async_op: the
-            # collective runs on NCCL's stream after this kernel; the next kernel of the OTHER group is enqueued
-            # right behind this one and overlaps it ("pipelined"); "nccl" waits for it at the next half-step.
-            gr.pending[layer] = self.dist.all_gather_into_tensor(dst.view(-1), blk[0].view(-1), group=self.group,
-                                                                 async_op=True)
-            self.gather_bytes += (self.G - 1) * blk[0].numel() * self.esz
-        else:
-            for i, g in enumerate(self.blocks):
-                dst[g].copy_(blk[i])
+        return self._layer(self.full_h)
 
     def run(self, nsteps, T, *, seed=0, step_offset=0):
         """nsteps synchronous SCA steps; T: array of nsteps temperatures (T[k] applies to step k)."""
         T = np.atleast_1d(np.asarray(T, dtype=np.float64))
         for k in range(int(nsteps)):
             Tk = float(T[min(k, len(T) - 1)])
-            for layer in (1, 0):
-                for gr in self.groups:
-                    self._half(gr, layer, seed, step_offset + k, Tk)
-        self._drain()
+            for layer in (1, 0):   # hidden from the visible layer, then visible from the hidden layer
+                src, dst = (self.full_v, self.full_h) if layer == 1 else (self.full_h, self.full_v)
+                # a half-step reads only src and its own slab of dst (MomentumAnnealing's previous values)
+                for g, m in enumerate(self.models):
+                    m.shard_halfstep(self.R, layer, self.rule, src.data_ptr(), dst[g].data_ptr(), seed, step_offset + k, Tk)
 
 
 class ShardRunSCA:
-    """The same path with the step loop INSIDE the library (isb_shard_run_*, include/ising_b200.h): the two replica
-    groups, the exchange after every half-step (``exchange="nccl"``: ncclAllGather through the library's own
-    communicator; ``"copy"``: copy-engine pushes into IPC-mapped peer matrices + stream memory operations) and their
-    ordering run in C; torch.distributed only carries the 128-byte NCCL id / the 64-byte IPC handles between the ranks
-    at construction.  What a C or Julia caller of the row-sharded path executes, step for step."""
+    """The row-sharded SCA, one process per GPU, with the step loop inside the library (isb_shard_run_*,
+    include/ising_b200.h): the two replica groups, the exchange after every half-step (``exchange="nccl"``:
+    ncclAllGather through the library's own communicator; ``"copy"``: copy-engine pushes into IPC-mapped peer matrices
+    + stream memory operations) and their ordering run in C; torch.distributed only carries the 128-byte NCCL id / the
+    64-byte IPC handles between the ranks at construction.  What a C or Julia caller of the row-sharded path executes,
+    step for step."""
 
     def __init__(self, n: int, R: int, *, seed: int | None = None, q: float = 1.0, W=None, h=None, rule=_lib.BIP_SCA,
                  prec=_lib.PREC_I8X3, device: int | None = None, group=None, exchange: str = "copy"):
@@ -266,7 +99,6 @@ class ShardRunSCA:
             raise ValueError("n must be divisible by the number of blocks")
         self.nb = self.n // self.G
         self.ctx = _lib.context(device)
-        self.esz = 1 if prec in _lib.I8_PRECS else 2
         if W is not None:
             Wa = np.asarray(W, dtype=np.float64)
             wmax = float((np.abs(Wa) - np.diag(np.abs(np.diag(Wa)))).max()) if prec in _lib.I8_PRECS else 0.0
@@ -280,7 +112,6 @@ class ShardRunSCA:
         if self.distributed:
             self.run_obj.wire(dist, group)
         self.launches = 0
-        self.gather_bytes = 0
 
     def set_spins(self, S):
         self.run_obj.set_spins(S)
@@ -295,5 +126,4 @@ class ShardRunSCA:
         self.run_obj.steps(self.rule, nsteps, T, seed=seed, step_offset=step_offset)
         st = self.run_obj.last_stats()
         self.launches += st["launches"]
-        self.gather_bytes += 2 * int(nsteps) * (self.G - 1) * self.R * self.nb * self.esz
         return st

@@ -1,6 +1,6 @@
-"""GPU tests of the row-sharded synchronous SCA (BASELINE config 5): the result must not depend on the number of
-row blocks, must equal the unsharded tensor-core path (itself checked against the oracle), and the NCCL
-all-gather variants (2, 4 and 8 processes, one per GPU) must equal the single-process emulation."""
+"""GPU tests of the row-sharded synchronous SCA (BASELINE config 5): the single-process emulation must not depend
+on the number of row blocks and must equal the unsharded tensor-core path (itself checked against the oracle), and
+the library's step loop (one block, and 2, 4 and 8 processes, one per GPU) must equal the emulation."""
 import os
 import subprocess
 import sys
@@ -106,8 +106,8 @@ def test_step_loop_inside_the_library_single_block(pkg, ctx, synth, prec_name, r
 
 @pytest.mark.parametrize("ranks", [2, 4, 8])
 def test_nccl_all_gather_ranks(pkg, ctx, ranks):
-    """One process per GPU under torchrun: every exchange mode (NCCL all-gather, the two-group pipeline, copy-engine pushes,
-    peer stores in the epilogue, and the library's own isb_shard_run_* loops) against the single-process emulation."""
+    """One process per GPU under torchrun: the library's isb_shard_run_* loop with either exchange (ncclAllGather,
+    copy-engine pushes) against the single-process emulation."""
     import torch
     if torch.cuda.device_count() < ranks:
         pytest.skip(f"needs {ranks} GPUs")
