@@ -321,8 +321,7 @@ static int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const
     const int npl = m->npl;
     const int jsize = jf ? 4 : 8;
     const int rowb = m->npad * jsize;
-    const int field_regs = npl * (hd ? 2 : 1);   // (int32 fields are budgeted like Float64 ones: SsfCfg)
-    const int max_chains = ssf_max_chains(field_regs);
+    const int max_chains = fixed ? SSF_FIXED_CHAINS : ssf_max_chains(npl * (hd ? 2 : 1));
 
     int ctas, nw;
     if (e->R <= ctx->num_sms) {
@@ -385,7 +384,7 @@ static int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const
     p.od_ratio = 0.8f;
 
     p.fluct_pitch = nsteps;
-    const int threads = 32 * (nw + 1);
+    const int threads = 32 * (nw + (fixed ? 0 : 1));   // (+ the producer warp of the ring kernels)
     // one launch over the steps [t0, t0 + len) of the run: every per-step input is offset on the host, the kernel sees a
     // run of `len` steps (t0 is a multiple of steps_per_T and of trace_every, see below)
     // mode 2: streaming kernel (TMA ring); 1: plain kernel (rows on demand, fields in registers); 0: cold kernel (fields in
@@ -447,8 +446,8 @@ static int ssf_run_device(isb_ens *e, int rule, int64_t nsteps, int order, const
     if (const char *env_th = getenv("ISB_SSF_SEG_THR")) thr = atof(env_th);
     cudaError_t ce = cudaSuccess;
     // ... below which the shared-memory-field kernel is the fastest (one wave of 28 chains per SM).  Fixed point: the cold
-    // kernel overtakes the plain one between 7.7 % and 5.5 % acceptance (C2 profile, profiles/ssf_fixed_ab_b200.json)
-    double thr_cold = fixed ? 0.06 : 0.03;
+    // kernel overtakes the plain one between 2.8 % and 2.0 % acceptance (C2 profile, profiles/ssf_fixed_ab_b200.json)
+    double thr_cold = 0.03;
     if (const char *env_tc = getenv("ISB_SSF_COLD_THR")) thr_cold = atof(env_tc);
     if (cold_chains < 16) thr_cold = -1.0;
     // ISB_SSF_MODE = 0 | 1 | 2: one launch of that kernel (A/B runs and tests).  A mode the run cannot take is an error, so

@@ -91,13 +91,15 @@ constexpr int SSF_EPOCH_OD = 8 * 1024;  // steps per on-demand epoch: chains re-
 __host__ __device__ constexpr int ssf_max_chains(int field_regs) {
     return field_regs > 32 ? 14 : (field_regs > 16 ? 20 : 28);
 }
+// The fixed-point kernel has no ring and hence no producer warp: 28 chains per CTA, 896 threads -> 72 registers/thread,
+// so that C2's 4096 replicas run in one wave (147 CTAs on 148 SMs)
+constexpr int SSF_FIXED_CHAINS = 28;
 
 template <typename HT, int NPL>
 struct SsfCfg {
-    // (int32 fixed-point fields are budgeted like Float64 ones: their decision step and fallback need the registers)
-    static constexpr int kFieldRegs = NPL * (std::is_same<HT, int32_t>::value ? 2 : (int)sizeof(HT) / 4);
-    static constexpr int kMaxChains = ssf_max_chains(kFieldRegs);
-    static constexpr int kMaxThreads = 32 * (kMaxChains + 1);
+    static constexpr bool kFixed = std::is_same<HT, int32_t>::value;
+    static constexpr int kMaxChains = kFixed ? SSF_FIXED_CHAINS : ssf_max_chains(NPL * (int)sizeof(HT) / 4);
+    static constexpr int kMaxThreads = 32 * (kMaxChains + (kFixed ? 0 : 1));
 };
 
 // compile-time loop: f(integral_constant<int, I>) for I in [0, N) — keeps register-array indices static
@@ -441,7 +443,11 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
             int len = 32 - l_first;
             if (p.n - site < len) len = p.n - site;
             if (p.nsteps - t < len) len = (int)(p.nsteps - t);
-            if (next_trace - t < len) len = (int)(next_trace - t);
+            // Fixed-point runs are never traced (ssf_run_device).  Compiling the trace points out of that kernel frees the
+            // registers that, at its 72-register budget, would otherwise hold two of the fields in local memory across
+            // the flip loop.
+            if constexpr (!FIXED)
+                if (next_trace - t < len) len = (int)(next_trace - t);
             if (TMA && ep_len - te < len) len = ep_len - te;
             const int off = lane - l_first;
             const bool mine = off >= 0 && off < len;
@@ -595,9 +601,11 @@ __global__ void __launch_bounds__(SsfCfg<HT, NPL>::kMaxThreads, 1) ssf_kernel(co
             }
             te += len;
             if (TMA && stream) advance_to((te - 1) / G);
-            if (t == next_trace) {
-                write_trace(trace_idx++);
-                next_trace += p.trace_every;
+            if constexpr (!FIXED) {
+                if (t == next_trace) {
+                    write_trace(trace_idx++);
+                    next_trace += p.trace_every;
+                }
             }
             if (TMA && te == ep_len) epoch_boundary(t);
         }

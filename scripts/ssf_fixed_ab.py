@@ -37,6 +37,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--thr", default="0.02,0.025,0.03,0.035,0.045,0.06", help="ISB_SSF_COLD_THR values of the grid")
     args = ap.parse_args()
     import bench
     from isingmodel_jl_b200 import _lib as L, synth
@@ -91,7 +92,7 @@ def main():
     res["profile"] = prof
 
     grid = []
-    for thr_cold in ("0.03", "0.045", "0.06", "0.08", "0.1"):
+    for thr_cold in args.thr.split(","):
         os.environ["ISB_SSF_COLD_THR"] = thr_cold
         ms = []
         for _ in range(args.reps):
